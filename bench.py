@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload c2|c1|c3|c3d|c4|c4x|c5a|c5b|c5b_build]   (one workload only; default: all of BASELINE.json)
+                    [--dump-outputs DIR]   (the headline's last timed step, see dump_outputs)
 
 Prints ONE JSON line (rank 0).  A "step" is one pass of the hot path over one query batch (one fused evaluation
 launch; three launches when a bilinear batch is binned).  The headline is BASELINE.json configs[1] (C2: Interp1D
@@ -444,6 +445,31 @@ def gather_samples(ctx, tensors):
     return per_rank
 
 
+DUMP_BYTES = 48 << 20          # --dump-outputs: sampled output bytes of all files together
+
+
+def dump_outputs(ctx, arrays, axis):
+    """--dump-outputs DIR: what the last timed step handed its caller, written by rank 0 as DIR/<name>.npy.
+    arrays: {name: device tensor}; an output too large for DUMP_BYTES keeps the slices along `axis` (query rows,
+    spline columns) at sorted indices drawn from a fixed seed, on every rank's shard, so that two builds run with
+    the same arguments write files that compare element for element."""
+    torch = ctx.torch
+    budget = DUMP_BYTES // (len(arrays) * ctx.world)
+    samples = []
+    for t in arrays.values():
+        n = t.shape[axis]
+        k = min(n, max(1, budget // (t.element_size() * t.numel() // n)))
+        idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        samples.append(t.index_select(axis, torch.from_numpy(idx).to(t.device)))
+    per_rank = gather_samples(ctx, samples)
+    if ctx.rank == 0:
+        os.makedirs(ctx.args.dump_outputs, exist_ok=True)
+        for i, name in enumerate(arrays):
+            a = np.concatenate([parts[i] for parts in per_rank], axis=axis)
+            np.save(os.path.join(ctx.args.dump_outputs, name + ".npy"), a)
+            print(f"dump-outputs: {name}.npy {a.dtype} {a.shape}", file=sys.stderr)
+
+
 def timed_steps(ctx, step, steps, flush_l2, sampler=None):
     """K steps, each bracketed by its own CUDA events on the launch stream.  Returns (ms per step from the first
     start to the last end -- or the sum of the steps when L2 is scrubbed in between --, sorted per-step list)."""
@@ -604,6 +630,8 @@ def measure_eval(ctx, name, wl, steps, warmup, role, sampler=None):
     ms_per_step, per = timed_steps(ctx, step, steps, flush_l2, sampler)
     launches = D.kernel_launch_count() - launches0
     assert D.err_word_value(err) == D.ERR_NONE, "a benchmark query failed"
+    if role == "headline" and ctx.args.dump_outputs:
+        dump_outputs(ctx, {name + "_out": out}, 0)
     value = world * nq / (ms_per_step * 1e-3)
     peak, peak_src = measured_peak()
     achieved = abytes / (ms_per_step * 1e-3) / 1e9
@@ -752,7 +780,7 @@ def time_builds(ctx, ip, wl):
     return out
 
 
-def measure_build(ctx, name, wl, steps, warmup):
+def measure_build(ctx, name, wl, steps, warmup, role):
     """C5's spline construction at scale: (4096, 131072) f32, columns sharded over the GPUs, coefficients all-gathered"""
     torch, dist = ctx.torch, ctx.dist
     from ndarray_interp_b200 import device as D
@@ -770,7 +798,6 @@ def measure_build(ctx, name, wl, steps, warmup):
         return torch.randn((n, cw), dtype=torch.float32, device=dev, generator=gen)
     y = shard_data(rank)
     part = D.DeviceInterp1D(g, y, assume_valid=True)
-    steps = max(2, min(steps, 5))
     for _ in range(2):
         st, _ = part.spline_build(BC_NATURAL)
         assert st == 0
@@ -784,6 +811,8 @@ def measure_build(ctx, name, wl, steps, warmup):
     nel = (n - 1) * cw
     a_sh = _tensor_from_ptr(torch, pa, nel, torch.float32, dev).view(n - 1, cw)
     b_sh = _tensor_from_ptr(torch, pb, nel, torch.float32, dev).view(n - 1, cw)
+    if role == "headline" and ctx.args.dump_outputs:
+        dump_outputs(ctx, {name + "_a": a_sh, name + "_b": b_sh}, 1)
     gather_ms, a_full, b_full = 0.0, a_sh, b_sh
     if world > 1:
         a_full = torch.empty((world, n - 1, cw), dtype=torch.float32, device=dev)
@@ -870,7 +899,7 @@ def run_b200(args):
     sampler.start()
     launches0 = D.kernel_launch_count()
     if wl["kind"] == "build":
-        head = measure_build(ctx, name, wl, args.steps, args.warmup)
+        head = measure_build(ctx, name, wl, args.steps, args.warmup, "headline")
         head.setdefault("ms_per_step", head["build_ms"])
     else:
         head = measure_eval(ctx, name, wl, args.steps, max(args.warmup, 3), "headline", sampler)
@@ -888,7 +917,7 @@ def run_b200(args):
             try:
                 owl = WORKLOADS[o]
                 k = max(3, min(args.steps, 10 if owl.get("strong") else 20))
-                others[o] = (measure_build(ctx, o, owl, k, 2) if owl["kind"] == "build"
+                others[o] = (measure_build(ctx, o, owl, min(k, 5), 2, "side") if owl["kind"] == "build"
                              else measure_eval(ctx, o, owl, k, 3, "side"))
                 if "e2e" in others[o]:
                     others[o]["e2e"]["frac_of_d2h_link_all_ranks"] = (others[o]["e2e"]["d2h_achieved_GBps_all_ranks"]
@@ -935,7 +964,7 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of the headline workload")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS),
@@ -944,6 +973,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--search-mode", type=int, default=0,
                     help="lower-index search strategy for measurement (0 auto, 1 global bisect, 2 smem bisect, 3 guess, 4 bucket table, 5 merge)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step computed as DIR/<name>.npy (a fixed, seeded sample "
+                         "of a large output; at most 48 MB in all) so that two builds can be compared output for output")
     args = ap.parse_args()
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints "NCCL version ..." at the
     # first communicator, seen on the GPU boxes), so everything but the final line goes to stderr: file

@@ -1,9 +1,13 @@
 """bench.py's reference arm runs on the host cores only, so its JSON contract can be checked without a GPU:
-one line, the keys the driver reads, rank != 0 silent."""
+one line, the keys a reader of the line relies on, rank != 0 silent.  On the GPU: --steps sets the timed steps and
+--dump-outputs writes the same values for the same arguments."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -35,6 +39,24 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
 def test_reference_arm_other_ranks_exit_silently():
     r = run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, "--gpus", "2")
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_steps_and_dump_outputs_on_the_gpu(tmp_path):
+    """the headline times exactly --steps steps, and two runs with the same arguments dump the same values"""
+    dumps = []
+    for i, steps in enumerate((4, 7)):
+        d = tmp_path / str(i)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c1", "--steps", str(steps),
+                            "--warmup", "1", "--no-cpu", "--e2e-steps", "1", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr
+        line = json.loads(r.stdout)
+        assert line["steps"] == steps and line["per_step"]["n"] == steps and line["check"]["bit_exact"]
+        assert sorted(os.listdir(d)) == ["c1_out.npy"]
+        dumps.append(np.load(d / "c1_out.npy"))
+    assert dumps[0].dtype == np.float64 and dumps[0].shape == (10_000, 1)
+    assert np.array_equal(dumps[0], dumps[1])
 
 
 def test_traffic_stamps_name_committed_captures_of_the_current_kernel_sources():
