@@ -5,12 +5,13 @@
 //   results <= 256 KB : the latency path of interp_scalar / interp / interp_into: queries and rows live in the
 //                   thread's pinned workspace, which the kernel reads and writes directly; completion is a flag
 //                   in that workspace (profiles/r01/latency.md).
-//   larger batches : (1) queries uploaded once, (2) K7 pre-pass finds the first query the reference
-//                   would fail on, (3) only the rows before it are evaluated, in chunks alternating
-//                   between two streams so the D2H copy of one chunk overlaps the kernel of the
-//                   next.  Rows at and after the failing query stay untouched, like the reference
-//                   (interp1d/mod.rs:321,336-340).  Page-locked output arrays receive the chunks directly;
-//                   ordinary pageable ones through three pinned staging buffers and a pool of copy threads.
+//   larger batches : chunk by chunk, (1) the queries go up on a copy-in stream a few chunks ahead, (2) the
+//                   K7 pre-pass over each chunk finds the first query the reference would fail on, (3) only
+//                   the rows before it are evaluated, alternating between two streams so the D2H copy of
+//                   one chunk overlaps the kernel of the next.  Rows at and after the failing query stay
+//                   untouched, like the reference (interp1d/mod.rs:321,336-340).  Page-locked output arrays
+//                   receive the chunks directly; ordinary pageable ones through three pinned staging
+//                   buffers and a pool of copy threads.
 // All per-call state lives in a thread-local workspace, so one handle can be used from many
 // threads at once (the reference's &self methods are called from rayon workers).
 #include <atomic>
@@ -86,11 +87,6 @@ struct DeviceGuard {
     ~DeviceGuard() { if (changed) cudaSetDevice(prev); }
 };
 
-static long env_long(const char* name, long dflt) {
-    const char* v = getenv(name);
-    return v && *v ? strtol(v, nullptr, 10) : dflt;
-}
-
 static size_t elem_size(ndi_dtype d) { return (d == NDI_F64 || d == NDI_I64 || d == NDI_U64) ? 8 : 4; }
 static bool dtype_ok(ndi_dtype d) { return d >= NDI_F32 && d <= NDI_U64; }
 
@@ -117,12 +113,9 @@ static ndi_status dispatch_float(ndi_dtype d, F&& f) {
 
 // ---- thread-local workspace --------------------------------------------------------------------------
 constexpr size_t kChunkBytes = 64ull << 20;    // output bytes per pipeline chunk
-#ifndef NDI_TINY_KB
-#define NDI_TINY_KB 256
-#endif
-constexpr size_t kSmallBytes = 256ull << 10;   // outputs up to this size take the single-sync path
-constexpr size_t kTinyBytes = NDI_TINY_KB * 1024ull;     // ... and up to this size the kernel reads / writes pinned host memory directly
-constexpr size_t kTinyQueryBytes = NDI_TINY_KB * 1024ull;
+// results up to this size (and so queries, never more bytes than their rows) go through the pinned workspace,
+// which the kernel reads and writes directly
+constexpr size_t kTinyBytes = 256ull << 10;
 
 struct Workspace {
     bool ready = false;
@@ -136,7 +129,7 @@ struct Workspace {
     unsigned long long* d_err = nullptr;      // 8 words: [0] call, [1] tiny-batch path, [4..6] chunks of the streaming pipeline
     int32_t* d_res = nullptr;                 // 2 words (grid classify result)
     uint32_t* d_scr = nullptr;                // grid classify scratch
-    unsigned char* h_pin = nullptr; size_t h_pin_cap = 0;   // pinned: [err word, flag | small outputs | tiny queries]
+    unsigned char* h_pin = nullptr; size_t h_pin_cap = 0;   // pinned: [err word, flag | tiny outputs | tiny queries x 2]
     unsigned char* h_stage[3] = {nullptr, nullptr, nullptr};   // pinned staging for pageable outputs (lazy)
     cudaEvent_t stage_ev[3] = {nullptr, nullptr, nullptr};
     unsigned long long seq = 0;               // completion counter of the tiny-batch path
@@ -158,7 +151,7 @@ static Workspace* workspace(int dev, ndi_status* st) {
     if ((e = cudaMalloc(&w.d_err, 8 * sizeof(unsigned long long))) != cudaSuccess) { *st = cuda_fail(e, "cudaMalloc"); return nullptr; }
     if ((e = cudaMalloc(&w.d_res, 2 * sizeof(int32_t))) != cudaSuccess) { *st = cuda_fail(e, "cudaMalloc"); return nullptr; }
     if ((e = cudaMalloc(&w.d_scr, grid_classify_scratch_words() * sizeof(uint32_t))) != cudaSuccess) { *st = cuda_fail(e, "cudaMalloc"); return nullptr; }
-    w.h_pin_cap = 64 + kSmallBytes + 2 * kTinyQueryBytes;
+    w.h_pin_cap = 64 + 3 * kTinyBytes;
     if ((e = cudaMallocHost(&w.h_pin, w.h_pin_cap)) != cudaSuccess) { *st = cuda_fail(e, "cudaMallocHost"); return nullptr; }
     w.ready = true;
     return &w;
@@ -240,9 +233,7 @@ static bool is_pageable_host(const void* p) {
 // ---- search configuration ----------------------------------------------------------------------------
 // A grid that does not fit the shared-memory budget gets a coarse table grid[0], grid[S], ... built
 // once per handle; the kernels bisect the coarse table in shared memory and finish in L1/L2.
-#ifndef NDI_LUT_PER_POINT
-#define NDI_LUT_PER_POINT 8                      // buckets per grid point (rounded up to a power of two)
-#endif
+constexpr int64_t kLutPerPoint = 8;              // buckets per grid point (rounded up to a power of two)
 constexpr size_t kFullStageBytes = 48 * 1024;    // stage the whole grid up to this size
 constexpr size_t kCoarseBytes = 16 * 1024;       // target size of a coarse table
 
@@ -315,7 +306,7 @@ static ndi_status build_aids(ndi_dtype dtype, const void* grid, int64_t n, cudaS
     CK(cudaMemcpyAsync(ends + 8, (const unsigned char*)grid + (size_t)(n - 1) * elem, elem, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     int nb = 16;
-    while (nb < (int64_t)NDI_LUT_PER_POINT * n && nb < (1 << 24)) nb <<= 1;
+    while (nb < kLutPerPoint * n && nb < (1 << 24)) nb <<= 1;
     while ((size_t)nb * lut_entry_bytes(elem) > ((size_t)128 << 20) && nb > 16) nb >>= 1;   // keep the table well inside L2
     double g0d, scale;
     if (dtype == NDI_F32) {
@@ -409,9 +400,8 @@ static ndi_status classify_grid(ndi_dtype dtype, const void* x_dev, int64_t n, W
 // one pass over an f32 table: may the kernels use the hoisted-reciprocal division? (ndi_device.cuh)
 static ndi_status scan_fast_tables(ndi_dtype dtype, const void* data_dev, size_t count, Workspace* ws, int* fast) {
     *fast = 0;
-    static const bool disabled = getenv("NDI_NO_FAST_DIV") != nullptr;
-    if (dtype == NDI_F64) { *fast = !disabled; return NDI_OK; }   // f64 checks every quotient itself (div_ok): no scan needed
-    if (dtype != NDI_F32 || disabled) return NDI_OK;
+    if (dtype == NDI_F64) { *fast = 1; return NDI_OK; }   // f64 checks every quotient itself (div_ok): no scan needed
+    if (dtype != NDI_F32) return NDI_OK;
     const int32_t one = 1;
     CK(cudaMemcpyAsync(ws->d_res, &one, sizeof(one), cudaMemcpyHostToDevice, ws->s[0]));
     CK(launch_table_fast_div((const float*)data_dev, count, ws->d_res, ws->s[0]));
@@ -485,12 +475,11 @@ static ndi_status pack_view(const void* base, size_t es, int ndim, const int64_t
 
 // Pair table for Linear on thin rows (ndi_eval.cu: interp1d_linear_pair_kernel): twice the table, so only while
 // it stays comfortably L2-resident -- beyond that the gathers are DRAM sectors either way and nothing is gained.
-// NDI_PAIR_TABLE=0 switches it off (A/B measurement).
+constexpr size_t kPairMaxBytes = 48ull << 20;
 static ndi_status build_pair_table(ndi_interp1d* h, cudaStream_t st) {
-    static const long enabled = env_long("NDI_PAIR_TABLE", 1), max_mb = env_long("NDI_PAIR_MAX_MB", 48);
     const size_t es = elem_size(h->dtype);
     const size_t bytes = (size_t)(h->n - 1) * 2 * (size_t)h->w * es;
-    if (!enabled || !pair_table_shape_ok(h->w, es) || bytes > ((size_t)max_mb << 20) || ((uintptr_t)h->data & 15)) return NDI_OK;
+    if (!pair_table_shape_ok(h->w, es) || bytes > kPairMaxBytes || ((uintptr_t)h->data & 15)) return NDI_OK;
     CK(cudaMalloc(&h->pair, bytes));
     ndi_status s2 = dispatch(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
@@ -499,6 +488,26 @@ static ndi_status build_pair_table(ndi_interp1d* h, cudaStream_t st) {
     });
     if (s2 != NDI_OK) return s2;
     CK(cudaStreamSynchronize(st));
+    return NDI_OK;
+}
+
+// A copy of handle h on another device: fill(c, copy) points the copy c at its own device arrays, made with
+// copy(&dst, src, bytes) (an NVLink peer copy), before anything in it can fail; a clone that fails is destroyed.
+template <class H, class Fill>
+static ndi_status clone_to_device(const H* h, int32_t device, H** out, ndi_status (*destroy)(H*), Fill&& fill) {
+    if (!h || !out) return fail(NDI_INVALID_ARGUMENT, "null pointer");
+    *out = nullptr;
+    DeviceGuard g(device);
+    H* c = new H(*h);
+    c->device = device;
+    auto copy = [&](void** dst, const void* src, size_t bytes) -> ndi_status {
+        CK(cudaMalloc(dst, bytes));
+        CK(cudaMemcpyPeer(*dst, device, src, h->device, bytes));
+        return NDI_OK;
+    };
+    const ndi_status st = fill(c, copy);
+    if (st != NDI_OK) { destroy(c); return st; }
+    *out = c;
     return NDI_OK;
 }
 
@@ -717,28 +726,19 @@ ndi_status ndi_interp1d_device_ptrs(const ndi_interp1d* h, const void** x, const
 }
 
 ndi_status ndi_interp1d_clone_to_device(const ndi_interp1d* h, int32_t device, ndi_interp1d** out) {
-    if (!h || !out) return fail(NDI_INVALID_ARGUMENT, "null pointer");
-    *out = nullptr;
-    DeviceGuard g(device);
-    const size_t es = elem_size(h->dtype);
-    ndi_interp1d* c = new ndi_interp1d(*h);
-    c->device = device; c->owns_tables = true; c->owns_coeffs = h->a != nullptr;
-    c->x = c->data = c->a = c->b = c->pair = nullptr;
-    auto copy = [&](void** dst, const void* src, size_t bytes) -> ndi_status {
-        CK(cudaMalloc(dst, bytes));
-        CK(cudaMemcpyPeer(*dst, device, src, h->device, bytes));   // NVLink peer copy
-        return NDI_OK;
-    };
-    ndi_status st = copy(&c->x, h->x, (size_t)h->n * es);
-    if (st == NDI_OK) st = copy(&c->data, h->data, (size_t)h->n * h->w * es);
-    if (st == NDI_OK && h->a) st = copy(&c->a, h->a, (size_t)(h->n - 1) * h->w * es);
-    if (st == NDI_OK && h->b) st = copy(&c->b, h->b, (size_t)(h->n - 1) * h->w * es);
-    c->aids = GridAids{};
-    if (st == NDI_OK && !h->uniform_hint) st = build_aids(c->dtype, c->x, c->n, nullptr, &c->aids);
-    if (st == NDI_OK && h->pair) st = copy(&c->pair, h->pair, (size_t)(h->n - 1) * 2 * h->w * es);
-    if (st != NDI_OK) { cudaFree(c->x); cudaFree(c->data); cudaFree(c->a); cudaFree(c->b); cudaFree(c->pair); c->aids.release(); delete c; return st; }
-    *out = c;
-    return NDI_OK;
+    return clone_to_device(h, device, out, ndi_interp1d_destroy, [&](ndi_interp1d* c, auto& copy) {
+        const size_t es = elem_size(h->dtype);
+        c->owns_tables = true; c->owns_coeffs = h->a != nullptr;
+        c->x = c->data = c->a = c->b = c->pair = nullptr;
+        c->aids = GridAids{};
+        ndi_status st = copy(&c->x, h->x, (size_t)h->n * es);
+        if (st == NDI_OK) st = copy(&c->data, h->data, (size_t)h->n * h->w * es);
+        if (st == NDI_OK && h->a) st = copy(&c->a, h->a, (size_t)(h->n - 1) * h->w * es);
+        if (st == NDI_OK && h->b) st = copy(&c->b, h->b, (size_t)(h->n - 1) * h->w * es);
+        if (st == NDI_OK && !h->uniform_hint) st = build_aids(c->dtype, c->x, c->n, nullptr, &c->aids);
+        if (st == NDI_OK && h->pair) st = copy(&c->pair, h->pair, (size_t)(h->n - 1) * 2 * h->w * es);
+        return st;
+    });
 }
 
 }  // extern "C"
@@ -746,18 +746,27 @@ ndi_status ndi_interp1d_clone_to_device(const ndi_interp1d* h, int32_t device, n
 // ---- host-buffer pipeline -----------------------------------------------------------------------------------
 namespace {
 
+// A batch fanned out over several devices (ndi_*_group_*) runs each device's block of queries in two calls on the
+// block's worker thread, because the reference stops at the first failing query of the WHOLE batch.
+enum class Phase {
+    whole,      // everything in one call
+    prepass,    // queries up, pre-pass: *err_word = first failing query of this block
+    evaluate,   // evaluate the first `nvalid` rows only (the caller knows the batch-wide first failure by now)
+};
+
 struct HostEval {
     int device; size_t es; int ncoord; int64_t w;
     const void* q[2]; int64_t nq; void* out;
     // launch(q0_dev, q1_dev, nq, out_dev, err_dev, stream) evaluates a contiguous range of queries
-    // validate(q0_dev, q1_dev, nq, err_dev, stream) is the K7 pre-pass over all queries
-    // A batch fanned out over several devices (ndi_*_group_*) runs the pipeline in two phases per shard, on the
-    // shard's worker thread, because the reference stops at the first failing query of the WHOLE batch:
-    //   phase 1  queries up, pre-pass: *err_word = first failing query of this shard
-    //   phase 2  evaluate the first `nvalid` rows only (the caller knows the batch-wide first failure by now)
-    int phase = 0;            // 0: everything in one call
-    int64_t nvalid = 0;       // phase 2
+    // validate(q0_dev, q1_dev, nq, err_dev, stream) is the K7 pre-pass over a contiguous range of queries
+    Phase phase;
+    int64_t nvalid;           // Phase::evaluate
 };
+
+// An error word is the index of the first failing query (2-D: 2 * index + axis) within the range it was taken over.
+inline int64_t err_query(uint64_t word, int ncoord) { return (int64_t)(ncoord > 1 ? word >> 1 : word); }
+// ... and, for a range that starts at query `lo`, this is the same word within the whole batch
+inline uint64_t err_rebase(uint64_t word, int ncoord, int64_t lo) { return word + (ncoord > 1 ? 2 : 1) * (uint64_t)lo; }
 
 template <class Launch, class Validate>
 ndi_status run_host_eval(const HostEval& he, Launch&& launch, Validate&& validate, uint64_t* err_word) {
@@ -767,13 +776,14 @@ ndi_status run_host_eval(const HostEval& he, Launch&& launch, Validate&& validat
     ndi_status st; Workspace* ws = workspace(he.device, &st); if (!ws) return st;
     const size_t qbytes = (size_t)he.nq * he.es;
     const size_t row = (size_t)he.w * he.es;
-    if (he.phase == 0 && (size_t)he.nq * row <= kTinyBytes && qbytes <= kTinyQueryBytes) {
+    const size_t total = (size_t)he.nq * row;
+    if (he.phase == Phase::whole && total <= kTinyBytes) {
         // scalar / tiny-batch latency path (interp_scalar, interp, interp_into: interp1d/mod.rs:108-175): the
         // pinned workspace is mapped into the device's address space, so the kernel reads the queries from
         // it and writes the rows into it over PCIe; publish_kernel hands over the error word and raises the
         // flag this thread spins on: two launches, no copy call, no driver synchronisation
-        unsigned char* hq0 = ws->h_pin + 64 + kSmallBytes;
-        unsigned char* hq1 = hq0 + kTinyQueryBytes;
+        unsigned char* hq0 = ws->h_pin + 64 + kTinyBytes;
+        unsigned char* hq1 = hq0 + kTinyBytes;
         memcpy(hq0, he.q[0], qbytes);
         if (he.ncoord > 1) memcpy(hq1, he.q[1], qbytes);
         unsigned long long* tiny_err = ws->d_err + 1;          // its own word: publish_kernel leaves it armed (~0)
@@ -793,62 +803,65 @@ ndi_status run_host_eval(const HostEval& he, Launch&& launch, Validate&& validat
         }
         std::atomic_thread_fence(std::memory_order_acquire);
         memcpy(err_word, ws->h_pin, sizeof(uint64_t));
-        int64_t nvalid = he.nq;
-        if (*err_word != NDI_ERR_WORD_NONE) nvalid = (int64_t)(he.ncoord > 1 ? *err_word >> 1 : *err_word);
+        const int64_t nvalid = *err_word == NDI_ERR_WORD_NONE ? he.nq : err_query(*err_word, he.ncoord);
         memcpy(he.out, ws->h_pin + 64, (size_t)nvalid * row);
         return NDI_OK;
     }
-    const size_t total = (size_t)he.nq * row;
-    // One call over a large batch STREAMS: the queries go up chunk by chunk on a copy-in stream, a few chunks ahead of
-    // the evaluation, each followed by the pre-pass over that chunk, so the upload (host -> device) runs beside the
+    unsigned long long* d_err = ws->d_err;
+    for (int c = 0; c < he.ncoord && he.phase != Phase::evaluate; ++c)   // Phase::evaluate: this thread's prepass uploaded them
+        if ((st = grow(&ws->d_q[c], &ws->d_q_cap[c], qbytes)) != NDI_OK) return st;
+    const void* dq0 = ws->d_q[0];
+    const void* dq1 = he.ncoord > 1 ? ws->d_q[1] : nullptr;
+
+    if (he.phase == Phase::prepass) {                            // K7 pre-pass over the whole block: where would the reference stop?
+        auto prepass = [&]() -> ndi_status {
+            for (int c = 0; c < he.ncoord; ++c) CK(cudaMemcpyAsync(ws->d_q[c], he.q[c], qbytes, cudaMemcpyHostToDevice, ws->s[0]));
+            CK(cudaMemsetAsync(d_err, 0xff, sizeof(uint64_t), ws->s[0]));
+            if ((st = validate(dq0, dq1, he.nq, d_err, ws->s[0])) != NDI_OK) return st;
+            CK(cudaMemcpyAsync(ws->h_pin, d_err, sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s[0]));
+            CK(cudaStreamSynchronize(ws->s[0]));
+            memcpy(err_word, ws->h_pin, sizeof(uint64_t));
+            return NDI_OK;
+        };
+        if ((st = prepass()) != NDI_OK) cudaStreamSynchronize(ws->s[0]);   // no upload from the caller's memory left in flight
+        return st;
+    }
+
+    // A whole call over a large batch STREAMS: the queries go up chunk by chunk on a copy-in stream, a few chunks ahead
+    // of the evaluation, each followed by the pre-pass over that chunk, so the upload (host -> device) runs beside the
     // copy-out of earlier chunks (device -> host) instead of in front of it -- PCIe is full duplex, and for thin rows
     // the queries are a fifth of the bytes on the link (C4: 134 MB up, 537 MB down).  Chunks are consumed in order, so
     // stopping at the first chunk whose pre-pass reports a failure is the reference's "first Err" exactly.
-    static const bool stream_upload = [] { const char* e = getenv("NDI_STREAM_UPLOAD"); return !(e && *e == '0'); }();   // A/B switch
-    const bool streaming = stream_upload && he.phase == 0 && total > kSmallBytes;
-    for (int c = 0; c < he.ncoord && he.phase != 2; ++c) {    // phase 2: this thread uploaded them in phase 1
-        if ((st = grow(&ws->d_q[c], &ws->d_q_cap[c], qbytes)) != NDI_OK) return st;
-        if (!streaming) CK(cudaMemcpyAsync(ws->d_q[c], he.q[c], qbytes, cudaMemcpyHostToDevice, ws->s[0]));
-    }
-    const void* dq0 = ws->d_q[0];
-    const void* dq1 = he.ncoord > 1 ? ws->d_q[1] : nullptr;
-    unsigned long long* d_err = ws->d_err;
+    const bool streaming = he.phase == Phase::whole;
+    const int64_t nvalid = streaming ? he.nq : (he.nvalid < he.nq ? he.nvalid : he.nq);
+    if (nvalid <= 0) return NDI_OK;
 
-    if (he.phase == 0 && total <= kSmallBytes) {
-        // latency path: fused launch, one synchronisation
-        if ((st = grow(&ws->d_out[0], &ws->d_out_cap[0], total)) != NDI_OK) return st;
-        CK(cudaMemsetAsync(d_err, 0xff, sizeof(uint64_t), ws->s[0]));
-        if ((st = launch(dq0, dq1, he.nq, ws->d_out[0], d_err, ws->s[0])) != NDI_OK) return st;
-        CK(cudaMemcpyAsync(ws->h_pin, d_err, sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s[0]));
-        CK(cudaMemcpyAsync(ws->h_pin + 64, ws->d_out[0], total, cudaMemcpyDeviceToHost, ws->s[0]));
-        CK(cudaStreamSynchronize(ws->s[0]));
-        memcpy(err_word, ws->h_pin, sizeof(uint64_t));
-        int64_t nvalid = he.nq;
-        if (*err_word != NDI_ERR_WORD_NONE) nvalid = (int64_t)(he.ncoord > 1 ? *err_word >> 1 : *err_word);
-        memcpy(he.out, ws->h_pin + 64, (size_t)nvalid * row);
+    // Where finished chunks go: page-locked memory (or rows too wide to stage) receives them straight from the device;
+    // ordinary pageable memory through three pinned staging buffers, which the copy pool empties into it.
+    const bool staged = row <= kStageBytes / 32 && is_pageable_host(he.out);
+    int64_t per = (int64_t)((staged ? kStageBytes : kChunkBytes) / row) & ~31ll;   // queries per chunk
+    if (per < 32) per = 32;
+    const size_t chunk_bytes = (size_t)per * row;
+    CopyPool* pool = nullptr;
+    uint64_t ticket[3] = {0, 0, 0};
+    int64_t staged_cnt[3] = {0, 0, 0};
+    if (staged) {
+        for (int k = 0; k < 3; ++k) {
+            if (!ws->h_stage[k]) CK(cudaMallocHost(&ws->h_stage[k], kStageBytes));
+            if (!ws->stage_ev[k]) CK(cudaEventCreateWithFlags(&ws->stage_ev[k], cudaEventDisableTiming));
+        }
+        pool = &CopyPool::get();
+    }
+    auto hand_over = [&](int64_t j) -> ndi_status {             // chunk j has landed in its staging buffer: hand it to the pool
+        const int k = (int)(j % 3);
+        CK(cudaEventSynchronize(ws->stage_ev[k]));
+        ticket[k] = pool->submit((unsigned char*)he.out + (size_t)(j * per) * row, ws->h_stage[k], (size_t)staged_cnt[k] * row);
         return NDI_OK;
-    }
-
-    // K7 pre-pass: where would the reference stop?
-    int64_t nvalid = he.nq;
-    if (streaming) {
-        // decided chunk by chunk below
-    } else if (he.phase != 2) {
-        CK(cudaMemsetAsync(d_err, 0xff, sizeof(uint64_t), ws->s[0]));
-        if ((st = validate(dq0, dq1, he.nq, d_err, ws->s[0])) != NDI_OK) return st;
-        CK(cudaMemcpyAsync(ws->h_pin, d_err, sizeof(uint64_t), cudaMemcpyDeviceToHost, ws->s[0]));
-        CK(cudaStreamSynchronize(ws->s[0]));
-        memcpy(err_word, ws->h_pin, sizeof(uint64_t));
-        if (*err_word != NDI_ERR_WORD_NONE) nvalid = (int64_t)(he.ncoord > 1 ? *err_word >> 1 : *err_word);
-        if (he.phase == 1) return NDI_OK;
-    } else {
-        nvalid = he.nvalid < he.nq ? he.nvalid : he.nq;
-        if (nvalid <= 0) return NDI_OK;
-    }
+    };
 
     // the copy-in side of the streaming pipeline: chunk i = queries [i * per, (i + 1) * per)
     constexpr int kFeedDepth = 3;
-    auto feed = [&](int64_t i, int64_t per) -> ndi_status {
+    auto feed = [&](int64_t i) -> ndi_status {
         const int64_t lo = i * per;
         if (!streaming || lo >= he.nq) return NDI_OK;
         const int64_t cnt = he.nq - lo < per ? he.nq - lo : per;
@@ -865,96 +878,73 @@ ndi_status run_host_eval(const HostEval& he, Launch&& launch, Validate&& validat
         return NDI_OK;
     };
     // chunk i has arrived: how many of its rows does the reference write?  (fewer than all: the batch ends there)
-    auto fed = [&](int64_t i, int64_t per, int64_t cnt, int64_t* cnt_valid) -> ndi_status {
+    auto fed = [&](int64_t i, int64_t cnt, int64_t* cnt_valid) -> ndi_status {
         *cnt_valid = cnt;
         if (!streaming) return NDI_OK;
         const int k = (int)(i % kFeedDepth);
         CK(cudaEventSynchronize(ws->feed_ev[k]));
         uint64_t word; memcpy(&word, ws->h_pin + 16 + 8 * k, sizeof(word));
         if (word != NDI_ERR_WORD_NONE) {
-            const uint64_t lo = (uint64_t)(i * per);
-            *cnt_valid = (int64_t)(he.ncoord > 1 ? word >> 1 : word);
-            *err_word = he.ncoord > 1 ? word + 2 * lo : word + lo;
+            *cnt_valid = err_query(word, he.ncoord);
+            *err_word = err_rebase(word, he.ncoord, i * per);
         }
         return NDI_OK;
     };
-    // never return while a copy from (or into) the caller's memory is in flight
-    auto drain = [&]() { if (streaming) cudaStreamSynchronize(ws->s_in); cudaStreamSynchronize(ws->s[0]); cudaStreamSynchronize(ws->s[1]); };
 
-    static const bool stage_pageable = [] { const char* e = getenv("NDI_STAGE_PAGEABLE"); return !(e && *e == '0'); }();
-    if (stage_pageable && row <= kStageBytes / 32 && is_pageable_host(he.out)) {
-        // pageable output: device -> pinned staging (three buffers in flight) -> caller memory by the copy pool
-        int64_t per = (int64_t)(kStageBytes / row) & ~31ll;
-        for (int k = 0; k < 3; ++k) {
-            if (!ws->h_stage[k]) CK(cudaMallocHost(&ws->h_stage[k], kStageBytes));
-            if (!ws->stage_ev[k]) CK(cudaEventCreateWithFlags(&ws->stage_ev[k], cudaEventDisableTiming));
-        }
-        CopyPool& pool = CopyPool::get();
-        uint64_t ticket[3] = {0, 0, 0};
-        int64_t staged_cnt[3] = {0, 0, 0};
-        const int64_t nch = (nvalid + per - 1) / per;
-        auto finish = [&](int64_t j) -> ndi_status {           // chunk j has landed in its staging buffer: hand it to the pool
-            const int k = (int)(j % 3);
-            CK(cudaEventSynchronize(ws->stage_ev[k]));
-            ticket[k] = pool.submit((unsigned char*)he.out + (size_t)(j * per) * row, ws->h_stage[k], (size_t)staged_cnt[k] * row);
-            return NDI_OK;
-        };
-        ndi_status pst = NDI_OK;
-        for (int64_t i = 0; i < kFeedDepth && pst == NDI_OK; ++i) pst = feed(i, per);
-        int64_t launched = 0;                                    // chunks whose copy-out was issued
-        for (int64_t i = 0; i < nch && pst == NDI_OK; ++i) {
-            const int k = (int)(i % 3), sl = (int)(i & 1);
-            const int64_t lo = i * per;
-            int64_t cnt = nvalid - lo < per ? nvalid - lo : per;
-            const int64_t full = cnt;
-            if ((pst = fed(i, per, cnt, &cnt)) != NDI_OK) break;
-            if ((pst = feed(i + kFeedDepth, per)) != NDI_OK) break;
-            pool.wait(ticket[k]);                                // the host copy that last used this staging buffer is done
-            if (cnt > 0) {
-                if ((pst = grow(&ws->d_out[sl], &ws->d_out_cap[sl], (size_t)per * row)) != NDI_OK) break;
-                const void* c0 = (const unsigned char*)dq0 + (size_t)lo * he.es;
-                const void* c1 = dq1 ? (const unsigned char*)dq1 + (size_t)lo * he.es : nullptr;
-                if ((pst = launch(c0, c1, cnt, ws->d_out[sl], nullptr, ws->s[sl])) != NDI_OK) break;
-                cudaError_t ce = cudaMemcpyAsync(ws->h_stage[k], ws->d_out[sl], (size_t)cnt * row, cudaMemcpyDeviceToHost, ws->s[sl]);
-                if (ce == cudaSuccess) ce = cudaEventRecord(ws->stage_ev[k], ws->s[sl]);
-                if (ce != cudaSuccess) { pst = cuda_fail(ce, "staged copy"); break; }
-                staged_cnt[k] = cnt;
-                if (launched >= 1) pst = finish(launched - 1);
-                ++launched;
-            }
-            if (cnt < full) break;                               // the reference stopped inside this chunk
-        }
-        if (pst == NDI_OK && launched >= 1) pst = finish(launched - 1);
-        for (int k = 0; k < 3; ++k) pool.wait(ticket[k]);      // never leave with copies into the caller's memory in flight
-        if (pst != NDI_OK || streaming) drain();
-        return pst;
-    }
-    int64_t per_chunk = (int64_t)(kChunkBytes / row);
-    per_chunk = per_chunk < 32 ? 32 : (per_chunk & ~31ll);
-    const size_t chunk_bytes = (size_t)per_chunk * row;
-    int slot = 0;
     st = NDI_OK;
-    for (int64_t i = 0; i < kFeedDepth && st == NDI_OK; ++i) st = feed(i, per_chunk);
-    for (int64_t lo = 0, i = 0; lo < nvalid && st == NDI_OK; lo += per_chunk, ++i, slot ^= 1) {
-        int64_t cnt = nvalid - lo < per_chunk ? nvalid - lo : per_chunk;
-        const int64_t full = cnt;
-        if ((st = fed(i, per_chunk, cnt, &cnt)) != NDI_OK) break;
-        if ((st = feed(i + kFeedDepth, per_chunk)) != NDI_OK) break;
+    for (int64_t i = 0; i < kFeedDepth && st == NDI_OK; ++i) st = feed(i);
+    int64_t launched = 0;                                        // chunks whose copy-out was issued
+    for (int64_t i = 0; i * per < nvalid && st == NDI_OK; ++i) {
+        const int64_t lo = i * per, full = nvalid - lo < per ? nvalid - lo : per;
+        const int slot = (int)(i & 1), k = (int)(i % 3);
+        int64_t cnt;
+        if ((st = fed(i, full, &cnt)) != NDI_OK) break;
+        if ((st = feed(i + kFeedDepth)) != NDI_OK) break;
+        if (staged) pool->wait(ticket[k]);                       // the host copy that last used this staging buffer is done
         if (cnt > 0) {
             if ((st = grow(&ws->d_out[slot], &ws->d_out_cap[slot], chunk_bytes < total ? chunk_bytes : total)) != NDI_OK) break;
             const void* c0 = (const unsigned char*)dq0 + (size_t)lo * he.es;
             const void* c1 = dq1 ? (const unsigned char*)dq1 + (size_t)lo * he.es : nullptr;
             if ((st = launch(c0, c1, cnt, ws->d_out[slot], nullptr, ws->s[slot])) != NDI_OK) break;
-            cudaError_t ce = cudaMemcpyAsync((unsigned char*)he.out + (size_t)lo * row, ws->d_out[slot], (size_t)cnt * row,
-                                             cudaMemcpyDeviceToHost, ws->s[slot]);
-            if (ce != cudaSuccess) { st = cuda_fail(ce, "copy-out"); break; }
+            void* dst = staged ? (void*)ws->h_stage[k] : (void*)((unsigned char*)he.out + (size_t)lo * row);
+            cudaError_t ce = cudaMemcpyAsync(dst, ws->d_out[slot], (size_t)cnt * row, cudaMemcpyDeviceToHost, ws->s[slot]);
+            if (ce == cudaSuccess && staged) ce = cudaEventRecord(ws->stage_ev[k], ws->s[slot]);
+            if (ce != cudaSuccess) { st = cuda_fail(ce, staged ? "staged copy" : "copy-out"); break; }
+            staged_cnt[k] = cnt;
+            if (staged && launched >= 1) st = hand_over(launched - 1);
+            ++launched;
         }
         if (cnt < full) break;                                   // the reference stopped inside this chunk
     }
-    if (st != NDI_OK) { drain(); return st; }
+    if (staged) {
+        if (st == NDI_OK && launched >= 1) st = hand_over(launched - 1);
+        for (uint64_t t : ticket) pool->wait(t);
+    }
+    // never return while a copy from (or into) the caller's memory is in flight
+    if (st != NDI_OK) {
+        if (streaming) cudaStreamSynchronize(ws->s_in);
+        cudaStreamSynchronize(ws->s[0]); cudaStreamSynchronize(ws->s[1]);
+        return st;
+    }
     if (streaming) CK(cudaStreamSynchronize(ws->s_in));
     CK(cudaStreamSynchronize(ws->s[0]));
     CK(cudaStreamSynchronize(ws->s[1]));
+    return NDI_OK;
+}
+
+// one evaluation of a device-resident batch, for the _dev entry points and the host pipeline
+template <class T>
+ndi_status linear_on_device(const ndi_interp1d* h, const SearchCfg& sc, const T* q, int64_t nq, int extrapolate, T* out,
+                            unsigned long long* err, cudaStream_t s) {
+    CK(launch_interp1d_linear<T>((const T*)h->x, h->n, sc, (const T*)h->data, h->w, q, nq, extrapolate != 0, out, err,
+                                 h->fast_tables, (const T*)h->pair, s));
+    return NDI_OK;
+}
+template <class T>
+ndi_status cubic_on_device(const ndi_interp1d* h, const SearchCfg& sc, const T* q, int64_t nq, int extrap_mode, T* out,
+                           unsigned long long* err, cudaStream_t s) {
+    CK(launch_interp1d_cubic<T>((const T*)h->x, h->n, sc, (const T*)h->data, (const T*)h->a, (const T*)h->b, h->w, q, nq,
+                                extrap_mode, out, err, s));
     return NDI_OK;
 }
 
@@ -977,23 +967,20 @@ ndi_status ndi_interp1d_linear_dev(const ndi_interp1d* h, const void* q_dev, int
     return dispatch(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
         SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
-        CK(launch_interp1d_linear<T>((const T*)h->x, h->n, sc, (const T*)h->data, h->w, (const T*)q_dev, nq, extrapolate != 0,
-                                     (T*)out_dev, (unsigned long long*)err_word_dev, h->fast_tables, (const T*)h->pair, s));
-        return NDI_OK;
+        return linear_on_device<T>(h, sc, (const T*)q_dev, nq, extrapolate, (T*)out_dev, (unsigned long long*)err_word_dev, s);
     });
 }
 
-// one shard of a host batch (phase 0: the whole call; 1 / 2: see HostEval)
+// one block of a host batch (Phase::whole: the whole call)
 static ndi_status linear_host(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrapolate, void* out,
-                              uint64_t* word, int phase, int64_t nvalid) {
+                              uint64_t* word, Phase phase, int64_t nvalid) {
     HostEval he{h->device, elem_size(h->dtype), 1, h->w, {q, nullptr}, nq, out, phase, nvalid};
     return dispatch(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
         SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
         return run_host_eval(he,
             [&](const void* q0, const void*, int64_t cnt, void* o, unsigned long long* err, cudaStream_t s) -> ndi_status {
-                CK(launch_interp1d_linear<T>((const T*)h->x, h->n, sc, (const T*)h->data, h->w, (const T*)q0, cnt, extrapolate != 0, (T*)o, err, h->fast_tables, (const T*)h->pair, s));
-                return NDI_OK;
+                return linear_on_device<T>(h, sc, (const T*)q0, cnt, extrapolate, (T*)o, err, s);
             },
             [&](const void* q0, const void*, int64_t cnt, unsigned long long* err, cudaStream_t s) -> ndi_status {
                 CK(launch_validate_queries<T>((const T*)h->x, h->n, nullptr, 0, (const T*)q0, nullptr, cnt,
@@ -1014,7 +1001,7 @@ ndi_status ndi_interp1d_linear(const ndi_interp1d* h, const void* q, int64_t nq,
     if (first_bad) *first_bad = -1;
     ndi_status st = check_eval_args(h, q, nq, out); if (st != NDI_OK) return st;
     uint64_t word;
-    if ((st = linear_host(h, q, nq, extrapolate, out, &word, 0, 0)) != NDI_OK) return st;
+    if ((st = linear_host(h, q, nq, extrapolate, out, &word, Phase::whole, 0)) != NDI_OK) return st;
     return eval1d_status(word, extrapolate, first_bad);
 }
 
@@ -1066,9 +1053,7 @@ ndi_status ndi_interp1d_spline_build(ndi_interp1d* h, int32_t bc_kind, const int
     DeviceGuard g(h->device);
     ndi_status st; Workspace* ws = workspace(h->device, &st); if (!ws) return st;
     // which solve: the reference's elimination order, or the row-split (PCR + Thomas) build
-    static const long env_mode = env_long("NDI_BUILD_MODE", -1), env_levels = env_long("NDI_BUILD_LEVELS", -1);
-    const int mode = env_mode >= 0 ? (int)env_mode : h->build_mode;
-    const int want_levels = env_levels >= 0 ? (int)env_levels : h->build_levels;
+    const int mode = h->build_mode, want_levels = h->build_levels;
     int levels = 0;
     // AUTO: the partition build from kPartitionAutoRows rows on -- it beats the reference order (serial chains of n steps)
     // and the row-split build at every measured shape from there on, few long columns (4096 x 1024 f64: 0.11 against 0.91
@@ -1222,14 +1207,12 @@ ndi_status ndi_interp1d_cubic_dev(const ndi_interp1d* h, const void* q_dev, int6
     return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
         SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
-        CK(launch_interp1d_cubic<T>((const T*)h->x, h->n, sc, (const T*)h->data, (const T*)h->a, (const T*)h->b, h->w,
-                                    (const T*)q_dev, nq, extrap_mode, (T*)out_dev, (unsigned long long*)err_word_dev, s));
-        return NDI_OK;
+        return cubic_on_device<T>(h, sc, (const T*)q_dev, nq, extrap_mode, (T*)out_dev, (unsigned long long*)err_word_dev, s);
     });
 }
 
 static ndi_status cubic_host(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrap_mode, void* out,
-                             uint64_t* word, int phase, int64_t nvalid) {
+                             uint64_t* word, Phase phase, int64_t nvalid) {
     HostEval he{h->device, elem_size(h->dtype), 1, h->w, {q, nullptr}, nq, out, phase, nvalid};
     return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
@@ -1237,9 +1220,7 @@ static ndi_status cubic_host(const ndi_interp1d* h, const void* q, int64_t nq, i
         const int check = extrap_mode == NDI_EXTRAP_NO ? CHECK_IN_RANGE : (extrap_mode == NDI_EXTRAP_YES ? CHECK_NOT_NAN : CHECK_FINITE_IF_OUTSIDE);
         return run_host_eval(he,
             [&](const void* q0, const void*, int64_t cnt, void* o, unsigned long long* err, cudaStream_t s) -> ndi_status {
-                CK(launch_interp1d_cubic<T>((const T*)h->x, h->n, sc, (const T*)h->data, (const T*)h->a, (const T*)h->b, h->w,
-                                            (const T*)q0, cnt, extrap_mode, (T*)o, err, s));
-                return NDI_OK;
+                return cubic_on_device<T>(h, sc, (const T*)q0, cnt, extrap_mode, (T*)o, err, s);
             },
             [&](const void* q0, const void*, int64_t cnt, unsigned long long* err, cudaStream_t s) -> ndi_status {
                 CK(launch_validate_queries<T>((const T*)h->x, h->n, nullptr, 0, (const T*)q0, nullptr, cnt, check, err, s));
@@ -1255,7 +1236,7 @@ ndi_status ndi_interp1d_cubic(const ndi_interp1d* h, const void* q, int64_t nq, 
     if (!h->a) return fail(NDI_NO_SPLINE, "no spline coefficients: call ndi_interp1d_spline_build first");
     if (extrap_mode < 0 || extrap_mode > 2) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", extrap_mode);
     uint64_t word;
-    if ((st = cubic_host(h, q, nq, extrap_mode, out, &word, 0, 0)) != NDI_OK) return st;
+    if ((st = cubic_host(h, q, nq, extrap_mode, out, &word, Phase::whole, 0)) != NDI_OK) return st;
     return eval1d_status(word, extrap_mode, first_bad);
 }
 
@@ -1357,27 +1338,18 @@ ndi_status ndi_interp2d_device_ptrs(const ndi_interp2d* h, const void** x, const
     return NDI_OK;
 }
 ndi_status ndi_interp2d_clone_to_device(const ndi_interp2d* h, int32_t device, ndi_interp2d** out) {
-    if (!h || !out) return fail(NDI_INVALID_ARGUMENT, "null pointer");
-    *out = nullptr;
-    DeviceGuard g(device);
-    const size_t es = elem_size(h->dtype);
-    ndi_interp2d* c = new ndi_interp2d(*h);
-    c->device = device; c->owns_tables = true;
-    c->x = c->y = c->data = nullptr;
-    auto copy = [&](void** dst, const void* src, size_t bytes) -> ndi_status {
-        CK(cudaMalloc(dst, bytes));
-        CK(cudaMemcpyPeer(*dst, device, src, h->device, bytes));
-        return NDI_OK;
-    };
-    ndi_status st = copy(&c->x, h->x, (size_t)h->n * es);
-    if (st == NDI_OK) st = copy(&c->y, h->y, (size_t)h->m * es);
-    if (st == NDI_OK) st = copy(&c->data, h->data, (size_t)h->n * h->m * h->w * es);
-    c->aids_x = c->aids_y = GridAids{};
-    if (st == NDI_OK && !h->hint_x) st = build_aids(c->dtype, c->x, c->n, nullptr, &c->aids_x);
-    if (st == NDI_OK && !h->hint_y) st = build_aids(c->dtype, c->y, c->m, nullptr, &c->aids_y);
-    if (st != NDI_OK) { cudaFree(c->x); cudaFree(c->y); cudaFree(c->data); c->aids_x.release(); c->aids_y.release(); delete c; return st; }
-    *out = c;
-    return NDI_OK;
+    return clone_to_device(h, device, out, ndi_interp2d_destroy, [&](ndi_interp2d* c, auto& copy) {
+        const size_t es = elem_size(h->dtype);
+        c->owns_tables = true;
+        c->x = c->y = c->data = nullptr;
+        c->aids_x = c->aids_y = GridAids{};
+        ndi_status st = copy(&c->x, h->x, (size_t)h->n * es);
+        if (st == NDI_OK) st = copy(&c->y, h->y, (size_t)h->m * es);
+        if (st == NDI_OK) st = copy(&c->data, h->data, (size_t)h->n * h->m * h->w * es);
+        if (st == NDI_OK && !h->hint_x) st = build_aids(c->dtype, c->x, c->n, nullptr, &c->aids_x);
+        if (st == NDI_OK && !h->hint_y) st = build_aids(c->dtype, c->y, c->m, nullptr, &c->aids_y);
+        return st;
+    });
 }
 
 static void search2(const ndi_interp2d* h, size_t es, int64_t nq, SearchCfg* sx, SearchCfg* sy) {
@@ -1401,13 +1373,12 @@ namespace {
 // (C4: 0.59 -> 0.62 ms), where the scattered output stores and the binning passes cost what the
 // gathers save and the evaluation is bound by L1 wavefronts either way.
 bool want_binning(const ndi_interp2d* h, int64_t nq, size_t es, BandPlan* bp) {
-    static const long env_mode = env_long("NDI_BIN_MODE", -1), env_band_mb = env_long("NDI_BAND_MB", 16);
-    const int mode = env_mode >= 0 ? (int)env_mode : h->bin_mode;
-    if (mode == NDI_BIN_OFF || mode == NDI_BIN_SWEEP || nq < 2 || nq > 0xffffffffll) return false;
+    constexpr size_t kBandBytes = 16ull << 20;
+    if (h->bin_mode == NDI_BIN_OFF || h->bin_mode == NDI_BIN_SWEEP || nq < 2 || nq > 0xffffffffll) return false;
     const double table = (double)h->n * (double)h->m * (double)h->w * (double)es;
-    *bp = plan_bands(h->n, h->m, h->w, es, (size_t)env_band_mb << 20, h->band_rows);
+    *bp = plan_bands(h->n, h->m, h->w, es, kBandBytes, h->band_rows);
     if (bp->nbands < 2) return false;
-    if (mode == NDI_BIN_ON) return true;
+    if (h->bin_mode == NDI_BIN_ON) return true;
     const double resident = 0.4 * (double)device_info().l2_bytes;   // what random gathers keep of L2 (two partitions, output stream)
     const double seg = (double)(h->w * es);
     if (table <= resident || nq < (1 << 18) || seg < 64) return false;
@@ -1421,13 +1392,12 @@ bool want_binning(const ndi_interp2d* h, int64_t nq, size_t es, BandPlan* bp) {
 // C4's DRAM traffic from 3.14 to 1.36 GB as designed, but the compaction, the scattered 32-byte output rows and the lower
 // occupancy cost more than the DRAM time they save -- 0.580 ms against 0.537 ms for the direct kernel, which already runs
 // at the DRAM ceiling of its access pattern (profiles/r02/sweeps_and_probes.md).  The mode stays selectable
-// (NDI_BIN_SWEEP, or NDI_SWEEP_MODE=1 for measurements) and is covered by the parity tests.
+// (NDI_BIN_SWEEP through ndi_interp2d_set_binning) and is covered by the parity tests.
 bool want_sweeps(const ndi_interp2d* h, int64_t nq, size_t es, const void* out, SweepPlan* sp) {
-    static const long env_mode = env_long("NDI_SWEEP_MODE", -1), env_band_mb = env_long("NDI_SWEEP_MB", 32);
-    const bool forced = env_mode > 0 && h->bin_mode == NDI_BIN_AUTO && nq >= (1 << 18);
-    if (h->bin_mode != NDI_BIN_SWEEP && !forced) return false;
+    constexpr size_t kSweepBandBytes = 32ull << 20;
+    if (h->bin_mode != NDI_BIN_SWEEP) return false;
     if (!sweep_shape_ok(h->n, h->m, h->w, es, h->data, out, nq)) return false;
-    *sp = plan_sweeps(h->n, h->m, h->w, es, (size_t)env_band_mb << 20, h->bin_mode == NDI_BIN_SWEEP ? h->band_rows : 0);
+    *sp = plan_sweeps(h->n, h->m, h->w, es, kSweepBandBytes, h->band_rows);
     return true;
 }
 
@@ -1487,7 +1457,7 @@ ndi_status ndi_interp2d_bilinear_dev(const ndi_interp2d* h, const void* qx_dev, 
 }
 
 static ndi_status bilinear_host(const ndi_interp2d* h, const void* qx, const void* qy, int64_t nq, int32_t extrapolate,
-                                void* out, uint64_t* word, int phase, int64_t nvalid) {
+                                void* out, uint64_t* word, Phase phase, int64_t nvalid) {
     HostEval he{h->device, elem_size(h->dtype), 2, h->w, {qx, qy}, nq, out, phase, nvalid};
     return dispatch(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
@@ -1520,7 +1490,7 @@ ndi_status ndi_interp2d_bilinear(const ndi_interp2d* h, const void* qx, const vo
     ndi_status st = check_eval_args(h, qx, nq, out); if (st != NDI_OK) return st;
     if (nq > 0 && !qy) return fail(NDI_INVALID_ARGUMENT, "null pointer");
     uint64_t word;
-    if ((st = bilinear_host(h, qx, qy, nq, extrapolate, out, &word, 0, 0)) != NDI_OK) return st;
+    if ((st = bilinear_host(h, qx, qy, nq, extrapolate, out, &word, Phase::whole, 0)) != NDI_OK) return st;
     return eval2d_status(word, extrapolate, first_bad, bad_axis);
 }
 
@@ -1581,51 +1551,27 @@ private:
 // block k of nq queries cut into nd contiguous blocks whose starts are multiples of 32
 inline int64_t block_start(int64_t nq, int nd, int k) { return k >= nd ? nq : ((nq * k / nd) & ~31ll); }
 
-// the two-phase fan-out shared by the three strategies.  word_of(k, lo, cnt, phase, nvalid, &word) runs one block.
-// Returns the batch-wide error word (1-D: query index; 2-D: 2 * index + axis) through *word.
-template <class Block>
-ndi_status fan_out(Workers& pool, int nd, int64_t nq, int ncoord, Block&& block, uint64_t* word) {
-    std::vector<uint64_t> words((size_t)nd, NDI_ERR_WORD_NONE);
-    ndi_status st = pool.all([&](int k) -> ndi_status {
-        const int64_t lo = block_start(nq, nd, k), cnt = block_start(nq, nd, k + 1) - lo;
-        return cnt > 0 ? block(k, lo, cnt, 1, 0, &words[(size_t)k]) : NDI_OK;
-    });
-    if (st != NDI_OK) return st;
-    *word = NDI_ERR_WORD_NONE;
-    int64_t first = nq;                                          // rows before `first` are evaluated
-    for (int k = 0; k < nd; ++k) {
-        if (words[(size_t)k] == NDI_ERR_WORD_NONE) continue;
-        const int64_t lo = block_start(nq, nd, k);
-        const uint64_t w = ncoord > 1 ? words[(size_t)k] + 2 * (uint64_t)lo : words[(size_t)k] + (uint64_t)lo;
-        if (w < *word) *word = w;
-    }
-    if (*word != NDI_ERR_WORD_NONE) first = (int64_t)(ncoord > 1 ? *word >> 1 : *word);
-    return pool.all([&](int k) -> ndi_status {
-        const int64_t lo = block_start(nq, nd, k), cnt = block_start(nq, nd, k + 1) - lo;
-        const int64_t nvalid = first - lo < cnt ? first - lo : cnt;
-        uint64_t unused;
-        return (cnt > 0 && nvalid > 0) ? block(k, lo, cnt, 2, nvalid, &unused) : NDI_OK;
-    });
-}
-
 constexpr int64_t kGroupMinQueries = 1 << 15;       // below this a batch stays on the first device (latency path)
 
 }  // namespace
 
-struct ndi_interp1d_group {
-    std::vector<ndi_interp1d*> members; std::vector<char> owned;
+// the C ABI's ndi_interp1d_group and ndi_interp2d_group: members[k] lives on the k-th device of the group
+template <class H>
+struct Group {
+    std::vector<H*> members; std::vector<char> owned;   // owned: a clone, destroyed with the group
     Workers pool;
-    explicit ndi_interp1d_group(int n) : pool(n) {}
+    ndi_status (*destroy)(H*);
+    Group(int n, ndi_status (*destroy_handle)(H*)) : pool(n), destroy(destroy_handle) {}
+    ~Group() { for (size_t k = 0; k < members.size(); ++k) if (owned[k]) destroy(members[k]); }
 };
-struct ndi_interp2d_group {
-    std::vector<ndi_interp2d*> members; std::vector<char> owned;
-    Workers pool;
-    explicit ndi_interp2d_group(int n) : pool(n) {}
-};
+struct ndi_interp1d_group : Group<ndi_interp1d> { using Group::Group; };
+struct ndi_interp2d_group : Group<ndi_interp2d> { using Group::Group; };
 
-extern "C" {
+namespace {
 
-ndi_status ndi_interp1d_replicate(const ndi_interp1d* h, const int32_t* devices, int32_t ndev, ndi_interp1d_group** out) {
+template <class G, class H>
+ndi_status replicate(const H* h, const int32_t* devices, int32_t ndev, G** out, ndi_status (*clone)(const H*, int32_t, H**),
+                     ndi_status (*destroy)(H*)) {
     if (!h || !devices || !out || ndev < 1 || ndev > 64) return fail(NDI_INVALID_ARGUMENT, "need a handle and 1..64 devices");
     *out = nullptr;
     int count = 0; CK(cudaGetDeviceCount(&count));
@@ -1633,20 +1579,59 @@ ndi_status ndi_interp1d_replicate(const ndi_interp1d* h, const int32_t* devices,
         if (devices[k] < 0 || devices[k] >= count) return fail(NDI_INVALID_ARGUMENT, "device %d does not exist (%d visible)", devices[k], count);
         for (int j = 0; j < k; ++j) if (devices[j] == devices[k]) return fail(NDI_INVALID_ARGUMENT, "device %d listed twice", devices[k]);
     }
-    ndi_interp1d_group* g = new ndi_interp1d_group(ndev);
+    G* g = new G(ndev, destroy);
     for (int k = 0; k < ndev; ++k) {
-        if (devices[k] == h->device) { g->members.push_back(const_cast<ndi_interp1d*>(h)); g->owned.push_back(0); continue; }
-        ndi_interp1d* c = nullptr;
-        const ndi_status st = ndi_interp1d_clone_to_device(h, devices[k], &c);
-        if (st != NDI_OK) { ndi_interp1d_group_destroy(g); return st; }
+        if (devices[k] == h->device) { g->members.push_back(const_cast<H*>(h)); g->owned.push_back(0); continue; }
+        H* c = nullptr;
+        const ndi_status st = clone(h, devices[k], &c);
+        if (st != NDI_OK) { delete g; return st; }
         g->members.push_back(c); g->owned.push_back(1);
     }
     *out = g;
     return NDI_OK;
 }
+
+// One host call on a group.  A batch below kGroupMinQueries, or on a group of one device, is single(first member).
+// A larger one is checked by check(first member) and fanned out in two phases: block(member, lo, cnt, phase, nvalid,
+// &word) runs the block of queries [lo, lo + cnt) on its member's worker thread, first Phase::prepass on every block,
+// then Phase::evaluate on the rows before the batch-wide first failure.  status(word) turns that failure's error
+// word into the call's status.
+template <class H, class Single, class Check, class Block, class Status>
+ndi_status group_call(Group<H>* g, int64_t nq, int ncoord, Single&& single, Check&& check, Block&& block, Status&& status) {
+    if (!g || g->members.empty()) return fail(NDI_INVALID_ARGUMENT, "null group");
+    const int nd = (int)g->members.size();
+    if (nd == 1 || nq < kGroupMinQueries) return single(g->members[0]);
+    ndi_status st = check(g->members[0]); if (st != NDI_OK) return st;
+    std::vector<uint64_t> words((size_t)nd, NDI_ERR_WORD_NONE);
+    st = g->pool.all([&](int k) -> ndi_status {
+        const int64_t lo = block_start(nq, nd, k), cnt = block_start(nq, nd, k + 1) - lo;
+        return cnt > 0 ? block(g->members[(size_t)k], lo, cnt, Phase::prepass, 0, &words[(size_t)k]) : NDI_OK;
+    });
+    if (st != NDI_OK) return st;
+    uint64_t word = NDI_ERR_WORD_NONE;
+    for (int k = 0; k < nd; ++k) {
+        if (words[(size_t)k] == NDI_ERR_WORD_NONE) continue;
+        const uint64_t w = err_rebase(words[(size_t)k], ncoord, block_start(nq, nd, k));
+        if (w < word) word = w;
+    }
+    const int64_t first = word == NDI_ERR_WORD_NONE ? nq : err_query(word, ncoord);   // rows before `first` are evaluated
+    st = g->pool.all([&](int k) -> ndi_status {
+        const int64_t lo = block_start(nq, nd, k), cnt = block_start(nq, nd, k + 1) - lo;
+        const int64_t nvalid = first - lo < cnt ? first - lo : cnt;
+        uint64_t unused;
+        return (cnt > 0 && nvalid > 0) ? block(g->members[(size_t)k], lo, cnt, Phase::evaluate, nvalid, &unused) : NDI_OK;
+    });
+    return st != NDI_OK ? st : status(word);
+}
+
+}  // namespace
+
+extern "C" {
+
+ndi_status ndi_interp1d_replicate(const ndi_interp1d* h, const int32_t* devices, int32_t ndev, ndi_interp1d_group** out) {
+    return replicate(h, devices, ndev, out, ndi_interp1d_clone_to_device, ndi_interp1d_destroy);
+}
 ndi_status ndi_interp1d_group_destroy(ndi_interp1d_group* g) {
-    if (!g) return NDI_OK;
-    for (size_t k = 0; k < g->members.size(); ++k) if (g->owned[k]) ndi_interp1d_destroy(g->members[k]);
     delete g;
     return NDI_OK;
 }
@@ -1659,63 +1644,40 @@ ndi_status ndi_interp1d_group_size(const ndi_interp1d_group* g, int32_t* ndev) {
 ndi_status ndi_interp1d_group_linear(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrapolate, void* out,
                                      int64_t* first_bad) {
     if (first_bad) *first_bad = -1;
-    if (!g || g->members.empty()) return fail(NDI_INVALID_ARGUMENT, "null group");
-    const ndi_interp1d* h0 = g->members[0];
-    const int nd = (int)g->members.size();
-    if (nd == 1 || nq < kGroupMinQueries) return ndi_interp1d_linear(h0, q, nq, extrapolate, out, first_bad);
-    ndi_status st = check_eval_args(h0, q, nq, out); if (st != NDI_OK) return st;
-    const size_t es = elem_size(h0->dtype), row = (size_t)h0->w * es;
-    uint64_t word;
-    st = fan_out(g->pool, nd, nq, 1, [&](int k, int64_t lo, int64_t cnt, int phase, int64_t nvalid, uint64_t* w) {
-        return linear_host(g->members[(size_t)k], (const unsigned char*)q + (size_t)lo * es, cnt, extrapolate,
-                           (unsigned char*)out + (size_t)lo * row, w, phase, nvalid);
-    }, &word);
-    if (st != NDI_OK) return st;
-    return eval1d_status(word, extrapolate, first_bad);
+    return group_call(g, nq, 1,
+        [&](const ndi_interp1d* h0) { return ndi_interp1d_linear(h0, q, nq, extrapolate, out, first_bad); },
+        [&](const ndi_interp1d* h0) { return check_eval_args(h0, q, nq, out); },
+        [&](const ndi_interp1d* h, int64_t lo, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return linear_host(h, (const unsigned char*)q + (size_t)lo * es, cnt, extrapolate,
+                               (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid);
+        },
+        [&](uint64_t word) { return eval1d_status(word, extrapolate, first_bad); });
 }
 
 ndi_status ndi_interp1d_group_cubic(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrap_mode, void* out,
                                     int64_t* first_bad) {
     if (first_bad) *first_bad = -1;
-    if (!g || g->members.empty()) return fail(NDI_INVALID_ARGUMENT, "null group");
-    const ndi_interp1d* h0 = g->members[0];
-    const int nd = (int)g->members.size();
-    if (nd == 1 || nq < kGroupMinQueries) return ndi_interp1d_cubic(h0, q, nq, extrap_mode, out, first_bad);
-    ndi_status st = check_eval_args(h0, q, nq, out); if (st != NDI_OK) return st;
-    if (!h0->a) return fail(NDI_NO_SPLINE, "no spline coefficients: build the spline before ndi_interp1d_replicate");
-    if (extrap_mode < 0 || extrap_mode > 2) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", extrap_mode);
-    const size_t es = elem_size(h0->dtype), row = (size_t)h0->w * es;
-    uint64_t word;
-    st = fan_out(g->pool, nd, nq, 1, [&](int k, int64_t lo, int64_t cnt, int phase, int64_t nvalid, uint64_t* w) {
-        return cubic_host(g->members[(size_t)k], (const unsigned char*)q + (size_t)lo * es, cnt, extrap_mode,
-                          (unsigned char*)out + (size_t)lo * row, w, phase, nvalid);
-    }, &word);
-    if (st != NDI_OK) return st;
-    return eval1d_status(word, extrap_mode, first_bad);
+    return group_call(g, nq, 1,
+        [&](const ndi_interp1d* h0) { return ndi_interp1d_cubic(h0, q, nq, extrap_mode, out, first_bad); },
+        [&](const ndi_interp1d* h0) {
+            ndi_status st = check_eval_args(h0, q, nq, out); if (st != NDI_OK) return st;
+            if (!h0->a) return fail(NDI_NO_SPLINE, "no spline coefficients: build the spline before ndi_interp1d_replicate");
+            if (extrap_mode < 0 || extrap_mode > 2) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", extrap_mode);
+            return NDI_OK;
+        },
+        [&](const ndi_interp1d* h, int64_t lo, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return cubic_host(h, (const unsigned char*)q + (size_t)lo * es, cnt, extrap_mode,
+                              (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid);
+        },
+        [&](uint64_t word) { return eval1d_status(word, extrap_mode, first_bad); });
 }
 
 ndi_status ndi_interp2d_replicate(const ndi_interp2d* h, const int32_t* devices, int32_t ndev, ndi_interp2d_group** out) {
-    if (!h || !devices || !out || ndev < 1 || ndev > 64) return fail(NDI_INVALID_ARGUMENT, "need a handle and 1..64 devices");
-    *out = nullptr;
-    int count = 0; CK(cudaGetDeviceCount(&count));
-    for (int k = 0; k < ndev; ++k) {
-        if (devices[k] < 0 || devices[k] >= count) return fail(NDI_INVALID_ARGUMENT, "device %d does not exist (%d visible)", devices[k], count);
-        for (int j = 0; j < k; ++j) if (devices[j] == devices[k]) return fail(NDI_INVALID_ARGUMENT, "device %d listed twice", devices[k]);
-    }
-    ndi_interp2d_group* g = new ndi_interp2d_group(ndev);
-    for (int k = 0; k < ndev; ++k) {
-        if (devices[k] == h->device) { g->members.push_back(const_cast<ndi_interp2d*>(h)); g->owned.push_back(0); continue; }
-        ndi_interp2d* c = nullptr;
-        const ndi_status st = ndi_interp2d_clone_to_device(h, devices[k], &c);
-        if (st != NDI_OK) { ndi_interp2d_group_destroy(g); return st; }
-        g->members.push_back(c); g->owned.push_back(1);
-    }
-    *out = g;
-    return NDI_OK;
+    return replicate(h, devices, ndev, out, ndi_interp2d_clone_to_device, ndi_interp2d_destroy);
 }
 ndi_status ndi_interp2d_group_destroy(ndi_interp2d_group* g) {
-    if (!g) return NDI_OK;
-    for (size_t k = 0; k < g->members.size(); ++k) if (g->owned[k]) ndi_interp2d_destroy(g->members[k]);
     delete g;
     return NDI_OK;
 }
@@ -1724,20 +1686,18 @@ ndi_status ndi_interp2d_group_bilinear(ndi_interp2d_group* g, const void* qx, co
                                        void* out, int64_t* first_bad, int32_t* bad_axis) {
     if (first_bad) *first_bad = -1;
     if (bad_axis) *bad_axis = -1;
-    if (!g || g->members.empty()) return fail(NDI_INVALID_ARGUMENT, "null group");
-    const ndi_interp2d* h0 = g->members[0];
-    const int nd = (int)g->members.size();
-    if (nd == 1 || nq < kGroupMinQueries) return ndi_interp2d_bilinear(h0, qx, qy, nq, extrapolate, out, first_bad, bad_axis);
-    ndi_status st = check_eval_args(h0, qx, nq, out); if (st != NDI_OK) return st;
-    if (!qy) return fail(NDI_INVALID_ARGUMENT, "null pointer");
-    const size_t es = elem_size(h0->dtype), row = (size_t)h0->w * es;
-    uint64_t word;
-    st = fan_out(g->pool, nd, nq, 2, [&](int k, int64_t lo, int64_t cnt, int phase, int64_t nvalid, uint64_t* w) {
-        return bilinear_host(g->members[(size_t)k], (const unsigned char*)qx + (size_t)lo * es, (const unsigned char*)qy + (size_t)lo * es,
-                             cnt, extrapolate, (unsigned char*)out + (size_t)lo * row, w, phase, nvalid);
-    }, &word);
-    if (st != NDI_OK) return st;
-    return eval2d_status(word, extrapolate, first_bad, bad_axis);
+    return group_call(g, nq, 2,
+        [&](const ndi_interp2d* h0) { return ndi_interp2d_bilinear(h0, qx, qy, nq, extrapolate, out, first_bad, bad_axis); },
+        [&](const ndi_interp2d* h0) {
+            ndi_status st = check_eval_args(h0, qx, nq, out); if (st != NDI_OK) return st;
+            return qy ? NDI_OK : fail(NDI_INVALID_ARGUMENT, "null pointer");
+        },
+        [&](const ndi_interp2d* h, int64_t lo, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return bilinear_host(h, (const unsigned char*)qx + (size_t)lo * es, (const unsigned char*)qy + (size_t)lo * es, cnt,
+                                 extrapolate, (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid);
+        },
+        [&](uint64_t word) { return eval2d_status(word, extrapolate, first_bad, bad_axis); });
 }
 
 }  // extern "C"
