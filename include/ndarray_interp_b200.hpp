@@ -292,6 +292,9 @@ public:
     bool uses_device() const override { return true; }
     void interp_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows) const override;
     void interp_into(const Interp1D<T>& ip, ArrayViewMut<T> target, T x) const override;      // linear.rs:73-98
+    // NOT in the reference (ndi_interp1d_linear_deriv): slope of each query's interval, interp_batch_into's query
+    // handling and errors; order must be 1 (std::invalid_argument otherwise)
+    void deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const;
 private:
     bool extrapolate_ = false;
 };
@@ -343,6 +346,9 @@ public:
     void bind(const Interp1D<T>& ip) const override;         // CubicSpline::calc_coefficients (:310-368) on the device
     void interp_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows) const override;
     void interp_into(const Interp1D<T>& ip, ArrayViewMut<T> target, T x) const override;      // :791-830
+    // NOT in the reference (ndi_interp1d_cubic_deriv): derivative of order 1 or 2 (std::invalid_argument otherwise),
+    // interp_batch_into's query handling and errors
+    void deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const;
     // (a, b) copied back from the device: shape (n-1, ...data.shape[1..])
     std::pair<Array<T>, Array<T>> coefficients(const Interp1D<T>& ip) const;
 private:
@@ -414,15 +420,34 @@ public:
     }
     // :272-324; one launch for the whole batch, whatever the query rank
     void interp_array_into(const ArrayView<T>& xs, ArrayViewMut<T> buffer) const {
-        const std::vector<size_t> expect = buffer_shape(xs.shape);
-        if (buffer.shape != expect)
-            throw Panic("ShapeError/IncompatibleShape: incompatible shapes expected: " + detail::shape_str(expect) + ", got: " + detail::shape_str(buffer.shape));
-        const std::vector<T> q = xs.to_vector();
-        if (buffer.c_contiguous()) { strategy_->interp_batch_into(*this, q.data(), q.size(), buffer.ptr); return; }
-        std::vector<T> rows = buffer.view().to_vector();       // rows the reference would leave untouched stay as they are
-        try { strategy_->interp_batch_into(*this, q.data(), q.size(), rows.data()); }
-        catch (...) { buffer.assign_rows(rows); throw; }
-        buffer.assign_rows(rows);
+        array_into(xs, buffer, [&](const T* q, size_t nq, T* rows) { strategy_->interp_batch_into(*this, q, nq, rows); });
+    }
+
+    // ---- derivatives: NOT in the reference (built-in strategies: Linear order 1, CubicSpline order 1 or 2) ----------
+    Array<T> interp_deriv(T x, int order = 1) const {
+        Array<T> target = Array<T>::zeros(trailing_shape());
+        std::vector<size_t> one_row = trailing_shape();
+        one_row.insert(one_row.begin(), 1);
+        std::vector<std::ptrdiff_t> st(one_row.size(), 1);
+        for (size_t i = one_row.size(); i-- > 1;) st[i - 1] = st[i] * (std::ptrdiff_t)one_row[i];
+        interp_array_deriv_into(ArrayView<T>{&x, {1}, {1}}, ArrayViewMut<T>{target.data(), one_row, st}, order);
+        return target;
+    }
+    Array<T> interp_array_deriv(const ArrayView<T>& xs, int order = 1) const {
+        Array<T> ys = Array<T>::zeros(buffer_shape(xs.shape));
+        interp_array_deriv_into(xs, ys.view_mut(), order);
+        return ys;
+    }
+    // buffer shape, errors and untouched rows after a failing query as interp_array_into
+    void interp_array_deriv_into(const ArrayView<T>& xs, ArrayViewMut<T> buffer, int order = 1) const {
+        const auto* lin = dynamic_cast<const Linear<T>*>(strategy_.get());
+        const auto* cub = dynamic_cast<const CubicSplineStrategy<T>*>(strategy_.get());
+        if (!lin && !cub) throw std::invalid_argument("derivatives are computed by the built-in strategies (Linear, CubicSpline) only");
+        if (order != 1 && (lin || order != 2)) throw std::invalid_argument("no derivative of order " + std::to_string(order) + " for this strategy");
+        array_into(xs, buffer, [&](const T* q, size_t nq, T* rows) {
+            if (lin) lin->deriv_batch_into(*this, q, nq, rows, order);
+            else cub->deriv_batch_into(*this, q, nq, rows, order);
+        });
     }
 
     // accessors strategies may call back (:371-386)
@@ -453,6 +478,18 @@ public:
 
 private:
     friend class Interp1DBuilder<T>;
+    template <class Batch>
+    void array_into(const ArrayView<T>& xs, ArrayViewMut<T> buffer, Batch&& batch) const {
+        const std::vector<size_t> expect = buffer_shape(xs.shape);
+        if (buffer.shape != expect)
+            throw Panic("ShapeError/IncompatibleShape: incompatible shapes expected: " + detail::shape_str(expect) + ", got: " + detail::shape_str(buffer.shape));
+        const std::vector<T> q = xs.to_vector();
+        if (buffer.c_contiguous()) { batch(q.data(), q.size(), buffer.ptr); return; }
+        std::vector<T> rows = buffer.view().to_vector();       // rows the reference would leave untouched stay as they are
+        try { batch(q.data(), q.size(), rows.data()); }
+        catch (...) { buffer.assign_rows(rows); throw; }
+        buffer.assign_rows(rows);
+    }
     Interp1D(Array<T> x, Array<T> data, std::shared_ptr<const Interp1DStrategy<T>> s) : x_(std::move(x)), data_(std::move(data)), strategy_(std::move(s)) {
         strategy_->bind(*this);
     }
@@ -526,6 +563,14 @@ void Linear<T>::interp_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq,
 }
 template <class T>
 void Linear<T>::interp_into(const Interp1D<T>& ip, ArrayViewMut<T> target, T x) const { detail::single_into<T>(*this, ip, target, x); }
+template <class T>
+void Linear<T>::deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const {
+    if (order != 1) throw std::invalid_argument("Linear has only a first derivative, got order " + std::to_string(order));
+    int64_t bad = -1;
+    const ndi_status st = ndi_interp1d_linear_deriv(ip.handle(), xs, (int64_t)nq, extrapolate_, out_rows, &bad);
+    detail::check(st);
+    if (st != NDI_OK) detail::raise_eval<T>(st, xs, bad, "x");
+}
 
 template <class T>
 void CubicSplineStrategy<T>::bind(const Interp1D<T>& ip) const {
@@ -549,6 +594,14 @@ void CubicSplineStrategy<T>::interp_batch_into(const Interp1D<T>& ip, const T* x
 }
 template <class T>
 void CubicSplineStrategy<T>::interp_into(const Interp1D<T>& ip, ArrayViewMut<T> target, T x) const { detail::single_into<T>(*this, ip, target, x); }
+template <class T>
+void CubicSplineStrategy<T>::deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const {
+    if (order != 1 && order != 2) throw std::invalid_argument("CubicSpline derivative order must be 1 or 2, got " + std::to_string(order));
+    int64_t bad = -1;
+    const ndi_status st = ndi_interp1d_cubic_deriv(ip.handle(), xs, (int64_t)nq, mode_, order, out_rows, &bad);
+    detail::check(st);
+    if (st != NDI_OK) detail::raise_eval<T>(st, xs, bad, "x");
+}
 template <class T>
 int CubicSplineStrategy<T>::rowsplit_levels(const Interp1D<T>& ip) const {
     int32_t lv = -1;

@@ -216,6 +216,27 @@ ndi_status ndi_interp1d_cubic(const ndi_interp1d* h, const void* q, int64_t nq, 
 ndi_status ndi_interp1d_cubic_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrap_mode,
                                   void* out_dev, uint64_t* err_word_dev, void* stream);
 
+/* ---- derivatives (NOT in the reference; scipy.interpolate.CubicSpline.__call__(x, nu)) ------------ */
+/* Query handling is exactly that of the value call for the same handle and mode: the same range check, periodic
+ * wrap (NDI_EXTRAP_PERIODIC), NaN handling, lower-index search, error statuses and untouched rows.  So a query on
+ * an interior knot x[i] gets the derivative of interval i (the right-hand one, as scipy), a query at x[n-1] that of
+ * interval n-2 at t = 1, and an extrapolated query that of the edge interval's polynomial.
+ * Cubic spline, order 1 or 2 (any other order: NDI_INVALID_ARGUMENT; order 0 is ndi_interp1d_cubic), with i, t, a, b
+ * as in the value call, h = x[i+1] - x[i], every operation rounded on its own:
+ *     cur = a (1-t) + b t,  ba = b - a
+ *     order 1:  (((y[i+1] - y[i]) + ((1-t) - t) cur) + (t (1-t)) ba) / h
+ *     order 2:  ((2 (((1-t) - t) ba - cur)) / h) / h
+ * Linear, order 1 only: (y[i+1] - y[i]) / (x[i+1] - x[i]), the slope term of linear.rs:29-36 in the handle's dtype
+ * (integers wrap and truncate like the value call; a zero quotient keeps IEEE's sign). */
+ndi_status ndi_interp1d_cubic_deriv(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrap_mode,
+                                    int32_t order, void* out, int64_t* first_bad);
+ndi_status ndi_interp1d_cubic_deriv_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrap_mode,
+                                        int32_t order, void* out_dev, uint64_t* err_word_dev, void* stream);
+ndi_status ndi_interp1d_linear_deriv(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrapolate,
+                                     void* out, int64_t* first_bad);
+ndi_status ndi_interp1d_linear_deriv_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrapolate,
+                                         void* out_dev, uint64_t* err_word_dev, void* stream);
+
 /* ---- src/interp2d ------------------------------------------------------------------------ */
 /* Interp2DBuilder::build data upload (interp2d/mod.rs:468-518).  x: n, y: m, data: (n, m, w).
  * NDI_NOT_MONOTONIC reports the failing axis in the message ("x-axis" before "y-axis"). */
@@ -270,6 +291,11 @@ ndi_status ndi_interp1d_group_linear(ndi_interp1d_group* g, const void* q, int64
                                      int64_t* first_bad);
 ndi_status ndi_interp1d_group_cubic(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrap_mode, void* out,
                                     int64_t* first_bad);
+/* the derivative calls above, on a group */
+ndi_status ndi_interp1d_group_linear_deriv(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrapolate,
+                                           void* out, int64_t* first_bad);
+ndi_status ndi_interp1d_group_cubic_deriv(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrap_mode,
+                                          int32_t order, void* out, int64_t* first_bad);
 ndi_status ndi_interp2d_replicate(const ndi_interp2d* h, const int32_t* devices, int32_t ndev, ndi_interp2d_group** out);
 ndi_status ndi_interp2d_group_destroy(ndi_interp2d_group* g);
 ndi_status ndi_interp2d_group_bilinear(ndi_interp2d_group* g, const void* qx, const void* qy, int64_t nq,

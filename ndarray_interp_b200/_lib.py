@@ -56,6 +56,10 @@ SIGNATURES = {
     "ndi_interp1d_spline_set_coeffs": (_i32, [_vp, _vp, _vp, _u32]),
     "ndi_interp1d_cubic": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
     "ndi_interp1d_cubic_dev": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "ndi_interp1d_cubic_deriv": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _pi64]),
+    "ndi_interp1d_cubic_deriv_dev": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
+    "ndi_interp1d_linear_deriv": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
+    "ndi_interp1d_linear_deriv_dev": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
     "ndi_interp2d_create": (_i32, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _u32, C.POINTER(_vp)]),
     "ndi_interp2d_create_strided": (_i32, [_i32, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _u32,
                                            C.POINTER(_vp)]),
@@ -74,6 +78,8 @@ SIGNATURES = {
     "ndi_interp1d_group_size": (_i32, [_vp, _pi32]),
     "ndi_interp1d_group_linear": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
     "ndi_interp1d_group_cubic": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
+    "ndi_interp1d_group_linear_deriv": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
+    "ndi_interp1d_group_cubic_deriv": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _pi64]),
     "ndi_interp2d_replicate": (_i32, [_vp, _pi32, _i32, C.POINTER(_vp)]),
     "ndi_interp2d_group_destroy": (_i32, [_vp]),
     "ndi_interp2d_group_bilinear": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),

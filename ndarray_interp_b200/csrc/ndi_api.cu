@@ -947,6 +947,20 @@ ndi_status cubic_on_device(const ndi_interp1d* h, const SearchCfg& sc, const T* 
                                 extrap_mode, out, err, s));
     return NDI_OK;
 }
+// derivatives (NOT in the reference): the same query handling, K3d / K5d per element
+template <class T>
+ndi_status linear_deriv_on_device(const ndi_interp1d* h, const SearchCfg& sc, const T* q, int64_t nq, int extrapolate, T* out,
+                                  unsigned long long* err, cudaStream_t s) {
+    CK(launch_interp1d_linear_slope<T>((const T*)h->x, h->n, sc, (const T*)h->data, h->w, q, nq, extrapolate != 0, out, err, s));
+    return NDI_OK;
+}
+template <class T>
+ndi_status cubic_deriv_on_device(const ndi_interp1d* h, const SearchCfg& sc, const T* q, int64_t nq, int extrap_mode, int order,
+                                 T* out, unsigned long long* err, cudaStream_t s) {
+    CK(launch_interp1d_cubic_deriv<T>((const T*)h->x, h->n, sc, (const T*)h->data, (const T*)h->a, (const T*)h->b, h->w, q, nq,
+                                      extrap_mode, order, out, err, s));
+    return NDI_OK;
+}
 
 }  // namespace
 
@@ -971,15 +985,28 @@ ndi_status ndi_interp1d_linear_dev(const ndi_interp1d* h, const void* q_dev, int
     });
 }
 
-// one block of a host batch (Phase::whole: the whole call)
+ndi_status ndi_interp1d_linear_deriv_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrapolate,
+                                         void* out_dev, uint64_t* err_word_dev, void* stream) {
+    ndi_status st = check_eval_args(h, q_dev, nq, out_dev); if (st != NDI_OK) return st;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (err_word_dev) CK(cudaMemsetAsync(err_word_dev, 0xff, sizeof(uint64_t), s));
+    return dispatch(h->dtype, [&](auto tag) -> ndi_status {
+        using T = decltype(tag);
+        SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
+        return linear_deriv_on_device<T>(h, sc, (const T*)q_dev, nq, extrapolate, (T*)out_dev, (unsigned long long*)err_word_dev, s);
+    });
+}
+
+// one block of a host batch (Phase::whole: the whole call); slope: the derivative instead of the values
 static ndi_status linear_host(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrapolate, void* out,
-                              uint64_t* word, Phase phase, int64_t nvalid) {
+                              uint64_t* word, Phase phase, int64_t nvalid, bool slope = false) {
     HostEval he{h->device, elem_size(h->dtype), 1, h->w, {q, nullptr}, nq, out, phase, nvalid};
     return dispatch(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
         SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
         return run_host_eval(he,
             [&](const void* q0, const void*, int64_t cnt, void* o, unsigned long long* err, cudaStream_t s) -> ndi_status {
+                if (slope) return linear_deriv_on_device<T>(h, sc, (const T*)q0, cnt, extrapolate, (T*)o, err, s);
                 return linear_on_device<T>(h, sc, (const T*)q0, cnt, extrapolate, (T*)o, err, s);
             },
             [&](const void* q0, const void*, int64_t cnt, unsigned long long* err, cudaStream_t s) -> ndi_status {
@@ -1002,6 +1029,15 @@ ndi_status ndi_interp1d_linear(const ndi_interp1d* h, const void* q, int64_t nq,
     ndi_status st = check_eval_args(h, q, nq, out); if (st != NDI_OK) return st;
     uint64_t word;
     if ((st = linear_host(h, q, nq, extrapolate, out, &word, Phase::whole, 0)) != NDI_OK) return st;
+    return eval1d_status(word, extrapolate, first_bad);
+}
+
+ndi_status ndi_interp1d_linear_deriv(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrapolate, void* out,
+                                     int64_t* first_bad) {
+    if (first_bad) *first_bad = -1;
+    ndi_status st = check_eval_args(h, q, nq, out); if (st != NDI_OK) return st;
+    uint64_t word;
+    if ((st = linear_host(h, q, nq, extrapolate, out, &word, Phase::whole, 0, true)) != NDI_OK) return st;
     return eval1d_status(word, extrapolate, first_bad);
 }
 
@@ -1211,8 +1247,31 @@ ndi_status ndi_interp1d_cubic_dev(const ndi_interp1d* h, const void* q_dev, int6
     });
 }
 
+// derivative calls: the argument checks of the value call, then the order (order 0 is ndi_interp1d_cubic itself)
+static ndi_status check_cubic_deriv_args(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrap_mode, int32_t order,
+                                         const void* out) {
+    ndi_status st = check_eval_args(h, q, nq, out); if (st != NDI_OK) return st;
+    if (!h->a) return fail(NDI_NO_SPLINE, "no spline coefficients: call ndi_interp1d_spline_build first");
+    if (extrap_mode < 0 || extrap_mode > 2) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", extrap_mode);
+    if (order != 1 && order != 2) return fail(NDI_INVALID_ARGUMENT, "derivative order must be 1 or 2, got %d", order);
+    return NDI_OK;
+}
+
+ndi_status ndi_interp1d_cubic_deriv_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrap_mode, int32_t order,
+                                        void* out_dev, uint64_t* err_word_dev, void* stream) {
+    ndi_status st = check_cubic_deriv_args(h, q_dev, nq, extrap_mode, order, out_dev); if (st != NDI_OK) return st;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (err_word_dev) CK(cudaMemsetAsync(err_word_dev, 0xff, sizeof(uint64_t), s));
+    return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
+        using T = decltype(tag);
+        SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
+        return cubic_deriv_on_device<T>(h, sc, (const T*)q_dev, nq, extrap_mode, order, (T*)out_dev, (unsigned long long*)err_word_dev, s);
+    });
+}
+
+// order 0: the values; 1, 2: the derivatives
 static ndi_status cubic_host(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrap_mode, void* out,
-                             uint64_t* word, Phase phase, int64_t nvalid) {
+                             uint64_t* word, Phase phase, int64_t nvalid, int32_t order = 0) {
     HostEval he{h->device, elem_size(h->dtype), 1, h->w, {q, nullptr}, nq, out, phase, nvalid};
     return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
         using T = decltype(tag);
@@ -1220,6 +1279,7 @@ static ndi_status cubic_host(const ndi_interp1d* h, const void* q, int64_t nq, i
         const int check = extrap_mode == NDI_EXTRAP_NO ? CHECK_IN_RANGE : (extrap_mode == NDI_EXTRAP_YES ? CHECK_NOT_NAN : CHECK_FINITE_IF_OUTSIDE);
         return run_host_eval(he,
             [&](const void* q0, const void*, int64_t cnt, void* o, unsigned long long* err, cudaStream_t s) -> ndi_status {
+                if (order) return cubic_deriv_on_device<T>(h, sc, (const T*)q0, cnt, extrap_mode, order, (T*)o, err, s);
                 return cubic_on_device<T>(h, sc, (const T*)q0, cnt, extrap_mode, (T*)o, err, s);
             },
             [&](const void* q0, const void*, int64_t cnt, unsigned long long* err, cudaStream_t s) -> ndi_status {
@@ -1237,6 +1297,15 @@ ndi_status ndi_interp1d_cubic(const ndi_interp1d* h, const void* q, int64_t nq, 
     if (extrap_mode < 0 || extrap_mode > 2) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", extrap_mode);
     uint64_t word;
     if ((st = cubic_host(h, q, nq, extrap_mode, out, &word, Phase::whole, 0)) != NDI_OK) return st;
+    return eval1d_status(word, extrap_mode, first_bad);
+}
+
+ndi_status ndi_interp1d_cubic_deriv(const ndi_interp1d* h, const void* q, int64_t nq, int32_t extrap_mode, int32_t order,
+                                    void* out, int64_t* first_bad) {
+    if (first_bad) *first_bad = -1;
+    ndi_status st = check_cubic_deriv_args(h, q, nq, extrap_mode, order, out); if (st != NDI_OK) return st;
+    uint64_t word;
+    if ((st = cubic_host(h, q, nq, extrap_mode, out, &word, Phase::whole, 0, order)) != NDI_OK) return st;
     return eval1d_status(word, extrap_mode, first_bad);
 }
 
@@ -1670,6 +1739,34 @@ ndi_status ndi_interp1d_group_cubic(ndi_interp1d_group* g, const void* q, int64_
             const size_t es = elem_size(h->dtype);
             return cubic_host(h, (const unsigned char*)q + (size_t)lo * es, cnt, extrap_mode,
                               (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid);
+        },
+        [&](uint64_t word) { return eval1d_status(word, extrap_mode, first_bad); });
+}
+
+ndi_status ndi_interp1d_group_linear_deriv(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrapolate, void* out,
+                                           int64_t* first_bad) {
+    if (first_bad) *first_bad = -1;
+    return group_call(g, nq, 1,
+        [&](const ndi_interp1d* h0) { return ndi_interp1d_linear_deriv(h0, q, nq, extrapolate, out, first_bad); },
+        [&](const ndi_interp1d* h0) { return check_eval_args(h0, q, nq, out); },
+        [&](const ndi_interp1d* h, int64_t lo, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return linear_host(h, (const unsigned char*)q + (size_t)lo * es, cnt, extrapolate,
+                               (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid, true);
+        },
+        [&](uint64_t word) { return eval1d_status(word, extrapolate, first_bad); });
+}
+
+ndi_status ndi_interp1d_group_cubic_deriv(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrap_mode, int32_t order,
+                                          void* out, int64_t* first_bad) {
+    if (first_bad) *first_bad = -1;
+    return group_call(g, nq, 1,
+        [&](const ndi_interp1d* h0) { return ndi_interp1d_cubic_deriv(h0, q, nq, extrap_mode, order, out, first_bad); },
+        [&](const ndi_interp1d* h0) { return check_cubic_deriv_args(h0, q, nq, extrap_mode, order, out); },
+        [&](const ndi_interp1d* h, int64_t lo, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return cubic_host(h, (const unsigned char*)q + (size_t)lo * es, cnt, extrap_mode,
+                              (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid, order);
         },
         [&](uint64_t word) { return eval1d_status(word, extrap_mode, first_bad); });
 }

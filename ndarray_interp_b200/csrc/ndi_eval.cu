@@ -527,6 +527,268 @@ __global__ void __launch_bounds__(kBlock, (sizeof(T) == 4 && LPQ < 32) ? NDI_THI
 }
 
 // ------------------------------------------------------------------------------------------------
+// K5d: first / second derivative of the cubic spline (NOT in the reference; scipy's CubicSpline(x, nu))
+// ------------------------------------------------------------------------------------------------
+// The exact derivatives of the value form (1-t) yl + t yr + t (1-t) (a (1-t) + b t) with t = (x - xl) / h, h = xr - xl:
+//     cur = a (1-t) + b t,  ba = b - a
+//     d1  = (((yr - yl) + ((1-t) - t) cur) + (t (1-t)) ba) / h
+//     d2  = ((2 (((1-t) - t) ba - cur)) / h) / h
+// every operation rounded on its own.  Query handling (range check, periodic wrap, NaN, lower index, t) is K5's.
+// The divisor h is the same for every column of a query: its reciprocal is formed once per query (Hoisted<T>::rcp)
+// and every quotient is finished with the hoisted sequence, which falls back to the IEEE division wherever it could
+// differ from it -- bit-identical to a true division per element.
+__device__ __forceinline__ F2 sub_halves(F2 p, F2 z) { return F2{__fsub_rn(p.lo, z.lo), __fsub_rn(p.hi, z.hi)}; }
+
+template <class T, int ORDER>
+__device__ __forceinline__ T cubic_deriv_point(T num, T h, T r) {
+    if constexpr (ORDER == 1) return Hoisted<T>::div(num, h, r);
+    else return Hoisted<T>::div(Hoisted<T>::div(num, h, r), h, r);
+}
+
+template <class T, int V, int ORDER>
+__device__ __forceinline__ Vec<T, V> cubic_deriv_vec(const Vec<T, V>& yl, const Vec<T, V>& yr, const Vec<T, V>& al,
+                                                     const Vec<T, V>& bl, T t, T omt, T h, T r) {
+    const T dmt = Ar<T>::sub(omt, t), tt = Ar<T>::mul(t, omt);
+    const T two = (T)2;
+    Vec<T, V> res;
+    if constexpr (std::is_same<T, float>::value && NDI_F32X2 && V % 2 == 0) {
+        const F2 t2 = F2::both(t), o2 = F2::both(omt), d2 = F2::both(dmt), tt2 = F2::both(tt), two2 = F2::both(two);
+#pragma unroll
+        for (int e = 0; e < V; e += 2) {
+            const F2 l{yl.v[e], yl.v[e + 1]}, rr{yr.v[e], yr.v[e + 1]}, a{al.v[e], al.v[e + 1]}, b{bl.v[e], bl.v[e + 1]};
+            const F2 cur = add_halves(mul2(a, o2), mul2(b, t2));       // sums and differences of products: per half
+            const F2 ba = sub2(b, a);
+            F2 num;
+            if constexpr (ORDER == 1) num = add_halves(mul2(tt2, ba), add_halves(mul2(d2, cur), sub2(rr, l)));
+            else num = mul2(two2, sub_halves(mul2(d2, ba), cur));
+            res.v[e] = cubic_deriv_point<T, ORDER>(num.lo, h, r);
+            res.v[e + 1] = cubic_deriv_point<T, ORDER>(num.hi, h, r);
+        }
+        return res;
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+        const T cur = Ar<T>::add(Ar<T>::mul(al.v[e], omt), Ar<T>::mul(bl.v[e], t));
+        const T ba = Ar<T>::sub(bl.v[e], al.v[e]);
+        T num;
+        if constexpr (ORDER == 1)
+            num = Ar<T>::add(Ar<T>::add(Ar<T>::sub(yr.v[e], yl.v[e]), Ar<T>::mul(dmt, cur)), Ar<T>::mul(tt, ba));
+        else num = Ar<T>::mul(two, Ar<T>::sub(Ar<T>::mul(dmt, ba), cur));
+        res.v[e] = cubic_deriv_point<T, ORDER>(num, h, r);
+    }
+    return res;
+}
+
+// K5's work decomposition (one tile per warp on thin rows, next tile's query loaded ahead, one-interval tiles, wide
+// rows in slices with the rows kept in registers while the interval does not change); each lane of a query gets t, h
+// and the hoisted reciprocal of h.
+template <class T, int V, int LPQ, int ORDER>
+__global__ void __launch_bounds__(kBlock) interp1d_cubic_deriv_kernel(const Eval1<T> p) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ uint64_t bar;
+    const GridView<T> g = make_grid_view<T>(p.grid, p.n, p.sc, smem_raw, &bar);
+    const T g0 = g.g0, gl = g.gl;
+    const T one = (T)1;
+    const int lane = threadIdx.x & 31;
+    const long long nwarps = (long long)gridDim.x * kWarpsPerBlock;
+    const long long task0 = (long long)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+    T x_ahead = g0;
+    if (LPQ < 32 && task0 < p.ntasks && task0 * 32 + lane < p.nq) x_ahead = ld_query(p.q + task0 * 32 + lane);
+    for (long long task = task0; task < p.ntasks; task += nwarps) {
+        if constexpr (LPQ < 32) {
+            constexpr int QPR = 32 / LPQ;
+            const long long qbase = task * 32, qi = qbase + lane;
+            T x[1] = {x_ahead};
+            const long long qn = (task + nwarps) * 32 + lane;
+            x_ahead = (task + nwarps < p.ntasks && qn < p.nq) ? ld_query(p.q + qn) : g0;
+            const bool bad = cubic_prepare<T>(x[0], g0, gl, p.mode) && qi < p.nq;
+            int idx[1]; T xls[1], xrs[1];
+            search_multi<T, 1>(g, x, idx, xls, xrs);
+            const T h = Ar<T>::sub(xrs[0], xls[0]);
+            const T t = Ar<T>::div(Ar<T>::sub(x[0], xls[0]), h);
+            const T r = Hoisted<T>::rcp(h);
+            report_first_bad(p.err, bad, (unsigned long long)qi);
+            const bool skip = bad || !(qi < p.nq);
+            const int sub = lane % LPQ, qsel = lane / LPQ;
+            const long long col = (long long)sub * V;
+            const bool colok = col < p.w;
+            const int idx0 = __shfl_sync(0xffffffffu, idx[0], __ffs(__ballot_sync(0xffffffffu, !skip) | 0x80000000u) - 1);
+            const bool one_interval = LPQ > 1 && __all_sync(0xffffffffu, skip || idx[0] == idx0);
+            Vec<T, V> yl, yr, al, bl;
+            if (one_interval && colok) {
+                const long long ro = (long long)idx0 * p.w + col;
+                yl = ld_table<T, V>(p.data + ro);
+                yr = ld_table<T, V>(p.data + ro + p.w);
+                al = ld_table<T, V>(p.a + ro);
+                bl = ld_table<T, V>(p.b + ro);
+            }
+#pragma unroll
+            for (int rd = 0; rd < LPQ; ++rd) {
+                const int src = rd * QPR + qsel;
+                const int is = __shfl_sync(0xffffffffu, skip ? -1 : idx[0], src);
+                const T ts = shfl_t(t, src), hs = shfl_t(h, src), rs = shfl_t(r, src);
+                if (is >= 0 && colok) {
+                    if (!one_interval) {
+                        const long long ro = (long long)is * p.w + col;
+                        yl = ld_table<T, V>(p.data + ro);
+                        yr = ld_table<T, V>(p.data + ro + p.w);
+                        al = ld_table<T, V>(p.a + ro);
+                        bl = ld_table<T, V>(p.b + ro);
+                    }
+                    st_stream<T, V>(p.out + (qbase + src) * p.w + col,
+                                    cubic_deriv_vec<T, V, ORDER>(yl, yr, al, bl, ts, Ar<T>::sub(one, ts), hs, rs));
+                }
+            }
+        } else {
+            const long long tile = task / p.nslices;
+            const int slice = (int)(task - tile * p.nslices);
+            const long long qbase = tile * 32;
+            const long long qi = qbase + lane;
+            const bool live = qi < p.nq;
+            T x[1] = {live ? ld_query(p.q + qi) : g0};
+            const bool bad = cubic_prepare<T>(x[0], g0, gl, p.mode) && live;
+            int idx[1]; T xls[1], xrs[1];
+            search_multi<T, 1>(g, x, idx, xls, xrs);
+            const T h = Ar<T>::sub(xrs[0], xls[0]);
+            const T t = Ar<T>::div(Ar<T>::sub(x[0], xls[0]), h);
+            const T omt = Ar<T>::sub(one, t);
+            const T r = Hoisted<T>::rcp(h);
+            if (slice == 0) report_first_bad(p.err, bad, (unsigned long long)qi);
+            const bool skip = bad || !live;
+            const long long col = ((long long)slice * 32 + lane) * V;
+            const bool colok = col < p.w;
+            int cur = -1;
+            Vec<T, V> yl, yr, al, bl;
+            const int nlive = (int)min((long long)32, p.nq - qbase);
+            for (int s = 0; s < nlive; ++s) {
+                const int is = __shfl_sync(0xffffffffu, skip ? -1 : idx[0], s);
+                const T ts = shfl_t(t, s), os = shfl_t(omt, s), hs = shfl_t(h, s), rs = shfl_t(r, s);
+                if (is < 0 || !colok) continue;
+                if (is != cur) {
+                    const long long ro = (long long)is * p.w + col;
+                    yl = ld_table<T, V>(p.data + ro);
+                    yr = ld_table<T, V>(p.data + ro + p.w);
+                    al = ld_table<T, V>(p.a + ro);
+                    bl = ld_table<T, V>(p.b + ro);
+                    cur = is;
+                }
+                st_stream<T, V>(p.out + (qbase + s) * p.w + col, cubic_deriv_vec<T, V, ORDER>(yl, yr, al, bl, ts, os, hs, rs));
+            }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// K3d: slope of Linear (NOT in the reference): m = (y2 - y1) / (x2 - x1), the first term of calc_frac (linear.rs:29-36)
+// ------------------------------------------------------------------------------------------------
+// K3's query handling and work decomposition; per element one division, nothing of x - x1.  The quotient IS the
+// output here, so the sign of a zero numerator must survive (y2 = -0, y1 = +0 gives -0): floats divide through
+// Hoisted<T>, which sends zero numerators to the IEEE division; integers wrap and truncate like K3's m.
+template <class T>
+__device__ __forceinline__ T slope_div(T num, T d, T r) {
+    if constexpr (std::is_floating_point<T>::value) return Hoisted<T>::div(num, d, r);
+    else return Ar<T>::div(num, d);
+}
+template <class T>
+__device__ __forceinline__ T slope_rcp(T d) {
+    if constexpr (std::is_floating_point<T>::value) return Hoisted<T>::rcp(d);
+    else return (T)0;
+}
+template <class T, int V>
+__device__ __forceinline__ Vec<T, V> slope_vec(const Vec<T, V>& y1, const Vec<T, V>& y2, T d, T r) {
+    Vec<T, V> res;
+#pragma unroll
+    for (int e = 0; e < V; ++e) res.v[e] = slope_div<T>(Ar<T>::sub(y2.v[e], y1.v[e]), d, r);
+    return res;
+}
+
+template <class T, int V, int LPQ>
+__global__ void __launch_bounds__(kBlock) interp1d_linear_slope_kernel(const Eval1<T> p) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ uint64_t bar;
+    const GridView<T> g = make_grid_view<T>(p.grid, p.n, p.sc, smem_raw, &bar);
+    const T g0 = g.g0, gl = g.gl;
+    const int lane = threadIdx.x & 31;
+    const long long nwarps = (long long)gridDim.x * kWarpsPerBlock;
+    const long long task0 = (long long)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+    T x_ahead = g0;
+    if (LPQ < 32 && task0 < p.ntasks && task0 * 32 + lane < p.nq) x_ahead = ld_query(p.q + task0 * 32 + lane);
+    for (long long task = task0; task < p.ntasks; task += nwarps) {
+        if constexpr (LPQ < 32) {
+            constexpr int QPR = 32 / LPQ;
+            const long long qbase = task * 32, qi = qbase + lane;
+            T x[1] = {x_ahead};
+            const long long qn = (task + nwarps) * 32 + lane;
+            x_ahead = (task + nwarps < p.ntasks && qn < p.nq) ? ld_query(p.q + qn) : g0;
+            int idx[1]; T x1s[1], x2s[1];
+            search_multi<T, 1>(g, x, idx, x1s, x2s);                                    // linear.rs:87, :90-91
+            const bool live = qi < p.nq;
+            const bool bad = live && (p.mode ? Ar<T>::is_nan(x[0]) : !in_range(g0, gl, x[0]));   // linear.rs:80-84
+            const T d = Ar<T>::sub(x2s[0], x1s[0]);
+            const T r = slope_rcp<T>(d);
+            report_first_bad(p.err, bad, (unsigned long long)qi);
+            const bool skip = bad || !live;
+            const int sub = lane % LPQ, qsel = lane / LPQ;
+            const long long col = (long long)sub * V;
+            const bool colok = col < p.w;
+            const int idx0 = __shfl_sync(0xffffffffu, idx[0], __ffs(__ballot_sync(0xffffffffu, !skip) | 0x80000000u) - 1);
+            const bool one_interval = LPQ > 1 && __all_sync(0xffffffffu, skip || idx[0] == idx0);
+            Vec<T, V> y1, y2;
+            if (one_interval && colok) {
+                const T* row = p.data + (long long)idx0 * p.w + col;
+                y1 = ld_table<T, V>(row);
+                y2 = ld_table<T, V>(row + p.w);
+            }
+#pragma unroll
+            for (int rd = 0; rd < LPQ; ++rd) {
+                const int src = rd * QPR + qsel;
+                const int is = __shfl_sync(0xffffffffu, skip ? -1 : idx[0], src);
+                const T ds = shfl_t(d, src), rs = shfl_t(r, src);
+                if (is >= 0 && colok) {
+                    if (!one_interval) {
+                        const T* row = p.data + (long long)is * p.w + col;
+                        y1 = ld_table<T, V>(row);
+                        y2 = ld_table<T, V>(row + p.w);
+                    }
+                    st_stream<T, V>(p.out + (qbase + src) * p.w + col, slope_vec<T, V>(y1, y2, ds, rs));
+                }
+            }
+        } else {
+            const long long tile = task / p.nslices;
+            const int slice = (int)(task - tile * p.nslices);
+            const long long qbase = tile * 32;
+            const long long qi = qbase + lane;
+            const bool live = qi < p.nq;
+            T x[1] = {live ? ld_query(p.q + qi) : g0};
+            int idx[1]; T x1s[1], x2s[1];
+            search_multi<T, 1>(g, x, idx, x1s, x2s);
+            const bool bad = live && (p.mode ? Ar<T>::is_nan(x[0]) : !in_range(g0, gl, x[0]));
+            const T d = Ar<T>::sub(x2s[0], x1s[0]);
+            const T r = slope_rcp<T>(d);
+            if (slice == 0) report_first_bad(p.err, bad, (unsigned long long)qi);
+            const bool skip = bad || !live;
+            const long long col = ((long long)slice * 32 + lane) * V;
+            const bool colok = col < p.w;
+            int cur = -1;
+            Vec<T, V> y1, y2;
+            const int nlive = (int)min((long long)32, p.nq - qbase);
+            for (int s = 0; s < nlive; ++s) {
+                const int is = __shfl_sync(0xffffffffu, skip ? -1 : idx[0], s);
+                const T ds = shfl_t(d, s), rs = shfl_t(r, s);
+                if (is < 0 || !colok) continue;
+                if (is != cur) {
+                    const T* row = p.data + (long long)is * p.w + col;
+                    y1 = ld_table<T, V>(row);
+                    y2 = ld_table<T, V>(row + p.w);
+                    cur = is;
+                }
+                st_stream<T, V>(p.out + (qbase + s) * p.w + col, slope_vec<T, V>(y1, y2, ds, rs));
+            }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // K4: Bilinear::interp_into x batch (bilinear.rs:64-99)
 // ------------------------------------------------------------------------------------------------
 // Very thin rows (LPQ <= 2, e.g. C4: 8 f32 columns) are bound by gather latency: five resident blocks
@@ -889,6 +1151,31 @@ cudaError_t launch_interp1d_cubic(const T* grid, int64_t n, SearchCfg sc, const 
     NDI_VEC_SWITCH(interp1d_cubic_kernel, T, sh, p, smem, st)
 }
 
+template <class T, int V, int LPQ> constexpr auto cubic_deriv1 = interp1d_cubic_deriv_kernel<T, V, LPQ, 1>;
+template <class T, int V, int LPQ> constexpr auto cubic_deriv2 = interp1d_cubic_deriv_kernel<T, V, LPQ, 2>;
+
+template <class T>
+cudaError_t launch_interp1d_cubic_deriv(const T* grid, int64_t n, SearchCfg sc, const T* data, const T* a, const T* b,
+                                        int64_t w, const T* q, int64_t nq, int extrap_mode, int order, T* out,
+                                        unsigned long long* err, cudaStream_t st) {
+    if (nq <= 0) return cudaSuccess;
+    Shape sh = pick_shape(w, nq, pick_vec<T>(w, {data, a, b, out}), 1);
+    Eval1<T> p{grid, (int)n, sc, data, a, b, (long long)w, q, (long long)nq, extrap_mode, out, err, sh.ntasks, sh.nslices, 0};
+    size_t smem = stage_bytes(sc, sizeof(T));
+    if (order == 1) { NDI_VEC_SWITCH(cubic_deriv1, T, sh, p, smem, st) }
+    NDI_VEC_SWITCH(cubic_deriv2, T, sh, p, smem, st)
+}
+
+template <class T>
+cudaError_t launch_interp1d_linear_slope(const T* grid, int64_t n, SearchCfg sc, const T* data, int64_t w, const T* q,
+                                         int64_t nq, int extrapolate, T* out, unsigned long long* err, cudaStream_t st) {
+    if (nq <= 0) return cudaSuccess;
+    Shape sh = pick_shape(w, nq, pick_vec<T>(w, {data, out}), 1);
+    Eval1<T> p{grid, (int)n, sc, data, nullptr, nullptr, (long long)w, q, (long long)nq, extrapolate, out, err, sh.ntasks, sh.nslices, 0};
+    size_t smem = stage_bytes(sc, sizeof(T));
+    NDI_VEC_SWITCH(interp1d_linear_slope_kernel, T, sh, p, smem, st)
+}
+
 template <class T>
 cudaError_t launch_interp2d_bilinear(const T* gx, int64_t n, SearchCfg scx, const T* gy, int64_t m, SearchCfg scy,
                                      const T* data, int64_t w, const T* qx, const T* qy, int64_t nq, int extrapolate,
@@ -940,7 +1227,9 @@ cudaError_t launch_validate_queries(const T* gx, int64_t n, const T* gy, int64_t
     template cudaError_t launch_lower_index<T>(const T*, int64_t, SearchCfg, const T*, int64_t, int64_t*,              \
                                                unsigned long long*, cudaStream_t);                                     \
     template cudaError_t launch_validate_queries<T>(const T*, int64_t, const T*, int64_t, const T*, const T*, int64_t, \
-                                                    int, unsigned long long*, cudaStream_t);
+                                                    int, unsigned long long*, cudaStream_t);                           \
+    template cudaError_t launch_interp1d_linear_slope<T>(const T*, int64_t, SearchCfg, const T*, int64_t, const T*,    \
+                                                         int64_t, int, T*, unsigned long long*, cudaStream_t);
 NDI_INST_COMMON(float)
 NDI_INST_COMMON(double)
 NDI_INST_COMMON(int32_t)
@@ -953,5 +1242,11 @@ template cudaError_t launch_interp1d_cubic<float>(const float*, int64_t, SearchC
 template cudaError_t launch_interp1d_cubic<double>(const double*, int64_t, SearchCfg, const double*, const double*,
                                                    const double*, int64_t, const double*, int64_t, int, double*,
                                                    unsigned long long*, cudaStream_t);
+template cudaError_t launch_interp1d_cubic_deriv<float>(const float*, int64_t, SearchCfg, const float*, const float*,
+                                                        const float*, int64_t, const float*, int64_t, int, int, float*,
+                                                        unsigned long long*, cudaStream_t);
+template cudaError_t launch_interp1d_cubic_deriv<double>(const double*, int64_t, SearchCfg, const double*, const double*,
+                                                         const double*, int64_t, const double*, int64_t, int, int, double*,
+                                                         unsigned long long*, cudaStream_t);
 
 }  // namespace ndi

@@ -63,6 +63,14 @@ template <class T>
 cudaError_t launch_interp1d_cubic(const T* grid, int64_t n, SearchCfg sc, const T* data, const T* a, const T* b,
                                   int64_t w, const T* q, int64_t nq, int extrap_mode, T* out,
                                   unsigned long long* err, cudaStream_t st);
+// derivative of order 1 or 2 of the cubic spline (K5d), slope of Linear (K3d): query handling as the value launchers
+template <class T>
+cudaError_t launch_interp1d_cubic_deriv(const T* grid, int64_t n, SearchCfg sc, const T* data, const T* a, const T* b,
+                                        int64_t w, const T* q, int64_t nq, int extrap_mode, int order, T* out,
+                                        unsigned long long* err, cudaStream_t st);
+template <class T>
+cudaError_t launch_interp1d_linear_slope(const T* grid, int64_t n, SearchCfg sc, const T* data, int64_t w, const T* q,
+                                         int64_t nq, int extrapolate, T* out, unsigned long long* err, cudaStream_t st);
 template <class T>
 cudaError_t launch_interp2d_bilinear(const T* gx, int64_t n, SearchCfg scx, const T* gy, int64_t m, SearchCfg scy,
                                      const T* data, int64_t w, const T* qx, const T* qy, int64_t nq, int extrapolate,

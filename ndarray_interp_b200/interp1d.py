@@ -77,6 +77,18 @@ class Linear(Interp1DStrategyBuilder, Interp1DStrategy):
     def interp_into(self, interpolator, target, x):        # linear.rs:73-98
         _single_into(self, interpolator, target, x)
 
+    def deriv_batch_into(self, interpolator, xs_flat, out_rows, order=1):
+        """NOT in the reference: slope (y[i+1] - y[i]) / (x[i+1] - x[i]) of the interval each query falls into, with
+        interp_batch_into's query handling and errors (include/ndi_b200.h: ndi_interp1d_linear_deriv).  A piecewise
+        linear interpolant has no second derivative: order must be 1."""
+        if order != 1:
+            raise ValueError(f"Linear has only a first derivative, got order {order}")
+        bad = C.c_int64(-1)
+        fn, h = ((L.load().ndi_interp1d_group_linear_deriv, interpolator._group.ptr) if getattr(interpolator, "_group", None)
+                 else (L.load().ndi_interp1d_linear_deriv, interpolator._handle()))
+        st = L.check(fn(h, L.ptr(xs_flat), xs_flat.size, int(self._extrapolate), L.ptr(out_rows), C.byref(bad)))
+        _raise_eval(st, xs_flat, bad.value, "x")
+
 
 # ---- CubicSpline -------------------------------------------------------------------------------------------
 class SingleBoundary:
@@ -287,6 +299,18 @@ class CubicSplineStrategy(Interp1DStrategy):
     def interp_into(self, interpolator, target, x):        # cubic_spline.rs:791-830
         _single_into(self, interpolator, target, x)
 
+    def deriv_batch_into(self, interpolator, xs_flat, out_rows, order=1):
+        """NOT in the reference: first (order 1) or second (order 2) derivative of the spline, as scipy's
+        CubicSpline(x, nu), with interp_batch_into's query handling and errors (include/ndi_b200.h:
+        ndi_interp1d_cubic_deriv)"""
+        if order not in (1, 2):
+            raise ValueError(f"CubicSpline derivative order must be 1 or 2, got {order}")
+        bad = C.c_int64(-1)
+        fn, h = ((L.load().ndi_interp1d_group_cubic_deriv, interpolator._group.ptr) if getattr(interpolator, "_group", None)
+                 else (L.load().ndi_interp1d_cubic_deriv, interpolator._handle()))
+        st = L.check(fn(h, L.ptr(xs_flat), xs_flat.size, self._mode, int(order), L.ptr(out_rows), C.byref(bad)))
+        _raise_eval(st, xs_flat, bad.value, "x")
+
 
 def _ndarray_debug(a):
     """`{:?}` of a 1-D C-contiguous ndarray view, as pinned by tests/cubic_spline_strat.rs:441-443"""
@@ -431,6 +455,33 @@ class Interp1D:
     def interp_array_into(self, xs, buffer):
         """like `interp_array`, into the provided buffer of shape xs.shape ++ data.shape[1:]
         (interp1d/mod.rs:272-324).  One launch for the whole batch, whatever the query rank."""
+        self._array_into(xs, buffer, self.strategy.interp_batch_into)
+
+    # -- derivatives: NOT in the reference ----------------------------------------------------------------------------
+    def interp_deriv(self, x, order=1):
+        """NOT in the reference: derivative of order `order` at `x`, shaped like `interp(x)` (the built-in strategies:
+        Linear order 1, CubicSpline order 1 or 2; scipy's CubicSpline(x, nu))"""
+        target = np.zeros(self.data.shape[1:], dtype=self.data.dtype)
+        self.interp_array_deriv_into(np.array([x], dtype=self.data.dtype), target.reshape((1,) + target.shape), order)
+        return target
+
+    def interp_array_deriv(self, xs, order=1):
+        """NOT in the reference: derivatives at all points in `xs`, shaped like `interp_array(xs)`"""
+        xs = np.asarray(xs)
+        ys = np.zeros(self._buffer_shape(xs.shape), dtype=self.data.dtype)
+        self.interp_array_deriv_into(xs, ys, order)
+        return ys
+
+    def interp_array_deriv_into(self, xs, buffer, order=1):
+        """NOT in the reference: like `interp_array_deriv`, into the provided buffer; buffer shape, query rank, errors
+        and untouched rows after a failing query as `interp_array_into`"""
+        if not _is_builtin(self.strategy):
+            raise TypeError("derivatives are computed by the built-in strategies (Linear, CubicSpline) only")
+        if order not in ((1,) if isinstance(self.strategy, Linear) else (1, 2)):   # before any shape check
+            raise ValueError(f"{type(self.strategy).__name__} has no derivative of order {order}")
+        self._array_into(xs, buffer, lambda i, q, rows: self.strategy.deriv_batch_into(i, q, rows, order))
+
+    def _array_into(self, xs, buffer, batch):
         xs = np.asarray(xs)
         expect = self._buffer_shape(xs.shape)
         got = tuple(np.shape(buffer))
@@ -443,7 +494,7 @@ class Interp1D:
         # rows at and after a failing query must come back untouched (interp1d/mod.rs:321, :336-340)
         rows = buffer.reshape(rows_shape) if direct else np.array(buffer, dtype=self.data.dtype).reshape(rows_shape)
         try:
-            self.strategy.interp_batch_into(self, q, rows)
+            batch(self, q, rows)
         finally:
             if not direct:
                 buffer[...] = rows.reshape(expect)

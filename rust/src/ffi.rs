@@ -42,6 +42,9 @@ extern "C" {
     pub fn ndi_interp1d_build_info(h: *const ndi_interp1d, rowsplit_levels: *mut i32) -> ndi_status;
     pub fn ndi_interp1d_spline_coeffs(h: *const ndi_interp1d, a: *mut c_void, b: *mut c_void) -> ndi_status;
     pub fn ndi_interp1d_cubic(h: *const ndi_interp1d, q: *const c_void, nq: i64, extrap_mode: i32, out: *mut c_void, first_bad: *mut i64) -> ndi_status;
+    /// derivatives (not in the reference): order 1 or 2 of the spline, the slope of Linear
+    pub fn ndi_interp1d_cubic_deriv(h: *const ndi_interp1d, q: *const c_void, nq: i64, extrap_mode: i32, order: i32, out: *mut c_void, first_bad: *mut i64) -> ndi_status;
+    pub fn ndi_interp1d_linear_deriv(h: *const ndi_interp1d, q: *const c_void, nq: i64, extrapolate: i32, out: *mut c_void, first_bad: *mut i64) -> ndi_status;
 
     pub fn ndi_interp1d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp1d) -> ndi_status;
     pub fn ndi_interp2d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, y: *const c_void, m: i64, y_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp2d) -> ndi_status;

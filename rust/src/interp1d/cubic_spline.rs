@@ -6,7 +6,7 @@ use std::{ffi::c_void, fmt::Debug};
 use ndarray::{Array, ArrayBase, ArrayViewMut, Axis, Data, Dimension, Ix1, RemoveAxis};
 use num_traits::{Euclid, Float};
 
-use super::{eval_result, DeviceTable1D, Interp1D, Interp1DStrategy, Interp1DStrategyBuilder};
+use super::{eval_result, DeviceTable1D, Interp1D, Interp1DDerivStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
 use crate::{ffi, BuilderError, InterpolateError, NdiElem};
 
 /// element types usable with the CubicSpline strategy (float only, like the reference's `SplineNum`)
@@ -247,6 +247,32 @@ where
                 xs.as_ptr() as *const c_void,
                 xs.len() as i64,
                 self.extrapolate as i32,
+                out.as_mut_ptr() as *mut c_void,
+                &mut first_bad,
+            )
+        };
+        eval_result(st, xs, first_bad, "x")
+    }
+}
+
+/// NOT in the reference: first and second derivative of the spline (scipy's `CubicSpline(x, nu)`)
+impl<Sd, Sx, D> Interp1DDerivStrategy<Sd, Sx, D> for CubicSplineStrategy<Sd, D>
+where
+    Sd: Data,
+    Sd::Elem: SplineNum,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+{
+    fn deriv_batch_into(&self, interp: &Interp1D<Sd, Sx, D, Self>, xs: &[Sd::Elem], out: &mut [Sd::Elem], order: i32) -> Result<(), InterpolateError> {
+        assert!(order == 1 || order == 2, "CubicSpline derivative order must be 1 or 2, got {order}");
+        let mut first_bad = -1i64;
+        let st = unsafe {
+            ffi::ndi_interp1d_cubic_deriv(
+                interp.table.0,
+                xs.as_ptr() as *const c_void,
+                xs.len() as i64,
+                self.extrapolate as i32,
+                order,
                 out.as_mut_ptr() as *mut c_void,
                 &mut first_bad,
             )

@@ -3,7 +3,7 @@ use std::ffi::c_void;
 
 use ndarray::{ArrayBase, ArrayViewMut, Data, Dimension, Ix1, RemoveAxis};
 
-use super::{eval_result, Interp1D, Interp1DStrategy, Interp1DStrategyBuilder};
+use super::{eval_result, Interp1D, Interp1DDerivStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
 use crate::{ffi, BuilderError, InterpolateError, NdiElem};
 
 /// Linear Interpolation Strategy
@@ -78,6 +78,31 @@ where
         let mut first_bad = -1i64;
         let st = unsafe {
             ffi::ndi_interp1d_linear(
+                interpolator.table.0,
+                xs.as_ptr() as *const c_void,
+                xs.len() as i64,
+                self.extrapolate as i32,
+                out.as_mut_ptr() as *mut c_void,
+                &mut first_bad,
+            )
+        };
+        eval_result(st, xs, first_bad, "x")
+    }
+}
+
+/// NOT in the reference: the slope `(y[i+1] - y[i]) / (x[i+1] - x[i])` of each query's interval
+impl<Sd, Sx, D> Interp1DDerivStrategy<Sd, Sx, D> for Linear
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+{
+    fn deriv_batch_into(&self, interpolator: &Interp1D<Sd, Sx, D, Self>, xs: &[Sd::Elem], out: &mut [Sd::Elem], order: i32) -> Result<(), InterpolateError> {
+        assert!(order == 1, "Linear has only a first derivative, got order {order}");
+        let mut first_bad = -1i64;
+        let st = unsafe {
+            ffi::ndi_interp1d_linear_deriv(
                 interpolator.table.0,
                 xs.as_ptr() as *const c_void,
                 xs.len() as i64,

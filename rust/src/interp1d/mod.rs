@@ -19,6 +19,25 @@ pub mod cubic_spline;
 mod linear;
 pub use linear::Linear;
 
+/// NOT in the reference: derivatives of an interpolant, computed on the device (`ndi_interp1d_*_deriv`).  A trait of
+/// its own, next to [`Interp1DStrategy`], so that the reference's strategy trait keeps exactly its items; implemented
+/// by the built-in strategies ([`Linear`]: order 1, [`cubic_spline::CubicSplineStrategy`]: order 1 and 2).
+pub trait Interp1DDerivStrategy<Sd, Sx, D>
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+    Self: Sized,
+{
+    /// derivative of order `order` at every query of `xs` into the rows of `out` (`xs.len() * row length`), with the
+    /// query handling and errors of [`Interp1DStrategy::interp_batch_into`].
+    ///
+    /// # panics
+    /// When the strategy has no derivative of that order
+    fn deriv_batch_into(&self, interpolator: &Interp1D<Sd, Sx, D, Self>, xs: &[Sd::Elem], out: &mut [Sd::Elem], order: i32) -> Result<(), InterpolateError>;
+}
+
 /// Owner of the opaque device handle (grid, data, spline coefficients in HBM).
 /// Immutable after build, so it is shared freely between threads like the reference's `&self`.
 #[derive(Debug)]
@@ -247,6 +266,85 @@ where
 
     pub fn is_in_range(&self, x: Sx::Elem) -> bool {
         self.x[0] <= x && x <= self.x[self.x.len() - 1]
+    }
+}
+
+/// NOT in the reference: derivatives (see [`Interp1DDerivStrategy`]); shapes, errors and panics as the value methods
+impl<Sd, Sx, D, Strat> Interp1D<Sd, Sx, D, Strat>
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+    Strat: Interp1DStrategy<Sd, Sx, D> + Interp1DDerivStrategy<Sd, Sx, D>,
+{
+    /// derivative of order `order` at `x`, one dimension smaller than the data
+    pub fn interp_deriv(&self, x: Sx::Elem, order: i32) -> Result<Array<Sd::Elem, D::Smaller>, InterpolateError> {
+        let mut target = Array::zeros(self.data.raw_dim().remove_axis(Axis(0)));
+        let out = target.as_slice_mut().unwrap_or_else(|| unreachable!());
+        self.strategy.deriv_batch_into(self, &[x], out, order).map(|_| target)
+    }
+
+    /// derivatives at all points in `xs`; output shape = `xs.shape() ++ data.shape()[1..]`
+    pub fn interp_array_deriv<Sq, Dq>(
+        &self,
+        xs: &ArrayBase<Sq, Dq>,
+        order: i32,
+    ) -> Result<Array<Sd::Elem, <Dq as DimAdd<D::Smaller>>::Output>, InterpolateError>
+    where
+        Sq: Data<Elem = Sd::Elem>,
+        Dq: Dimension + DimAdd<D::Smaller>,
+    {
+        let mut shape = <Dq as DimAdd<D::Smaller>>::Output::zeros(xs.ndim() + self.data.ndim() - 1);
+        for (dst, src) in shape.slice_mut().iter_mut().zip(xs.shape().iter().chain(self.data.shape()[1..].iter())) {
+            *dst = *src;
+        }
+        let mut ys = Array::zeros(shape);
+        self.interp_array_deriv_into(xs, ys.view_mut(), order).map(|_| ys)
+    }
+
+    /// like [`interp_array_deriv`](Interp1D::interp_array_deriv), into the provided buffer, which may have any
+    /// layout (C order, Fortran order, permuted or reversed axes), as for
+    /// [`interp_array_into`](Interp1D::interp_array_into):
+    ///
+    /// ```no_run
+    /// use ndarray::{array, Array2, ShapeBuilder};
+    /// use ndarray_interp_b200::interp1d::Interp1D;
+    /// let ip = Interp1D::builder(array![[0.0, 1.0], [2.0, 4.0], [3.0, 9.0]]).build().unwrap();
+    /// let xs = array![0.5, 1.5];
+    /// let mut f_order = Array2::<f64>::zeros((2, 2).f());
+    /// ip.interp_array_deriv_into(&xs, f_order.view_mut(), 1).unwrap();
+    /// assert_eq!(f_order, array![[2.0, 3.0], [1.0, 5.0]]);
+    /// ```
+    ///
+    /// # panics
+    /// When the provided buffer has the wrong shape, or the strategy has no derivative of that order
+    pub fn interp_array_deriv_into<Sq, Dq>(
+        &self,
+        xs: &ArrayBase<Sq, Dq>,
+        mut buffer: ArrayViewMut<'_, Sd::Elem, <Dq as DimAdd<D::Smaller>>::Output>,
+        order: i32,
+    ) -> Result<(), InterpolateError>
+    where
+        Sq: Data<Elem = Sd::Elem>,
+        Dq: Dimension + DimAdd<D::Smaller>,
+    {
+        let expect: Vec<usize> = xs.shape().iter().chain(self.data.shape()[1..].iter()).copied().collect();
+        assert!(buffer.shape() == expect.as_slice(), "expected: {:?}, got: {:?}", expect, buffer.shape());
+        let queries = xs.as_standard_layout();
+        let q = queries.as_slice().unwrap_or_else(|| unreachable!());
+        match buffer.as_slice_mut() {
+            Some(out) => self.strategy.deriv_batch_into(self, q, out, order),
+            None => {
+                // strided destination: start from the caller's values, so rows after a failing query stay untouched
+                // (standard layout: `to_owned` would keep an F-order or reversed buffer's strides)
+                let mut scratch = Array::<Sd::Elem, _>::zeros(buffer.raw_dim());
+                scratch.assign(&buffer);
+                let res = self.strategy.deriv_batch_into(self, q, scratch.as_slice_mut().unwrap_or_else(|| unreachable!()), order);
+                buffer.assign(&scratch);
+                res
+            }
+        }
     }
 }
 
