@@ -37,6 +37,7 @@
 #include <functional>
 #include <initializer_list>
 #include <memory>
+#include <mutex>
 #include <numeric>
 #include <stdexcept>
 #include <string>
@@ -62,7 +63,8 @@ struct LibraryError : std::runtime_error { using std::runtime_error::runtime_err
 
 namespace detail {
 inline void check(ndi_status st) {
-    if (st >= NDI_CUDA_ERROR || st == NDI_INVALID_ARGUMENT || st == NDI_UNSUPPORTED_DTYPE || st == NDI_NO_DEVICE || st == NDI_NO_SPLINE)
+    if (st >= NDI_CUDA_ERROR || st == NDI_INVALID_ARGUMENT || st == NDI_UNSUPPORTED_DTYPE || st == NDI_NO_DEVICE || st == NDI_NO_SPLINE ||
+        st == NDI_NO_INTEGRAL)
         throw LibraryError(std::string("ndi status ") + std::to_string((int)st) + ": " + ndi_last_error_message());
 }
 template <class T> struct dtype_of;
@@ -295,6 +297,9 @@ public:
     // NOT in the reference (ndi_interp1d_linear_deriv): slope of each query's interval, interp_batch_into's query
     // handling and errors; order must be 1 (std::invalid_argument otherwise)
     void deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const;
+    // NOT in the reference (ndi_interp1d_linear_integral): integral from lo[i] to hi[i], each bound handled as
+    // interp_batch_into handles a query
+    void integral_batch_into(const Interp1D<T>& ip, const T* lo, const T* hi, size_t nq, T* out_rows) const;
 private:
     bool extrapolate_ = false;
 };
@@ -349,6 +354,8 @@ public:
     // NOT in the reference (ndi_interp1d_cubic_deriv): derivative of order 1 or 2 (std::invalid_argument otherwise),
     // interp_batch_into's query handling and errors
     void deriv_batch_into(const Interp1D<T>& ip, const T* xs, size_t nq, T* out_rows, int order) const;
+    // NOT in the reference (ndi_interp1d_cubic_integral, scipy's CubicSpline.integrate): integral from lo[i] to hi[i]
+    void integral_batch_into(const Interp1D<T>& ip, const T* lo, const T* hi, size_t nq, T* out_rows) const;
     // (a, b) copied back from the device: shape (n-1, ...data.shape[1..])
     std::pair<Array<T>, Array<T>> coefficients(const Interp1D<T>& ip) const;
 private:
@@ -450,6 +457,46 @@ public:
         });
     }
 
+    // ---- definite integrals: NOT in the reference (built-in strategies, float data) ----------------------------------
+    // the integral from a to b, one dimension smaller than the data
+    Array<T> integrate(T a, T b) const {
+        Array<T> target = Array<T>::zeros(trailing_shape());
+        std::vector<size_t> one_row = trailing_shape();
+        one_row.insert(one_row.begin(), 1);
+        std::vector<std::ptrdiff_t> st(one_row.size(), 1);
+        for (size_t i = one_row.size(); i-- > 1;) st[i - 1] = st[i] * (std::ptrdiff_t)one_row[i];
+        interp_array_integral_into(ArrayView<T>{&a, {1}, {1}}, ArrayView<T>{&b, {1}, {1}}, ArrayViewMut<T>{target.data(), one_row, st});
+        return target;
+    }
+    // integrals over the pairs (lo[i], hi[i]) of two arrays of one shape; output shape lo.shape ++ data.shape[1..]
+    Array<T> interp_array_integral(const ArrayView<T>& lo, const ArrayView<T>& hi) const {
+        Array<T> ys = Array<T>::zeros(buffer_shape(lo.shape));
+        interp_array_integral_into(lo, hi, ys.view_mut());
+        return ys;
+    }
+    // buffer shape, errors (the failing bound's value) and untouched rows as interp_array_into
+    void interp_array_integral_into(const ArrayView<T>& lo, const ArrayView<T>& hi, ArrayViewMut<T> buffer) const {
+        const auto* lin = dynamic_cast<const Linear<T>*>(strategy_.get());
+        const auto* cub = dynamic_cast<const CubicSplineStrategy<T>*>(strategy_.get());
+        if (!lin && !cub) throw std::invalid_argument("integrals are computed by the built-in strategies (Linear, CubicSpline) only");
+        if (lo.shape != hi.shape) throw std::invalid_argument("lo and hi need the same shape");
+        prepare_integral();
+        const std::vector<T> h = hi.to_vector();
+        array_into(lo, buffer, [&](const T* q, size_t nq, T* rows) {
+            if (lin) lin->integral_batch_into(*this, q, h.data(), nq, rows);
+            else cub->integral_batch_into(*this, q, h.data(), nq, rows);
+        });
+    }
+    // build the cumulative table the integral calls evaluate over (done on first use otherwise)
+    void prepare_integral() const {
+        if (!std::is_floating_point<T>::value) throw std::invalid_argument("integrals need float data");
+        const int kind = dynamic_cast<const CubicSplineStrategy<T>*>(strategy_.get()) ? NDI_INTEGRAL_CUBIC : NDI_INTEGRAL_LINEAR;
+        std::lock_guard<std::mutex> lock(integral_->m);
+        if (integral_->built[kind]) return;
+        detail::check(ndi_interp1d_integral_build(handle(), kind));
+        integral_->built[kind] = true;
+    }
+
     // accessors strategies may call back (:371-386)
     std::pair<T, ArrayView<T>> index_point(size_t index) const {
         auto sh = trailing_shape();
@@ -501,6 +548,8 @@ private:
     Array<T> x_, data_;
     std::shared_ptr<const Interp1DStrategy<T>> strategy_;
     mutable std::shared_ptr<ndi_interp1d> handle_;
+    struct IntegralTables { std::mutex m; bool built[2] = {false, false}; };
+    std::shared_ptr<IntegralTables> integral_ = std::make_shared<IntegralTables>();     // shared with copies, like the handle
 };
 
 // Create and configure a Interp1D Interpolator (src/interp1d/mod.rs:53-70, :389-477).
@@ -601,6 +650,22 @@ void CubicSplineStrategy<T>::deriv_batch_into(const Interp1D<T>& ip, const T* xs
     const ndi_status st = ndi_interp1d_cubic_deriv(ip.handle(), xs, (int64_t)nq, mode_, order, out_rows, &bad);
     detail::check(st);
     if (st != NDI_OK) detail::raise_eval<T>(st, xs, bad, "x");
+}
+template <class T>
+void CubicSplineStrategy<T>::integral_batch_into(const Interp1D<T>& ip, const T* lo, const T* hi, size_t nq, T* out_rows) const {
+    int64_t bad = -1;
+    int32_t bound = -1;
+    const ndi_status st = ndi_interp1d_cubic_integral(ip.handle(), lo, hi, (int64_t)nq, mode_, out_rows, &bad, &bound);
+    detail::check(st);
+    if (st != NDI_OK) detail::raise_eval<T>(st, bound == 1 ? hi : lo, bad, "x");
+}
+template <class T>
+void Linear<T>::integral_batch_into(const Interp1D<T>& ip, const T* lo, const T* hi, size_t nq, T* out_rows) const {
+    int64_t bad = -1;
+    int32_t bound = -1;
+    const ndi_status st = ndi_interp1d_linear_integral(ip.handle(), lo, hi, (int64_t)nq, extrapolate_, out_rows, &bad, &bound);
+    detail::check(st);
+    if (st != NDI_OK) detail::raise_eval<T>(st, bound == 1 ? hi : lo, bad, "x");
 }
 template <class T>
 int CubicSplineStrategy<T>::rowsplit_levels(const Interp1D<T>& ip) const {

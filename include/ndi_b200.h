@@ -57,6 +57,8 @@ typedef int32_t ndi_status;
 #define NDI_NO_SPLINE 6
 #define NDI_UNSUPPORTED_DTYPE 7
 #define NDI_NO_DEVICE 8
+/* integral requested before ndi_interp1d_integral_build built that kind's table (again, after the spline changed) */
+#define NDI_NO_INTEGRAL 9
 /* 100 + cudaError_t; text via ndi_last_error_message() */
 #define NDI_CUDA_ERROR 100
 
@@ -237,6 +239,50 @@ ndi_status ndi_interp1d_linear_deriv(const ndi_interp1d* h, const void* q, int64
 ndi_status ndi_interp1d_linear_deriv_dev(const ndi_interp1d* h, const void* q_dev, int64_t nq, int32_t extrapolate,
                                          void* out_dev, uint64_t* err_word_dev, void* stream);
 
+/* ---- definite integrals (NOT in the reference; scipy's CubicSpline.integrate(a, b, extrapolate)) ------------- */
+/* A query is a pair (lo, hi) of the handle's float dtype; output row q holds, per column, the integral from lo to hi
+ * of the interpolant the value call evaluates with the same handle and mode.
+ * Bounds: each bound is checked as the value call checks a query, lo (bound 0) before hi (bound 1): without
+ * extrapolation a bound outside [x[0], x[n-1]] or NaN stops the batch with NDI_OUT_OF_BOUNDS; NDI_EXTRAP_YES integrates
+ * the edge interval's polynomial beyond the grid and a NaN bound gives NDI_NAN_QUERY; NDI_EXTRAP_PERIODIC (cubic only)
+ * gives NDI_NAN_QUERY for a non-finite bound outside the grid.  *first_bad / *bad_bound (error word 2 * query + bound on
+ * the device) name the first failing bound; rows at and after its query are left untouched.
+ * Cumulative table C (n, w), built by ndi_interp1d_integral_build: C[0] = 0 and C[i] = the integral from x[0] to x[i],
+ * summed in double precision (also for f32 tables, rounded once when stored) from the interval integrals
+ *     e[i] = h * ((y[i] + y[i+1]) * 0.5 + (a[i] + b[i]) / 12)     (Linear: h * ((y[i] + y[i+1]) * 0.5)),  h = x[i+1] - x[i]
+ * in this order: the intervals are cut into blocks of 32 (block k: intervals 32k .. 32k+31); local(k, j) is the running
+ * sum ((e[32k] + e[32k+1]) + ...) + e[32k+j-1] (local(k, 0) = 0); off(0) = 0 and off(k) = off(k-1) + local(k-1, 32),
+ * a sequential sum over the block totals; C[32k + j] = off(k) + local(k, j).
+ * Evaluation: with i the lower index of a point x (the value call's search), h = x[i+1] - x[i], t = (x - x[i]) / h:
+ *     c2 = t t * 0.5,  c3 = (t t) t / 3,  c4 = (t t)(t t) * 0.25
+ *     W0 = h (t - c2),  W1 = h c2,  W2 = h ((c2 - (c3 + c3)) + c4),  W3 = h (c3 - c4)        (once per bound)
+ *     F_i(x) = ((W0 y[i] + W1 y[i+1]) + W2 a[i]) + W3 b[i]      (Linear: W0 y[i] + W1 y[i+1])
+ *     I(u, v) = ((C[j] - C[i]) + F_j(v)) - F_i(u)              (i, j: lower indices of u, v)
+ * so both bounds in one interval give C[j] - C[i] = 0 exactly.  Every operation is rounded on its own.  If hi < lo
+ * the bounds are swapped and the result negated, so I(lo, hi) = -I(hi, lo) exactly, and lo == hi gives exactly 0.
+ * Without NDI_EXTRAP_PERIODIC the result is I(lo, hi).  With it (scipy's PPoly.integrate, periodic branch):
+ *     P = x[n-1] - x[0],  d = hi - lo,  left = rem_euclid(d, P),  k = rint((d - left) / P)
+ *     lo' = lo wrapped into the grid as the value call wraps a query (only when outside),  e = lo' + left
+ *     seg = I(lo', e) if e <= x[n-1], else (across the end of the period, e' = x[0] + (e - x[n-1]), j its lower index)
+ *           (((C[j] + C[n-1]) - C[i]) + F_j(e')) - F_i(lo')
+ *     result = k C[n-1] + seg.
+ * ndi_interp1d_integral_build builds the table of one kind on the handle's device; like ndi_interp1d_spline_build it
+ * changes the handle, so it must not run concurrently with any other call on it.  NDI_INTEGRAL_CUBIC needs the spline
+ * (NDI_NO_SPLINE), integer dtypes give NDI_UNSUPPORTED_DTYPE, another kind NDI_INVALID_ARGUMENT.
+ * ndi_interp1d_spline_build and ndi_interp1d_spline_set_coeffs drop the cubic table (calls give NDI_NO_INTEGRAL until
+ * it is built again); ndi_interp1d_clone_to_device / ndi_interp1d_replicate copy the tables the handle holds. */
+#define NDI_INTEGRAL_LINEAR 0
+#define NDI_INTEGRAL_CUBIC 1
+ndi_status ndi_interp1d_integral_build(ndi_interp1d* h, int32_t kind);
+ndi_status ndi_interp1d_cubic_integral(const ndi_interp1d* h, const void* lo, const void* hi, int64_t nq,
+                                       int32_t extrap_mode, void* out, int64_t* first_bad, int32_t* bad_bound);
+ndi_status ndi_interp1d_cubic_integral_dev(const ndi_interp1d* h, const void* lo_dev, const void* hi_dev, int64_t nq,
+                                           int32_t extrap_mode, void* out_dev, uint64_t* err_word_dev, void* stream);
+ndi_status ndi_interp1d_linear_integral(const ndi_interp1d* h, const void* lo, const void* hi, int64_t nq,
+                                        int32_t extrapolate, void* out, int64_t* first_bad, int32_t* bad_bound);
+ndi_status ndi_interp1d_linear_integral_dev(const ndi_interp1d* h, const void* lo_dev, const void* hi_dev, int64_t nq,
+                                            int32_t extrapolate, void* out_dev, uint64_t* err_word_dev, void* stream);
+
 /* ---- src/interp2d ------------------------------------------------------------------------ */
 /* Interp2DBuilder::build data upload (interp2d/mod.rs:468-518).  x: n, y: m, data: (n, m, w).
  * NDI_NOT_MONOTONIC reports the failing axis in the message ("x-axis" before "y-axis"). */
@@ -296,6 +342,11 @@ ndi_status ndi_interp1d_group_linear_deriv(ndi_interp1d_group* g, const void* q,
                                            void* out, int64_t* first_bad);
 ndi_status ndi_interp1d_group_cubic_deriv(ndi_interp1d_group* g, const void* q, int64_t nq, int32_t extrap_mode,
                                           int32_t order, void* out, int64_t* first_bad);
+/* the integral calls above, on a group (build the tables before replicating) */
+ndi_status ndi_interp1d_group_linear_integral(ndi_interp1d_group* g, const void* lo, const void* hi, int64_t nq,
+                                              int32_t extrapolate, void* out, int64_t* first_bad, int32_t* bad_bound);
+ndi_status ndi_interp1d_group_cubic_integral(ndi_interp1d_group* g, const void* lo, const void* hi, int64_t nq,
+                                             int32_t extrap_mode, void* out, int64_t* first_bad, int32_t* bad_bound);
 ndi_status ndi_interp2d_replicate(const ndi_interp2d* h, const int32_t* devices, int32_t ndev, ndi_interp2d_group** out);
 ndi_status ndi_interp2d_group_destroy(ndi_interp2d_group* g);
 ndi_status ndi_interp2d_group_bilinear(ndi_interp2d_group* g, const void* qx, const void* qy, int64_t nq,

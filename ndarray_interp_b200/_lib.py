@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get("NDI_B200_LIB") or os.path.join(_HERE, "libndi_b200.so")
 
 OK, OUT_OF_BOUNDS, NAN_QUERY, PERIODIC_MISMATCH, INVALID_ARGUMENT, NOT_MONOTONIC, NO_SPLINE, UNSUPPORTED_DTYPE, \
-    NO_DEVICE = range(9)
+    NO_DEVICE, NO_INTEGRAL = range(10)
 CUDA_ERROR = 100
 F32, F64, I32, I64, U32, U64 = 0, 1, 2, 3, 4, 5
 ASSUME_VALID, DEVICE_POINTERS, BORROW = 1, 2, 4
@@ -21,6 +21,7 @@ SEARCH_AUTO, SEARCH_BINARY_GLOBAL, SEARCH_BINARY_SMEM, SEARCH_UNIFORM_GUESS, SEA
 EXTRAP_NO, EXTRAP_YES, EXTRAP_PERIODIC = 0, 1, 2
 BIN_AUTO, BIN_OFF, BIN_ON, BIN_SWEEP = 0, 1, 2, 3
 BUILD_AUTO, BUILD_SEQUENTIAL, BUILD_ROWSPLIT, BUILD_PARTITION = 0, 1, 2, 3
+INTEGRAL_LINEAR, INTEGRAL_CUBIC = 0, 1
 ERR_WORD_NONE = 2 ** 64 - 1
 
 DTYPES = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.int32): I32,
@@ -60,6 +61,11 @@ SIGNATURES = {
     "ndi_interp1d_cubic_deriv_dev": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     "ndi_interp1d_linear_deriv": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
     "ndi_interp1d_linear_deriv_dev": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "ndi_interp1d_integral_build": (_i32, [_vp, _i32]),
+    "ndi_interp1d_cubic_integral": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
+    "ndi_interp1d_cubic_integral_dev": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "ndi_interp1d_linear_integral": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
+    "ndi_interp1d_linear_integral_dev": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp]),
     "ndi_interp2d_create": (_i32, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _u32, C.POINTER(_vp)]),
     "ndi_interp2d_create_strided": (_i32, [_i32, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _u32,
                                            C.POINTER(_vp)]),
@@ -80,6 +86,8 @@ SIGNATURES = {
     "ndi_interp1d_group_cubic": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
     "ndi_interp1d_group_linear_deriv": (_i32, [_vp, _vp, _i64, _i32, _vp, _pi64]),
     "ndi_interp1d_group_cubic_deriv": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _pi64]),
+    "ndi_interp1d_group_linear_integral": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
+    "ndi_interp1d_group_cubic_integral": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
     "ndi_interp2d_replicate": (_i32, [_vp, _pi32, _i32, C.POINTER(_vp)]),
     "ndi_interp2d_group_destroy": (_i32, [_vp]),
     "ndi_interp2d_group_bilinear": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
@@ -131,7 +139,7 @@ def last_error():
 
 def check(st):
     """turn a non-domain status into an exception"""
-    if st >= CUDA_ERROR or st in (INVALID_ARGUMENT, UNSUPPORTED_DTYPE, NO_DEVICE, NO_SPLINE):
+    if st >= CUDA_ERROR or st in (INVALID_ARGUMENT, UNSUPPORTED_DTYPE, NO_DEVICE, NO_SPLINE, NO_INTEGRAL):
         raise NdiLibraryError(f"ndi status {st}: {last_error()}")
     return st
 

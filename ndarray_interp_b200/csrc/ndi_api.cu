@@ -359,6 +359,7 @@ struct ndi_interp1d {
     int build_mode = NDI_BUILD_AUTO, build_levels = 0;   // spline solve: reference order or row-split (ndi_rowsplit.cu)
     int built_levels = kNotBuilt;    // how the current coefficients were built: 0 reference order, L > 0 row-split levels, -m partition blocks
     double nak_pivot = -1.0;         // last eliminated pivot of the NotAKnot system relative to its diagonal entry (< 0: not formed yet)
+    void* cum[2] = {nullptr, nullptr};   // cumulative tables (n, w) of the integral calls, [NDI_INTEGRAL_LINEAR / _CUBIC], owned
     GridAids aids;
     GridMeta meta() const { return aids.meta(x, n, elem_size(dtype), uniform_hint); }
 };
@@ -697,6 +698,7 @@ ndi_status ndi_interp1d_destroy(ndi_interp1d* h) {
     if (h->owns_tables) { cudaFree(h->x); cudaFree(h->data); }
     if (h->owns_coeffs) { cudaFree(h->a); cudaFree(h->b); }
     cudaFree(h->pair);
+    cudaFree(h->cum[0]); cudaFree(h->cum[1]);
     h->aids.release();
     delete h;
     return NDI_OK;
@@ -729,7 +731,7 @@ ndi_status ndi_interp1d_clone_to_device(const ndi_interp1d* h, int32_t device, n
     return clone_to_device(h, device, out, ndi_interp1d_destroy, [&](ndi_interp1d* c, auto& copy) {
         const size_t es = elem_size(h->dtype);
         c->owns_tables = true; c->owns_coeffs = h->a != nullptr;
-        c->x = c->data = c->a = c->b = c->pair = nullptr;
+        c->x = c->data = c->a = c->b = c->pair = c->cum[0] = c->cum[1] = nullptr;
         c->aids = GridAids{};
         ndi_status st = copy(&c->x, h->x, (size_t)h->n * es);
         if (st == NDI_OK) st = copy(&c->data, h->data, (size_t)h->n * h->w * es);
@@ -737,6 +739,8 @@ ndi_status ndi_interp1d_clone_to_device(const ndi_interp1d* h, int32_t device, n
         if (st == NDI_OK && h->b) st = copy(&c->b, h->b, (size_t)(h->n - 1) * h->w * es);
         if (st == NDI_OK && !h->uniform_hint) st = build_aids(c->dtype, c->x, c->n, nullptr, &c->aids);
         if (st == NDI_OK && h->pair) st = copy(&c->pair, h->pair, (size_t)(h->n - 1) * 2 * h->w * es);
+        for (int k = 0; k < 2 && st == NDI_OK; ++k)
+            if (h->cum[k]) st = copy(&c->cum[k], h->cum[k], (size_t)h->n * h->w * es);
         return st;
     });
 }
@@ -1052,6 +1056,11 @@ ndi_status ndi_interp1d_linear_deriv(const ndi_interp1d* h, const void* q, int64
 // whenever a right NotAKnot row meets such a grid.  The pivot ratio is formed once per handle from the last grid points
 // (the elimination forgets its start at a rate of ~0.07 per row; 64 rows are exact to double precision).
 constexpr double kNakPivotFloor = 0.1;
+
+// new spline coefficients: the cubic cumulative table no longer matches them (integral calls: NDI_NO_INTEGRAL until rebuilt)
+static void drop_cubic_integral(ndi_interp1d* h) {
+    if (h->cum[NDI_INTEGRAL_CUBIC]) { cudaFree(h->cum[NDI_INTEGRAL_CUBIC]); h->cum[NDI_INTEGRAL_CUBIC] = nullptr; }
+}
 static ndi_status nak_pivot_ratio(ndi_interp1d* h, cudaStream_t st, double* ratio) {
     if (h->nak_pivot >= 0.0) { *ratio = h->nak_pivot; return NDI_OK; }
     const int64_t n = h->n, cnt = n < 67 ? n : 67;
@@ -1190,6 +1199,7 @@ ndi_status ndi_interp1d_spline_build(ndi_interp1d* h, int32_t bc_kind, const int
         cleanup(true);
         if (h->owns_coeffs) { cudaFreeAsync(h->a, bs); cudaFreeAsync(h->b, bs); }
         h->a = a; h->b = b; h->owns_coeffs = true;
+        drop_cubic_integral(h);
         h->built_levels = levels;
         return NDI_OK;
     });
@@ -1229,6 +1239,7 @@ ndi_status ndi_interp1d_spline_set_coeffs(ndi_interp1d* h, const void* a, const 
     if (st != NDI_OK) { if (oa) cudaFree(na); if (ob) cudaFree(nb); return st; }
     if (h->owns_coeffs) { cudaFree(h->a); cudaFree(h->b); }
     h->a = na; h->b = nb; h->owns_coeffs = oa;
+    drop_cubic_integral(h);
     h->built_levels = kNotBuilt;
     return NDI_OK;
 }
@@ -1307,6 +1318,134 @@ ndi_status ndi_interp1d_cubic_deriv(const ndi_interp1d* h, const void* q, int64_
     uint64_t word;
     if ((st = cubic_host(h, q, nq, extrap_mode, out, &word, Phase::whole, 0, order)) != NDI_OK) return st;
     return eval1d_status(word, extrap_mode, first_bad);
+}
+
+// ---- definite integrals (NOT in the reference) -----------------------------------------------------------------------
+ndi_status ndi_interp1d_integral_build(ndi_interp1d* h, int32_t kind) {
+    if (!h) return fail(NDI_INVALID_ARGUMENT, "null handle");
+    if (kind != NDI_INTEGRAL_LINEAR && kind != NDI_INTEGRAL_CUBIC) return fail(NDI_INVALID_ARGUMENT, "bad integral kind %d", kind);
+    if (h->dtype != NDI_F32 && h->dtype != NDI_F64)
+        return fail(NDI_UNSUPPORTED_DTYPE, "integrals need a float dtype (the integral of integer data is not an integer)");
+    if (kind == NDI_INTEGRAL_CUBIC && !h->a) return fail(NDI_NO_SPLINE, "no spline coefficients: call ndi_interp1d_spline_build first");
+    DeviceGuard g(h->device);
+    ndi_status st; Workspace* ws = workspace(h->device, &st); if (!ws) return st;
+    cudaStream_t bs = ws->s[0];
+    // scratch (block totals, then offsets: (n-1)/32 + 1 doubles per column) in the per-thread build buffer
+    if ((st = grow(&ws->d_build, &ws->d_build_cap, integral_build_scratch(h->n, h->w) * sizeof(double))) != NDI_OK) return st;
+    // the table outlives the call: from the stream-ordered pool, as the spline's a / b (a cudaMalloc + cudaFree per
+    // build cost several times the build itself)
+    void* cum = nullptr;
+    CK(cudaMallocAsync(&cum, (size_t)h->n * h->w * elem_size(h->dtype), bs));
+    st = dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
+        using T = decltype(tag);
+        const bool cubic = kind == NDI_INTEGRAL_CUBIC;
+        CK(launch_integral_build<T>((const T*)h->x, h->n, (const T*)h->data, cubic ? (const T*)h->a : nullptr,
+                                    cubic ? (const T*)h->b : nullptr, h->w, (T*)cum, (double*)ws->d_build, bs));
+        CK(cudaStreamSynchronize(bs));
+        return NDI_OK;
+    });
+    if (st != NDI_OK) { cudaFreeAsync(cum, bs); cudaStreamSynchronize(bs); return st; }
+    if (h->cum[kind]) cudaFreeAsync(h->cum[kind], bs);
+    h->cum[kind] = cum;
+    return NDI_OK;
+}
+
+static ndi_status check_integral_args(const ndi_interp1d* h, const void* lo, const void* hi, int64_t nq, int32_t mode, int kind,
+                                      const void* out) {
+    ndi_status st = check_eval_args(h, lo, nq, out); if (st != NDI_OK) return st;
+    if (nq > 0 && !hi) return fail(NDI_INVALID_ARGUMENT, "null pointer");
+    if (h->dtype != NDI_F32 && h->dtype != NDI_F64) return fail(NDI_UNSUPPORTED_DTYPE, "integrals need a float dtype");
+    if (kind == NDI_INTEGRAL_CUBIC && (mode < 0 || mode > 2)) return fail(NDI_INVALID_ARGUMENT, "bad extrapolation mode %d", mode);
+    if (!h->cum[kind])
+        return fail(NDI_NO_INTEGRAL, "no %s integral table: call ndi_interp1d_integral_build first%s",
+                    kind == NDI_INTEGRAL_CUBIC ? "cubic" : "linear", kind == NDI_INTEGRAL_CUBIC ? " (again after a new spline)" : "");
+    return NDI_OK;
+}
+
+// the value call's check of a query, for each bound
+static int integral_check(int kind, int32_t mode) {
+    if (kind == NDI_INTEGRAL_LINEAR) return mode ? CHECK_NOT_NAN : CHECK_IN_RANGE;
+    return mode == NDI_EXTRAP_NO ? CHECK_IN_RANGE : (mode == NDI_EXTRAP_YES ? CHECK_NOT_NAN : CHECK_FINITE_IF_OUTSIDE);
+}
+
+}  // extern "C"
+template <class T>
+static ndi_status integral_on_device(const ndi_interp1d* h, int kind, const SearchCfg& sc, const T* lo, const T* hi, int64_t nq,
+                                     int32_t mode, T* out, unsigned long long* err, cudaStream_t s) {
+    const bool cubic = kind == NDI_INTEGRAL_CUBIC;
+    CK(launch_interp1d_integral<T>((const T*)h->x, h->n, sc, (const T*)h->data, cubic ? (const T*)h->a : nullptr,
+                                   cubic ? (const T*)h->b : nullptr, (const T*)h->cum[kind], h->w, lo, hi, nq,
+                                   cubic ? mode : (mode != 0), out, err, s));
+    return NDI_OK;
+}
+extern "C" {
+
+static ndi_status integral_dev(const ndi_interp1d* h, int kind, const void* lo, const void* hi, int64_t nq, int32_t mode,
+                               void* out, uint64_t* err_word_dev, void* stream) {
+    ndi_status st = check_integral_args(h, lo, hi, nq, mode, kind, out); if (st != NDI_OK) return st;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (err_word_dev) CK(cudaMemsetAsync(err_word_dev, 0xff, sizeof(uint64_t), s));
+    return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
+        using T = decltype(tag);
+        SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
+        return integral_on_device<T>(h, kind, sc, (const T*)lo, (const T*)hi, nq, mode, (T*)out, (unsigned long long*)err_word_dev, s);
+    });
+}
+
+// one block of a host batch: two query arrays (lo, hi), error word 2 * query + bound, as Bilinear's
+static ndi_status integral_host(const ndi_interp1d* h, int kind, const void* lo, const void* hi, int64_t nq, int32_t mode, void* out,
+                                uint64_t* word, Phase phase, int64_t nvalid) {
+    HostEval he{h->device, elem_size(h->dtype), 2, h->w, {lo, hi}, nq, out, phase, nvalid};
+    const int check = integral_check(kind, mode);
+    return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
+        using T = decltype(tag);
+        SearchCfg sc = make_search(h->meta(), h->search_mode, nq, 0);
+        return run_host_eval(he,
+            [&](const void* q0, const void* q1, int64_t cnt, void* o, unsigned long long* err, cudaStream_t s) -> ndi_status {
+                return integral_on_device<T>(h, kind, sc, (const T*)q0, (const T*)q1, cnt, mode, (T*)o, err, s);
+            },
+            [&](const void* q0, const void* q1, int64_t cnt, unsigned long long* err, cudaStream_t s) -> ndi_status {
+                CK(launch_validate_bounds<T>((const T*)h->x, h->n, (const T*)q0, (const T*)q1, cnt, check, err, s));
+                return NDI_OK;
+            }, word);
+    });
+}
+
+static ndi_status integral_status(uint64_t word, int nan_only, int64_t* first_bad, int32_t* bad_bound) {
+    if (word == NDI_ERR_WORD_NONE) return NDI_OK;
+    const int64_t idx = (int64_t)(word >> 1);
+    const int bound = (int)(word & 1);
+    if (first_bad) *first_bad = idx;
+    if (bad_bound) *bad_bound = bound;
+    return nan_only ? fail(NDI_NAN_QUERY, "not implemented: failed to convert NaN to usize (query %lld)", (long long)idx)
+                    : fail(NDI_OUT_OF_BOUNDS, "%s of query %lld is not in range", bound ? "hi" : "lo", (long long)idx);
+}
+
+static ndi_status integral_call(const ndi_interp1d* h, int kind, const void* lo, const void* hi, int64_t nq, int32_t mode,
+                                void* out, int64_t* first_bad, int32_t* bad_bound) {
+    if (first_bad) *first_bad = -1;
+    if (bad_bound) *bad_bound = -1;
+    ndi_status st = check_integral_args(h, lo, hi, nq, mode, kind, out); if (st != NDI_OK) return st;
+    uint64_t word;
+    if ((st = integral_host(h, kind, lo, hi, nq, mode, out, &word, Phase::whole, 0)) != NDI_OK) return st;
+    return integral_status(word, mode, first_bad, bad_bound);
+}
+
+ndi_status ndi_interp1d_cubic_integral(const ndi_interp1d* h, const void* lo, const void* hi, int64_t nq, int32_t extrap_mode,
+                                       void* out, int64_t* first_bad, int32_t* bad_bound) {
+    return integral_call(h, NDI_INTEGRAL_CUBIC, lo, hi, nq, extrap_mode, out, first_bad, bad_bound);
+}
+ndi_status ndi_interp1d_cubic_integral_dev(const ndi_interp1d* h, const void* lo_dev, const void* hi_dev, int64_t nq,
+                                           int32_t extrap_mode, void* out_dev, uint64_t* err_word_dev, void* stream) {
+    return integral_dev(h, NDI_INTEGRAL_CUBIC, lo_dev, hi_dev, nq, extrap_mode, out_dev, err_word_dev, stream);
+}
+ndi_status ndi_interp1d_linear_integral(const ndi_interp1d* h, const void* lo, const void* hi, int64_t nq, int32_t extrapolate,
+                                        void* out, int64_t* first_bad, int32_t* bad_bound) {
+    return integral_call(h, NDI_INTEGRAL_LINEAR, lo, hi, nq, extrapolate, out, first_bad, bad_bound);
+}
+ndi_status ndi_interp1d_linear_integral_dev(const ndi_interp1d* h, const void* lo_dev, const void* hi_dev, int64_t nq,
+                                            int32_t extrapolate, void* out_dev, uint64_t* err_word_dev, void* stream) {
+    return integral_dev(h, NDI_INTEGRAL_LINEAR, lo_dev, hi_dev, nq, extrapolate, out_dev, err_word_dev, stream);
 }
 
 // ---- Interp2D ---------------------------------------------------------------------------------------------------
@@ -1769,6 +1908,29 @@ ndi_status ndi_interp1d_group_cubic_deriv(ndi_interp1d_group* g, const void* q, 
                               (unsigned char*)out + (size_t)lo * h->w * es, w, phase, nvalid, order);
         },
         [&](uint64_t word) { return eval1d_status(word, extrap_mode, first_bad); });
+}
+
+static ndi_status group_integral(ndi_interp1d_group* g, int kind, const void* lo, const void* hi, int64_t nq, int32_t mode,
+                                 void* out, int64_t* first_bad, int32_t* bad_bound) {
+    if (first_bad) *first_bad = -1;
+    if (bad_bound) *bad_bound = -1;
+    return group_call(g, nq, 2,
+        [&](const ndi_interp1d* h0) { return integral_call(h0, kind, lo, hi, nq, mode, out, first_bad, bad_bound); },
+        [&](const ndi_interp1d* h0) { return check_integral_args(h0, lo, hi, nq, mode, kind, out); },
+        [&](const ndi_interp1d* h, int64_t b0, int64_t cnt, Phase phase, int64_t nvalid, uint64_t* w) {
+            const size_t es = elem_size(h->dtype);
+            return integral_host(h, kind, (const unsigned char*)lo + (size_t)b0 * es, (const unsigned char*)hi + (size_t)b0 * es, cnt,
+                                 mode, (unsigned char*)out + (size_t)b0 * h->w * es, w, phase, nvalid);
+        },
+        [&](uint64_t word) { return integral_status(word, mode, first_bad, bad_bound); });
+}
+ndi_status ndi_interp1d_group_linear_integral(ndi_interp1d_group* g, const void* lo, const void* hi, int64_t nq, int32_t extrapolate,
+                                              void* out, int64_t* first_bad, int32_t* bad_bound) {
+    return group_integral(g, NDI_INTEGRAL_LINEAR, lo, hi, nq, extrapolate, out, first_bad, bad_bound);
+}
+ndi_status ndi_interp1d_group_cubic_integral(ndi_interp1d_group* g, const void* lo, const void* hi, int64_t nq, int32_t extrap_mode,
+                                             void* out, int64_t* first_bad, int32_t* bad_bound) {
+    return group_integral(g, NDI_INTEGRAL_CUBIC, lo, hi, nq, extrap_mode, out, first_bad, bad_bound);
 }
 
 ndi_status ndi_interp2d_replicate(const ndi_interp2d* h, const int32_t* devices, int32_t ndev, ndi_interp2d_group** out) {

@@ -789,6 +789,286 @@ __global__ void __launch_bounds__(kBlock) interp1d_linear_slope_kernel(const Eva
 }
 
 // ------------------------------------------------------------------------------------------------
+// K9c / K9l: definite integrals of the cubic spline / Linear (NOT in the reference; scipy's CubicSpline.integrate)
+// ------------------------------------------------------------------------------------------------
+// A query is a pair of bounds; each is checked as K5 / K3 check a query, searched like one (two searches in lock
+// step), and turned into four weights once per bound in the lane that owns the query (include/ndi_b200.h):
+//     F_i(x) = ((W0 y[i] + W1 y[i+1]) + W2 a[i]) + W3 b[i],   I(u, v) = ((C[j] - C[i]) + F_j(v)) - F_i(u)
+// The per-query record (weights, intervals, periodic terms) is written once per task to a per-warp slab of shared
+// memory; every lane of a query reads it from there (one broadcast read instead of a dozen shuffles).  K5's work
+// decomposition otherwise: thin rows with the next tile's bounds loaded ahead and one-interval tiles, wide rows in
+// slices with the gathered rows kept in registers.  On wide rows the rows of the upper bound become those of the next
+// query's lower bound without a load, and when that bound IS the previous upper bound (consecutive bins) its F is
+// reused as well.  f32 works on two columns per instruction; every sum of a product is done per half.
+template <class T>
+struct Integ1 {
+    const T* grid; int n; SearchCfg sc;
+    const T* data; const T* a; const T* b; const T* cum; long long w;
+    const T* lo; const T* hi; long long nq; int mode;
+    T* out; unsigned long long* err;
+    long long ntasks; int nslices;
+};
+
+// fl: 1 negate (hi < lo), 2 the upper bound lies across the end of the period, 4 the lower bound is the previous
+// query's upper bound.  il < 0: the query is not evaluated.
+template <class T> struct alignas(16) IntRec { T wl[4], wh[4]; T k; int il, ih, fl; };
+
+template <class T, bool CUBIC>
+__device__ __forceinline__ void integral_weights(T x, T xl, T xr, T (&W)[4]) {
+    const T h = Ar<T>::sub(xr, xl);
+    const T t = Ar<T>::div(Ar<T>::sub(x, xl), h);
+    const T tt = Ar<T>::mul(t, t);
+    const T c2 = Ar<T>::mul(tt, (T)0.5);
+    W[0] = Ar<T>::mul(h, Ar<T>::sub(t, c2));
+    W[1] = Ar<T>::mul(h, c2);
+    if constexpr (CUBIC) {
+        const T c3 = Ar<T>::div(Ar<T>::mul(tt, t), (T)3);
+        const T c4 = Ar<T>::mul(Ar<T>::mul(tt, tt), (T)0.25);
+        W[2] = Ar<T>::mul(h, Ar<T>::add(Ar<T>::sub(c2, Ar<T>::add(c3, c3)), c4));
+        W[3] = Ar<T>::mul(h, Ar<T>::sub(c3, c4));
+    }
+}
+
+// one bound, checked as the value call checks a query
+template <class T, bool CUBIC>
+__device__ __forceinline__ bool integral_bound_bad(T x, T g0, T gl, int mode) {
+    if constexpr (CUBIC) return cubic_prepare<T>(x, g0, gl, mode);
+    else return mode ? Ar<T>::is_nan(x) : !in_range(g0, gl, x);
+}
+
+// the two points the integral is evaluated between, whole periods k, flags 1 / 2 of IntRec::fl
+template <class T, bool CUBIC>
+__device__ __forceinline__ void integral_points(T lo, T hi, T g0, T gl, int mode, T& u, T& v, T& k, int& fl) {
+    fl = 0;
+    if (hi < lo) { const T s = lo; lo = hi; hi = s; fl = 1; }
+    u = lo; v = hi; k = (T)0;
+    if (CUBIC && mode == 2) {                                       // scipy's PPoly.integrate, periodic branch
+        const T P = Ar<T>::sub(gl, g0);
+        const T d = Ar<T>::sub(hi, lo);
+        const T left = rem_euclid<T>(d, P);
+        const T kq = Ar<T>::div(Ar<T>::sub(d, left), P);
+        if constexpr (std::is_same<T, float>::value) k = rintf(kq); else k = rint(kq);
+        cubic_prepare<T>(u, g0, gl, 2);                             // lo wrapped as K5 wraps a query
+        const T e = Ar<T>::add(u, left);
+        if (e <= gl) v = e;
+        else { v = Ar<T>::add(g0, Ar<T>::sub(e, gl)); fl |= 2; }
+    }
+}
+
+template <class T, int V>
+struct IRows { Vec<T, V> y0, y1, a, b, c; };
+
+template <class T, int V, bool CUBIC>
+__device__ __forceinline__ void ld_irows(const Integ1<T>& p, int i, long long col, IRows<T, V>& r) {
+    const long long ro = (long long)i * p.w + col;
+    r.y0 = ld_table<T, V>(p.data + ro);
+    r.y1 = ld_table<T, V>(p.data + ro + p.w);
+    if constexpr (CUBIC) {
+        r.a = ld_table<T, V>(p.a + ro);
+        r.b = ld_table<T, V>(p.b + ro);
+    }
+    r.c = ld_table<T, V>(p.cum + ro);
+}
+
+template <class T, int V, bool CUBIC>
+__device__ __forceinline__ Vec<T, V> integral_f(const IRows<T, V>& r, const T (&W)[4]) {
+    Vec<T, V> f;
+    if constexpr (std::is_same<T, float>::value && NDI_F32X2 && V % 2 == 0) {
+        const F2 w0 = F2::both(W[0]), w1 = F2::both(W[1]);
+#pragma unroll
+        for (int e = 0; e < V; e += 2) {
+            F2 s = add_halves(mul2(w0, F2{r.y0.v[e], r.y0.v[e + 1]}), mul2(w1, F2{r.y1.v[e], r.y1.v[e + 1]}));
+            if constexpr (CUBIC) {
+                s = add_halves(s, mul2(F2::both(W[2]), F2{r.a.v[e], r.a.v[e + 1]}));
+                s = add_halves(s, mul2(F2::both(W[3]), F2{r.b.v[e], r.b.v[e + 1]}));
+            }
+            f.v[e] = s.lo; f.v[e + 1] = s.hi;
+        }
+        return f;
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+        T s = Ar<T>::add(Ar<T>::mul(W[0], r.y0.v[e]), Ar<T>::mul(W[1], r.y1.v[e]));
+        if constexpr (CUBIC) s = Ar<T>::add(Ar<T>::add(s, Ar<T>::mul(W[2], r.a.v[e])), Ar<T>::mul(W[3], r.b.v[e]));
+        f.v[e] = s;
+    }
+    return f;
+}
+
+// ((C[j] (+ C[n-1] across the period's end) - C[i]) + F_hi) - F_lo, then k C[n-1] + . (periodic), then the sign
+template <class T, int V>
+__device__ __forceinline__ Vec<T, V> integral_combine(const Vec<T, V>& cl, const Vec<T, V>& ch, const Vec<T, V>& fl,
+                                                      const Vec<T, V>& fh, const Vec<T, V>& cn, int flags, bool periodic, T k) {
+    Vec<T, V> res;
+    if constexpr (std::is_same<T, float>::value && NDI_F32X2 && V % 2 == 0) {
+#pragma unroll
+        for (int e = 0; e < V; e += 2) {
+            const F2 n2{cn.v[e], cn.v[e + 1]};
+            F2 c{ch.v[e], ch.v[e + 1]};
+            if (flags & 2) c = add2(c, n2);
+            F2 r = sub2(add2(sub2(c, F2{cl.v[e], cl.v[e + 1]}), F2{fh.v[e], fh.v[e + 1]}), F2{fl.v[e], fl.v[e + 1]});
+            if (periodic) r = add_halves(mul2(F2::both(k), n2), r);
+            res.v[e] = (flags & 1) ? -r.lo : r.lo;
+            res.v[e + 1] = (flags & 1) ? -r.hi : r.hi;
+        }
+        return res;
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+        const T c = (flags & 2) ? Ar<T>::add(ch.v[e], cn.v[e]) : ch.v[e];
+        T r = Ar<T>::sub(Ar<T>::add(Ar<T>::sub(c, cl.v[e]), fh.v[e]), fl.v[e]);
+        if (periodic) r = Ar<T>::add(Ar<T>::mul(k, cn.v[e]), r);
+        res.v[e] = (flags & 1) ? -r : r;
+    }
+    return res;
+}
+
+template <class T, int V, int LPQ, bool CUBIC>
+__device__ __forceinline__ void integral_body(const Integ1<T>& p) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ uint64_t bar;
+    const GridView<T> g = make_grid_view<T>(p.grid, p.n, p.sc, smem_raw, &bar);
+    IntRec<T>* slab = reinterpret_cast<IntRec<T>*>(smem_raw + stage_bytes(p.sc, sizeof(T))) + (threadIdx.x >> 5) * 32;
+    const T g0 = g.g0, gl = g.gl;
+    const bool periodic = CUBIC && p.mode == 2;
+    const int lane = threadIdx.x & 31;
+    const long long nwarps = (long long)gridDim.x * kWarpsPerBlock;
+    const long long task0 = (long long)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+    T lo_ahead = g0, hi_ahead = g0;                           // thin rows: the next tile's bounds, loaded one tile ahead
+    if (LPQ < 32 && task0 < p.ntasks && task0 * 32 + lane < p.nq) {
+        lo_ahead = ld_query(p.lo + task0 * 32 + lane);
+        hi_ahead = ld_query(p.hi + task0 * 32 + lane);
+    }
+    for (long long task = task0; task < p.ntasks; task += nwarps) {
+        long long qbase; int slice = 0;
+        T xlo, xhi;
+        if constexpr (LPQ < 32) {
+            qbase = task * 32;
+            xlo = lo_ahead; xhi = hi_ahead;
+            const long long qn = (task + nwarps) * 32 + lane;
+            const bool more = task + nwarps < p.ntasks && qn < p.nq;
+            lo_ahead = more ? ld_query(p.lo + qn) : g0;
+            hi_ahead = more ? ld_query(p.hi + qn) : g0;
+        } else {
+            const long long tile = task / p.nslices;
+            slice = (int)(task - tile * p.nslices);
+            qbase = tile * 32;
+            const bool live = qbase + lane < p.nq;
+            xlo = live ? ld_query(p.lo + qbase + lane) : g0;
+            xhi = live ? ld_query(p.hi + qbase + lane) : g0;
+        }
+        const long long qi = qbase + lane;
+        const bool live = qi < p.nq;
+        const bool bad_lo = live && integral_bound_bad<T, CUBIC>(xlo, g0, gl, p.mode);
+        const bool bad_hi = live && integral_bound_bad<T, CUBIC>(xhi, g0, gl, p.mode);
+        if (slice == 0) report_first_bad(p.err, bad_lo || bad_hi, 2ull * (unsigned long long)qi + (bad_lo ? 0ull : 1ull));
+        const bool skip = !live || bad_lo || bad_hi;
+        T x[2], k; int fl;
+        integral_points<T, CUBIC>(xlo, xhi, g0, gl, p.mode, x[0], x[1], k, fl);
+        if (skip) x[0] = x[1] = g0;
+        int idx[2]; T xl[2], xr[2];
+        search_multi<T, 2>(g, x, idx, xl, xr);
+        IntRec<T> rec;
+        integral_weights<T, CUBIC>(x[0], xl[0], xr[0], rec.wl);
+        integral_weights<T, CUBIC>(x[1], xl[1], xr[1], rec.wh);
+        const T vprev = __shfl_up_sync(0xffffffffu, x[1], 1);
+        const int sprev = __shfl_up_sync(0xffffffffu, (int)skip, 1);
+        if (lane > 0 && !sprev && x[0] == vprev) fl |= 4;
+        rec.k = k; rec.il = skip ? -1 : idx[0]; rec.ih = idx[1]; rec.fl = fl;
+        slab[lane] = rec;
+        __syncwarp();
+        if constexpr (LPQ < 32) {
+            constexpr int QPR = 32 / LPQ;
+            const int sub = lane % LPQ, qsel = lane / LPQ;
+            const long long col = (long long)sub * V;
+            const bool colok = col < p.w;
+            Vec<T, V> cn;
+            if (periodic && colok) cn = ld_table<T, V>(p.cum + (long long)(p.n - 1) * p.w + col);
+            const int first = __ffs(__ballot_sync(0xffffffffu, !skip) | 0x80000000u) - 1;
+            const int il0 = __shfl_sync(0xffffffffu, idx[0], first), ih0 = __shfl_sync(0xffffffffu, idx[1], first);
+            const bool one_interval = LPQ > 1 && __all_sync(0xffffffffu, skip || (idx[0] == il0 && idx[1] == ih0));
+            IRows<T, V> L, H;
+            if (one_interval && colok) {
+                ld_irows<T, V, CUBIC>(p, il0, col, L);
+                if (ih0 == il0) H = L; else ld_irows<T, V, CUBIC>(p, ih0, col, H);
+            }
+#pragma unroll
+            for (int rd = 0; rd < LPQ; ++rd) {
+                const int src = rd * QPR + qsel;
+                const IntRec<T> rc = slab[src];
+                if (rc.il >= 0 && colok) {
+                    if (!one_interval) {
+                        ld_irows<T, V, CUBIC>(p, rc.il, col, L);
+                        if (rc.ih == rc.il) H = L; else ld_irows<T, V, CUBIC>(p, rc.ih, col, H);
+                    }
+                    st_stream<T, V>(p.out + (qbase + src) * p.w + col,
+                                    integral_combine<T, V>(L.c, H.c, integral_f<T, V, CUBIC>(L, rc.wl),
+                                                           integral_f<T, V, CUBIC>(H, rc.wh), cn, rc.fl, periodic, rc.k));
+                }
+            }
+        } else {
+            const long long col = ((long long)slice * 32 + lane) * V;
+            const bool colok = col < p.w;
+            Vec<T, V> cn;
+            if (periodic && colok) cn = ld_table<T, V>(p.cum + (long long)(p.n - 1) * p.w + col);
+            int curl = -1, curh = -1;
+            IRows<T, V> L, H;
+            Vec<T, V> fh;
+            const int nlive = (int)min((long long)32, p.nq - qbase);
+            for (int s = 0; s < nlive; ++s) {
+                const IntRec<T> rc = slab[s];
+                if (rc.il < 0 || !colok) continue;
+                if (rc.il != curl) {
+                    if (rc.il == curh) L = H; else ld_irows<T, V, CUBIC>(p, rc.il, col, L);
+                    curl = rc.il;
+                }
+                if (rc.ih != curh) {
+                    if (rc.ih == curl) H = L; else ld_irows<T, V, CUBIC>(p, rc.ih, col, H);
+                    curh = rc.ih;
+                }
+                const Vec<T, V> fl = (rc.fl & 4) ? fh : integral_f<T, V, CUBIC>(L, rc.wl);
+                fh = integral_f<T, V, CUBIC>(H, rc.wh);
+                st_stream<T, V>(p.out + (qbase + s) * p.w + col, integral_combine<T, V>(L.c, H.c, fl, fh, cn, rc.fl, periodic, rc.k));
+            }
+        }
+        __syncwarp();                                         // the slab is rewritten by the next task
+    }
+}
+
+template <class T, int V, int LPQ>
+__global__ void __launch_bounds__(kBlock) interp1d_cubic_integral_kernel(const Integ1<T> p) {
+    integral_body<T, V, LPQ, true>(p);
+}
+template <class T, int V, int LPQ>
+__global__ void __launch_bounds__(kBlock) interp1d_linear_integral_kernel(const Integ1<T> p) {
+    integral_body<T, V, LPQ, false>(p);
+}
+
+// pre-pass of the integral calls: each bound checked as the value call checks a query (K7's check on both)
+template <class T>
+__global__ void __launch_bounds__(kBlock) validate_bounds_kernel(const T* __restrict__ g, int n, const T* __restrict__ lo,
+                                                                 const T* __restrict__ hi, long long nq, int check,
+                                                                 unsigned long long* err) {
+    const T g0 = g[0], gl = g[n - 1];
+    auto bad = [&](T x) {
+        if (check == CHECK_IN_RANGE) return !in_range(g0, gl, x);
+        if (check == CHECK_NOT_NAN) return Ar<T>::is_nan(x);
+        return !in_range(g0, gl, x) && !Ar<T>::is_finite(x);
+    };
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long nq_pad = (nq + 31) & ~31ll;
+    unsigned long long first = ~0ull;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nq_pad; i += stride) {
+        if (i >= nq) continue;
+        const bool bl = bad(ld_query(lo + i)), bh = bad(ld_query(hi + i));
+        if (bl || bh) first = min(first, 2ull * (unsigned long long)i + (bl ? 0ull : 1ull));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) first = min(first, __shfl_xor_sync(0xffffffffu, first, o));
+    if ((threadIdx.x & 31) == 0 && first != ~0ull) atomicMin(err, first);
+}
+
+// ------------------------------------------------------------------------------------------------
 // K4: Bilinear::interp_into x batch (bilinear.rs:64-99)
 // ------------------------------------------------------------------------------------------------
 // Very thin rows (LPQ <= 2, e.g. C4: 8 f32 columns) are bound by gather latency: five resident blocks
@@ -1177,6 +1457,29 @@ cudaError_t launch_interp1d_linear_slope(const T* grid, int64_t n, SearchCfg sc,
 }
 
 template <class T>
+cudaError_t launch_interp1d_integral(const T* grid, int64_t n, SearchCfg sc, const T* data, const T* a, const T* b,
+                                     const T* cum, int64_t w, const T* lo, const T* hi, int64_t nq, int mode, T* out,
+                                     unsigned long long* err, cudaStream_t st) {
+    if (nq <= 0) return cudaSuccess;
+    Shape sh = pick_shape(w, nq, a ? pick_vec<T>(w, {data, a, b, cum, out}) : pick_vec<T>(w, {data, cum, out}), 1);
+    Integ1<T> p{grid, (int)n, sc, data, a, b, cum, (long long)w, lo, hi, (long long)nq, mode, out, err, sh.ntasks, sh.nslices};
+    const size_t smem = stage_bytes(sc, sizeof(T)) + (size_t)kBlock * sizeof(IntRec<T>);   // grid stage + record slabs
+    if (a) { NDI_VEC_SWITCH(interp1d_cubic_integral_kernel, T, sh, p, smem, st) }
+    NDI_VEC_SWITCH(interp1d_linear_integral_kernel, T, sh, p, smem, st)
+}
+
+template <class T>
+cudaError_t launch_validate_bounds(const T* grid, int64_t n, const T* lo, const T* hi, int64_t nq, int check,
+                                   unsigned long long* err, cudaStream_t st) {
+    if (nq <= 0) return cudaSuccess;
+    long long blocks = (nq + kBlock - 1) / kBlock;
+    long long cap = (long long)device_info().sm_count * 8;
+    validate_bounds_kernel<T><<<(int)(blocks < cap ? blocks : cap), kBlock, 0, st>>>(grid, (int)n, lo, hi, (long long)nq, check, err);
+    count_launch();
+    return cudaGetLastError();
+}
+
+template <class T>
 cudaError_t launch_interp2d_bilinear(const T* gx, int64_t n, SearchCfg scx, const T* gy, int64_t m, SearchCfg scy,
                                      const T* data, int64_t w, const T* qx, const T* qy, int64_t nq, int extrapolate,
                                      T* out, unsigned long long* err, const unsigned* perm, int fast_tables,
@@ -1248,5 +1551,13 @@ template cudaError_t launch_interp1d_cubic_deriv<float>(const float*, int64_t, S
 template cudaError_t launch_interp1d_cubic_deriv<double>(const double*, int64_t, SearchCfg, const double*, const double*,
                                                          const double*, int64_t, const double*, int64_t, int, int, double*,
                                                          unsigned long long*, cudaStream_t);
+#define NDI_INST_INTEGRAL(T)                                                                                           \
+    template cudaError_t launch_interp1d_integral<T>(const T*, int64_t, SearchCfg, const T*, const T*, const T*,       \
+                                                     const T*, int64_t, const T*, const T*, int64_t, int, T*,          \
+                                                     unsigned long long*, cudaStream_t);                               \
+    template cudaError_t launch_validate_bounds<T>(const T*, int64_t, const T*, const T*, int64_t, int,                \
+                                                   unsigned long long*, cudaStream_t);
+NDI_INST_INTEGRAL(float)
+NDI_INST_INTEGRAL(double)
 
 }  // namespace ndi

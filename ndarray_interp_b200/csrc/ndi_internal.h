@@ -71,6 +71,20 @@ cudaError_t launch_interp1d_cubic_deriv(const T* grid, int64_t n, SearchCfg sc, 
 template <class T>
 cudaError_t launch_interp1d_linear_slope(const T* grid, int64_t n, SearchCfg sc, const T* data, int64_t w, const T* q,
                                          int64_t nq, int extrapolate, T* out, unsigned long long* err, cudaStream_t st);
+// definite integrals (K9c / K9l) over the cumulative table C (ndi_integral.cu: K9b builds it); a == nullptr: Linear
+template <class T>
+cudaError_t launch_interp1d_integral(const T* grid, int64_t n, SearchCfg sc, const T* data, const T* a, const T* b,
+                                     const T* cum, int64_t w, const T* lo, const T* hi, int64_t nq, int mode, T* out,
+                                     unsigned long long* err, cudaStream_t st);
+// pre-pass of the integral calls: the value call's check on each bound, error word 2 * query + bound
+template <class T>
+cudaError_t launch_validate_bounds(const T* grid, int64_t n, const T* lo, const T* hi, int64_t nq, int check,
+                                   unsigned long long* err, cudaStream_t st);
+// scratch: integral_build_scratch(n, w) doubles
+size_t integral_build_scratch(int64_t n, int64_t w);
+template <class T>
+cudaError_t launch_integral_build(const T* x, int64_t n, const T* data, const T* a, const T* b, int64_t w, T* cum,
+                                  double* scratch, cudaStream_t st);
 template <class T>
 cudaError_t launch_interp2d_bilinear(const T* gx, int64_t n, SearchCfg scx, const T* gy, int64_t m, SearchCfg scy,
                                      const T* data, int64_t w, const T* qx, const T* qy, int64_t nq, int extrapolate,

@@ -9,6 +9,7 @@ that the reference runs around it (interp1d/mod.rs:300-343) is the method `inter
 whose default is that loop; the built-in strategies override it with one kernel launch.
 """
 import ctypes as C
+import threading
 
 import numpy as np
 
@@ -88,6 +89,11 @@ class Linear(Interp1DStrategyBuilder, Interp1DStrategy):
                  else (L.load().ndi_interp1d_linear_deriv, interpolator._handle()))
         st = L.check(fn(h, L.ptr(xs_flat), xs_flat.size, int(self._extrapolate), L.ptr(out_rows), C.byref(bad)))
         _raise_eval(st, xs_flat, bad.value, "x")
+
+    def integral_batch_into(self, interpolator, lo_flat, hi_flat, out_rows):
+        """NOT in the reference: integral from lo_flat[i] to hi_flat[i] of the piecewise linear interpolant, with
+        interp_batch_into's handling of each bound (include/ndi_b200.h: ndi_interp1d_linear_integral)"""
+        _integral_batch(interpolator, L.INTEGRAL_LINEAR, int(self._extrapolate), lo_flat, hi_flat, out_rows)
 
 
 # ---- CubicSpline -------------------------------------------------------------------------------------------
@@ -311,6 +317,12 @@ class CubicSplineStrategy(Interp1DStrategy):
         st = L.check(fn(h, L.ptr(xs_flat), xs_flat.size, self._mode, int(order), L.ptr(out_rows), C.byref(bad)))
         _raise_eval(st, xs_flat, bad.value, "x")
 
+    def integral_batch_into(self, interpolator, lo_flat, hi_flat, out_rows):
+        """NOT in the reference: integral from lo_flat[i] to hi_flat[i] of the spline, as scipy's
+        CubicSpline.integrate(a, b, extrapolate), with interp_batch_into's handling of each bound (include/ndi_b200.h:
+        ndi_interp1d_cubic_integral)"""
+        _integral_batch(interpolator, L.INTEGRAL_CUBIC, self._mode, lo_flat, hi_flat, out_rows)
+
 
 def _ndarray_debug(a):
     """`{:?}` of a 1-D C-contiguous ndarray view, as pinned by tests/cubic_spline_strat.rs:441-443"""
@@ -326,6 +338,20 @@ def _raise_eval(st, xs_flat, first_bad, name):
         raise InterpolateError.OutOfBounds(f"{name} = {rust_debug(xs_flat[first_bad])} is not in range")
     if st == L.NAN_QUERY:                                  # vector_extensions.rs:83-84
         raise Panic("not implemented: failed to convert NaN to usize")
+
+
+def _integral_batch(interpolator, kind, mode, lo_flat, hi_flat, out_rows):
+    interpolator.prepare_integral()
+    group = getattr(interpolator, "_group", None)
+    if group is not None:
+        fn, h = (L.load().ndi_interp1d_group_cubic_integral if kind == L.INTEGRAL_CUBIC
+                 else L.load().ndi_interp1d_group_linear_integral), group.ptr
+    else:
+        fn, h = (L.load().ndi_interp1d_cubic_integral if kind == L.INTEGRAL_CUBIC
+                 else L.load().ndi_interp1d_linear_integral), interpolator._handle()
+    bad, bound = C.c_int64(-1), C.c_int32(-1)
+    st = L.check(fn(h, L.ptr(lo_flat), L.ptr(hi_flat), lo_flat.size, mode, L.ptr(out_rows), C.byref(bad), C.byref(bound)))
+    _raise_eval(st, hi_flat if bound.value == 1 else lo_flat, bad.value, "x")
 
 
 def _single_into(strategy, interpolator, target, x):
@@ -391,6 +417,8 @@ class Interp1D:
     def __init__(self, x, data, strategy, _handle=None):
         self.x, self.data, self.strategy = x, data, strategy
         self._h = _handle
+        self._integral_lock = threading.Lock()
+        self._integral_tables = set()          # kinds of cumulative table built on the handle (ndi_interp1d_integral_build)
         if isinstance(strategy, Interp1DStrategy):
             strategy._bind(self)
 
@@ -415,6 +443,8 @@ class Interp1D:
             raise TypeError("only the built-in strategies run on the device")
         other = Interp1D.__new__(Interp1D)
         other.x, other.data, other.strategy, other._h = self.x, self.data, self.strategy, self._h
+        other._integral_lock = threading.Lock()
+        other._integral_tables = frozenset(self._integral_tables)    # the tables the devices received
         other._group = _Group(L.load().ndi_interp1d_replicate, L.load().ndi_interp1d_group_destroy, self._handle(), devices, self)
         return other
 
@@ -480,6 +510,49 @@ class Interp1D:
         if order not in ((1,) if isinstance(self.strategy, Linear) else (1, 2)):   # before any shape check
             raise ValueError(f"{type(self.strategy).__name__} has no derivative of order {order}")
         self._array_into(xs, buffer, lambda i, q, rows: self.strategy.deriv_batch_into(i, q, rows, order))
+
+    # -- definite integrals: NOT in the reference ------------------------------------------------------------------------
+    def integrate(self, a, b):
+        """NOT in the reference: the integral from `a` to `b` of the interpolant (scipy's CubicSpline.integrate); `a` and
+        `b` broadcast, so a scalar `a` and an array `b` give the antiderivative from `a` at every point of `b`"""
+        return self.interp_array_integral(a, b)
+
+    def interp_array_integral(self, a, b):
+        """NOT in the reference: integrals over all pairs of the broadcast of `a` and `b`, shaped
+        broadcast_shape ++ data.shape[1:]"""
+        shape = np.broadcast_shapes(np.shape(a), np.shape(b))
+        ys = np.zeros(self._buffer_shape(shape), dtype=self.data.dtype)
+        self.interp_array_integral_into(a, b, ys)
+        return ys
+
+    def interp_array_integral_into(self, a, b, buffer):
+        """NOT in the reference: like `interp_array_integral`, into the provided buffer; buffer layouts, errors and
+        untouched rows after a failing pair as `interp_array_into` (the failing bound's value is reported)"""
+        self._check_integral()
+        shape = np.broadcast_shapes(np.shape(a), np.shape(b))
+        lo = np.broadcast_to(np.asarray(a, dtype=self.data.dtype), shape)
+        hi = np.ascontiguousarray(np.broadcast_to(np.asarray(b, dtype=self.data.dtype), shape)).reshape(-1)
+        self._array_into(lo, buffer, lambda i, q, rows: self.strategy.integral_batch_into(i, q, hi, rows))
+
+    def prepare_integral(self):
+        """NOT in the reference: build the cumulative table the integral calls evaluate over (otherwise built on first
+        use).  On a replicated interpolator the table must have been built before `replicate`."""
+        self._check_integral()
+        kind = L.INTEGRAL_CUBIC if isinstance(self.strategy, CubicSplineStrategy) else L.INTEGRAL_LINEAR
+        with self._integral_lock:
+            if kind in self._integral_tables:
+                return
+            if getattr(self, "_group", None) is not None:
+                raise L.NdiLibraryError("this interpolator was replicated before its integral table was built: call "
+                                        "prepare_integral() on the source interpolator before replicate()")
+            L.check(L.load().ndi_interp1d_integral_build(self._handle(), kind))
+            self._integral_tables.add(kind)
+
+    def _check_integral(self):
+        if not _is_builtin(self.strategy):
+            raise TypeError("integrals are computed by the built-in strategies (Linear, CubicSpline) only")
+        if self.data.dtype.kind not in "f":
+            raise TypeError(f"integrals need float data (the integral of {self.data.dtype} data is not an integer)")
 
     def _array_into(self, xs, buffer, batch):
         xs = np.asarray(xs)

@@ -8,6 +8,10 @@ pub const NDI_OUT_OF_BOUNDS: ndi_status = 1;
 pub const NDI_NAN_QUERY: ndi_status = 2;
 pub const NDI_PERIODIC_MISMATCH: ndi_status = 3;
 pub const NDI_NOT_MONOTONIC: ndi_status = 5;
+pub const NDI_NO_INTEGRAL: ndi_status = 9;
+
+pub const NDI_INTEGRAL_LINEAR: i32 = 0;
+pub const NDI_INTEGRAL_CUBIC: i32 = 1;
 
 pub const NDI_F32: i32 = 0;
 pub const NDI_F64: i32 = 1;
@@ -45,6 +49,10 @@ extern "C" {
     /// derivatives (not in the reference): order 1 or 2 of the spline, the slope of Linear
     pub fn ndi_interp1d_cubic_deriv(h: *const ndi_interp1d, q: *const c_void, nq: i64, extrap_mode: i32, order: i32, out: *mut c_void, first_bad: *mut i64) -> ndi_status;
     pub fn ndi_interp1d_linear_deriv(h: *const ndi_interp1d, q: *const c_void, nq: i64, extrapolate: i32, out: *mut c_void, first_bad: *mut i64) -> ndi_status;
+    /// definite integrals (not in the reference): the cumulative table of one kind, then integrals over (lo, hi) pairs
+    pub fn ndi_interp1d_integral_build(h: *mut ndi_interp1d, kind: i32) -> ndi_status;
+    pub fn ndi_interp1d_cubic_integral(h: *const ndi_interp1d, lo: *const c_void, hi: *const c_void, nq: i64, extrap_mode: i32, out: *mut c_void, first_bad: *mut i64, bad_bound: *mut i32) -> ndi_status;
+    pub fn ndi_interp1d_linear_integral(h: *const ndi_interp1d, lo: *const c_void, hi: *const c_void, nq: i64, extrapolate: i32, out: *mut c_void, first_bad: *mut i64, bad_bound: *mut i32) -> ndi_status;
 
     pub fn ndi_interp1d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp1d) -> ndi_status;
     pub fn ndi_interp2d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, y: *const c_void, m: i64, y_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp2d) -> ndi_status;

@@ -6,7 +6,7 @@ use std::{ffi::c_void, fmt::Debug};
 use ndarray::{Array, ArrayBase, ArrayViewMut, Axis, Data, Dimension, Ix1, RemoveAxis};
 use num_traits::{Euclid, Float};
 
-use super::{eval_result, DeviceTable1D, Interp1D, Interp1DDerivStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
+use super::{eval_result, integral_result, DeviceTable1D, Interp1D, Interp1DDerivStrategy, Interp1DIntegralStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
 use crate::{ffi, BuilderError, InterpolateError, NdiElem};
 
 /// element types usable with the CubicSpline strategy (float only, like the reference's `SplineNum`)
@@ -278,5 +278,32 @@ where
             )
         };
         eval_result(st, xs, first_bad, "x")
+    }
+}
+
+/// NOT in the reference: the integral of the spline between two bounds (scipy's `CubicSpline.integrate`)
+impl<Sd, Sx, D> Interp1DIntegralStrategy<Sd, Sx, D> for CubicSplineStrategy<Sd, D>
+where
+    Sd: Data,
+    Sd::Elem: SplineNum,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+{
+    const INTEGRAL_KIND: i32 = ffi::NDI_INTEGRAL_CUBIC;
+    fn integral_batch_into(&self, interp: &Interp1D<Sd, Sx, D, Self>, lo: &[Sd::Elem], hi: &[Sd::Elem], out: &mut [Sd::Elem]) -> Result<(), InterpolateError> {
+        let (mut first_bad, mut bad_bound) = (-1i64, -1i32);
+        let st = unsafe {
+            ffi::ndi_interp1d_cubic_integral(
+                interp.table.0,
+                lo.as_ptr() as *const c_void,
+                hi.as_ptr() as *const c_void,
+                lo.len() as i64,
+                self.extrapolate as i32,
+                out.as_mut_ptr() as *mut c_void,
+                &mut first_bad,
+                &mut bad_bound,
+            )
+        };
+        integral_result(st, lo, hi, first_bad, bad_bound)
     }
 }

@@ -3,7 +3,7 @@ use std::ffi::c_void;
 
 use ndarray::{ArrayBase, ArrayViewMut, Data, Dimension, Ix1, RemoveAxis};
 
-use super::{eval_result, Interp1D, Interp1DDerivStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
+use super::{eval_result, integral_result, Interp1D, Interp1DDerivStrategy, Interp1DIntegralStrategy, Interp1DStrategy, Interp1DStrategyBuilder};
 use crate::{ffi, BuilderError, InterpolateError, NdiElem};
 
 /// Linear Interpolation Strategy
@@ -112,5 +112,32 @@ where
             )
         };
         eval_result(st, xs, first_bad, "x")
+    }
+}
+
+/// NOT in the reference: the integral of the piecewise linear interpolant between two bounds
+impl<Sd, Sx, D> Interp1DIntegralStrategy<Sd, Sx, D> for Linear
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+{
+    const INTEGRAL_KIND: i32 = ffi::NDI_INTEGRAL_LINEAR;
+    fn integral_batch_into(&self, interpolator: &Interp1D<Sd, Sx, D, Self>, lo: &[Sd::Elem], hi: &[Sd::Elem], out: &mut [Sd::Elem]) -> Result<(), InterpolateError> {
+        let (mut first_bad, mut bad_bound) = (-1i64, -1i32);
+        let st = unsafe {
+            ffi::ndi_interp1d_linear_integral(
+                interpolator.table.0,
+                lo.as_ptr() as *const c_void,
+                hi.as_ptr() as *const c_void,
+                lo.len() as i64,
+                self.extrapolate as i32,
+                out.as_mut_ptr() as *mut c_void,
+                &mut first_bad,
+                &mut bad_bound,
+            )
+        };
+        integral_result(st, lo, hi, first_bad, bad_bound)
     }
 }

@@ -38,6 +38,27 @@ where
     fn deriv_batch_into(&self, interpolator: &Interp1D<Sd, Sx, D, Self>, xs: &[Sd::Elem], out: &mut [Sd::Elem], order: i32) -> Result<(), InterpolateError>;
 }
 
+/// NOT in the reference: definite integrals of an interpolant, computed on the device (`ndi_interp1d_*_integral`, scipy's
+/// `CubicSpline.integrate`).  A trait of its own, like [`Interp1DDerivStrategy`]; implemented by the built-in
+/// strategies for float data.
+pub trait Interp1DIntegralStrategy<Sd, Sx, D>
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+    Self: Sized,
+{
+    /// which cumulative table the strategy evaluates over (`ffi::NDI_INTEGRAL_LINEAR` / `ffi::NDI_INTEGRAL_CUBIC`)
+    const INTEGRAL_KIND: i32;
+    /// integral from `lo[i]` to `hi[i]` into the rows of `out`, each bound handled as
+    /// [`Interp1DStrategy::interp_batch_into`] handles a query (the failing bound's value is reported).
+    ///
+    /// # panics
+    /// When [`Interp1D::prepare_integral`] has not built the table
+    fn integral_batch_into(&self, interpolator: &Interp1D<Sd, Sx, D, Self>, lo: &[Sd::Elem], hi: &[Sd::Elem], out: &mut [Sd::Elem]) -> Result<(), InterpolateError>;
+}
+
 /// Owner of the opaque device handle (grid, data, spline coefficients in HBM).
 /// Immutable after build, so it is shared freely between threads like the reference's `&self`.
 #[derive(Debug)]
@@ -346,6 +367,64 @@ where
             }
         }
     }
+}
+
+/// NOT in the reference: definite integrals (see [`Interp1DIntegralStrategy`])
+impl<Sd, Sx, D, Strat> Interp1D<Sd, Sx, D, Strat>
+where
+    Sd: Data,
+    Sd::Elem: NdiElem,
+    Sx: Data<Elem = Sd::Elem>,
+    D: Dimension + RemoveAxis,
+    Strat: Interp1DStrategy<Sd, Sx, D> + Interp1DIntegralStrategy<Sd, Sx, D>,
+{
+    /// build the cumulative table the integral methods evaluate over; it changes the device handle, hence `&mut self`
+    ///
+    /// # panics
+    /// For integer data (the integral of integer data is not an integer)
+    pub fn prepare_integral(&mut self) {
+        let st = unsafe { ffi::ndi_interp1d_integral_build(self.table.0, Strat::INTEGRAL_KIND) };
+        assert!(st == ffi::NDI_OK, "ndi_interp1d_integral_build failed ({st}): {}", ffi::last_error());
+    }
+
+    /// the integral from `a` to `b`, one dimension smaller than the data
+    pub fn integrate(&self, a: Sx::Elem, b: Sx::Elem) -> Result<Array<Sd::Elem, D::Smaller>, InterpolateError> {
+        let mut target = Array::zeros(self.data.raw_dim().remove_axis(Axis(0)));
+        let out = target.as_slice_mut().unwrap_or_else(|| unreachable!());
+        self.strategy.integral_batch_into(self, &[a], &[b], out).map(|_| target)
+    }
+
+    /// integrals over the pairs of `lo` and `hi` (one shape); output shape = `lo.shape() ++ data.shape()[1..]`
+    ///
+    /// # panics
+    /// When `lo` and `hi` differ in shape
+    pub fn interp_array_integral<Sq, Dq>(
+        &self,
+        lo: &ArrayBase<Sq, Dq>,
+        hi: &ArrayBase<Sq, Dq>,
+    ) -> Result<Array<Sd::Elem, <Dq as DimAdd<D::Smaller>>::Output>, InterpolateError>
+    where
+        Sq: Data<Elem = Sd::Elem>,
+        Dq: Dimension + DimAdd<D::Smaller>,
+    {
+        assert!(lo.shape() == hi.shape(), "lo and hi need the same shape: {:?}, {:?}", lo.shape(), hi.shape());
+        let mut shape = <Dq as DimAdd<D::Smaller>>::Output::zeros(lo.ndim() + self.data.ndim() - 1);
+        for (dst, src) in shape.slice_mut().iter_mut().zip(lo.shape().iter().chain(self.data.shape()[1..].iter())) {
+            *dst = *src;
+        }
+        let mut ys = Array::zeros(shape);
+        let (l, h) = (lo.as_standard_layout(), hi.as_standard_layout());
+        let out = ys.as_slice_mut().unwrap_or_else(|| unreachable!());
+        self.strategy
+            .integral_batch_into(self, l.as_slice().unwrap_or_else(|| unreachable!()), h.as_slice().unwrap_or_else(|| unreachable!()), out)
+            .map(|_| ys)
+    }
+}
+
+/// map the status of an integral call (first failing query and bound) to the reference's error / panic
+pub(crate) fn integral_result<T: Debug>(st: ffi::ndi_status, lo: &[T], hi: &[T], first_bad: i64, bad_bound: i32) -> Result<(), InterpolateError> {
+    assert!(st != ffi::NDI_NO_INTEGRAL, "no integral table: call Interp1D::prepare_integral first");
+    eval_result(st, if bad_bound == 1 { hi } else { lo }, first_bad, "x")
 }
 
 /// upload of `(x, data)` as the views lie in memory (any strides: the library makes them dense on the device,
