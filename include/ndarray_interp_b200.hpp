@@ -392,6 +392,70 @@ private:
     BoundaryCondition<T> boundary_ = BoundaryCondition<T>::NotAKnot();
 };
 
+// ---- shape-preserving cubics: NOT in the reference (ndi_interp1d_hermite_build; scipy's PchipInterpolator,
+// Akima1DInterpolator and CubicHermiteSpline).  The strategy is a CubicSplineStrategy whose coefficients come from knot
+// slopes computed on the device, so values, derivatives and integrals are evaluated exactly as for the spline.
+template <class T>
+class HermiteStrategy : public CubicSplineStrategy<T> {
+public:
+    HermiteStrategy(int kind, std::vector<T> dydx, int mode)
+        : CubicSplineStrategy<T>(BoundaryCondition<T>::NotAKnot(), mode), kind_(kind), dydx_(std::move(dydx)) {}
+    void bind(const Interp1D<T>& ip) const override;
+private:
+    int kind_;
+    std::vector<T> dydx_;                                    // NDI_HERMITE_GIVEN: the slopes, shaped like the data
+};
+namespace detail {
+template <class T, class Self>
+class HermiteBuilder : public Interp1DStrategyBuilder<T> {
+    static_assert(std::is_floating_point<T>::value, "cubic Hermite interpolants need a float element type");
+public:
+    static Self new_() { return Self(); }
+    Self extrapolate(bool e) const { Self s(static_cast<const Self&>(*this)); s.extrapolate_ = e; return s; }   // default false
+    size_t MINIMUM_DATA_LENGHT() const override { return 2; }
+protected:
+    std::shared_ptr<const Interp1DStrategy<T>> make(int kind, std::vector<T> dydx = {}) const {
+        return std::make_shared<HermiteStrategy<T>>(kind, std::move(dydx), extrapolate_ ? NDI_EXTRAP_YES : NDI_EXTRAP_NO);
+    }
+    bool extrapolate_ = false;
+};
+}  // namespace detail
+template <class T>
+class Pchip : public detail::HermiteBuilder<T, Pchip<T>> {
+public:
+    std::shared_ptr<const Interp1DStrategy<T>> build(const ArrayView<T>&, const ArrayView<T>&) const override {
+        return this->make(NDI_HERMITE_PCHIP);
+    }
+};
+template <class T>
+class Akima : public detail::HermiteBuilder<T, Akima<T>> {
+public:
+    // "akima" (default) or "makima"; std::invalid_argument otherwise
+    Akima method(const std::string& m) const {
+        if (m != "akima" && m != "makima") throw std::invalid_argument("Akima method must be \"akima\" or \"makima\", got " + m);
+        Akima a(*this); a.makima_ = m == "makima"; return a;
+    }
+    std::shared_ptr<const Interp1DStrategy<T>> build(const ArrayView<T>&, const ArrayView<T>&) const override {
+        return this->make(makima_ ? NDI_HERMITE_MAKIMA : NDI_HERMITE_AKIMA);
+    }
+private:
+    bool makima_ = false;
+};
+template <class T>
+class CubicHermite : public detail::HermiteBuilder<T, CubicHermite<T>> {
+public:
+    CubicHermite() = default;
+    static CubicHermite new_(Array<T> dydx) { CubicHermite c; c.dydx_ = std::move(dydx); return c; }   // slopes shaped like the data
+    std::shared_ptr<const Interp1DStrategy<T>> build(const ArrayView<T>&, const ArrayView<T>& data) const override {
+        if (dydx_.shape() != data.shape)
+            throw BuilderError(BuilderError::ShapeError, "dydx has wrong shape. Expected: " + detail::shape_str(data.shape) +
+                               ", got: " + detail::shape_str(dydx_.shape()));
+        return this->make(NDI_HERMITE_GIVEN, std::vector<T>(dydx_.data(), dydx_.data() + dydx_.size()));
+    }
+private:
+    Array<T> dydx_;
+};
+
 template <class T> class Interp1DBuilder;
 
 // One dimensional interpolator (src/interp1d/mod.rs:38-51)
@@ -680,6 +744,10 @@ std::pair<Array<T>, Array<T>> CubicSplineStrategy<T>::coefficients(const Interp1
     Array<T> a = Array<T>::zeros(sh), b = Array<T>::zeros(sh);
     detail::check(ndi_interp1d_spline_coeffs(ip.handle(), a.data(), b.data()));
     return {std::move(a), std::move(b)};
+}
+template <class T>
+void HermiteStrategy<T>::bind(const Interp1D<T>& ip) const {
+    detail::check(ndi_interp1d_hermite_build(ip.handle(), kind_, kind_ == NDI_HERMITE_GIVEN ? dydx_.data() : nullptr, 0));
 }
 
 // ---- 2-D (src/interp2d) ----------------------------------------------------------------------------------------

@@ -283,6 +283,39 @@ ndi_status ndi_interp1d_linear_integral(const ndi_interp1d* h, const void* lo, c
 ndi_status ndi_interp1d_linear_integral_dev(const ndi_interp1d* h, const void* lo_dev, const void* hi_dev, int64_t nq,
                                             int32_t extrapolate, void* out_dev, uint64_t* err_word_dev, void* stream);
 
+/* ---- shape-preserving cubics (NOT in the reference; scipy's PchipInterpolator, Akima1DInterpolator and
+ * CubicHermiteSpline) --------------------------------------------------------------------------------------- */
+/* Builds the handle's cubic coefficients from knot slopes d (n, w) instead of the spline's tridiagonal solve:
+ *     a[i] = d[i] h - dy,  b[i] = dy - d[i+1] h,   h = x[i+1] - x[i],  dy = y[i+1] - y[i]
+ * so the cubic value, derivative and integral calls (and their _dev and group forms) evaluate the piecewise cubic
+ * Hermite interpolant with these slopes.  Every operation is rounded on its own in the handle's dtype, in scipy's
+ * order (scipy 1.18, interpolate/_cubic.py), so in f64 the slopes are scipy's bit for bit.  Segment slopes
+ * m[k] = (y[k+1] - y[k]) / h[k], k = 0 .. n-2; sign() is numpy's (sign(+-0) = 0, sign(NaN) = NaN, unequal to all).
+ *   NDI_HERMITE_PCHIP   n == 2: d[0] = d[1] = m[0].  Interior knot k: d[k] = 0 if sign(m[k-1]) != sign(m[k]) or
+ *                       m[k] == 0 or m[k-1] == 0, else, with w1 = 2 h[k] + h[k-1], w2 = h[k] + 2 h[k-1],
+ *                       d[k] = 1 / ((w1 / m[k-1] + w2 / m[k]) / (w1 + w2)).  Ends: e = ((2 h0 + h1) m0 - h0 m1) / (h0 + h1);
+ *                       d = 0 if sign(e) != sign(m0), else 3 m0 if sign(m0) != sign(m1) and |e| > 3 |m0|, else e;
+ *                       (h0, h1, m0, m1) = (h[0], h[1], m[0], m[1]) on the left, (h[n-2], h[n-3], m[n-2], m[n-3]) on
+ *                       the right.
+ *   NDI_HERMITE_AKIMA   n == 2: d[0] = d[1] = m[0].  Otherwise m[-1] = 2 m[0] - m[1], m[-2] = 2 m[-1] - m[0],
+ *   NDI_HERMITE_MAKIMA  m[n-1] = 2 m[n-2] - m[n-3], m[n] = 2 m[n-1] - m[n-2]; at knot i f1 = |m[i+1] - m[i]|,
+ *                       f2 = |m[i-1] - m[i-2]| (makima adds 0.5 |m[i+1] + m[i]| to f1 and 0.5 |m[i-1] + m[i-2]| to
+ *                       f2), f12 = f1 + f2;  d[i] = m[i-1] + (f2 / f12) (m[i] - m[i-1]) if f12 > 1e-9 M, else
+ *                       0.5 (m[i+1] + m[i-2]), where M is the maximum of f12 over the whole table (all knots, all
+ *                       columns), NaN if any f12 is NaN.
+ *   NDI_HERMITE_GIVEN   d = dydx, (n, w) in the handle's dtype: host memory, or device memory on the handle's device
+ *                       with NDI_DEVICE_POINTERS in flags (read in place during the call, not kept).
+ * n >= 2.  Integer dtypes give NDI_UNSUPPORTED_DTYPE; another kind, GIVEN without dydx, or dydx with another kind
+ * NDI_INVALID_ARGUMENT.  Like ndi_interp1d_spline_build the call changes the handle and must not run concurrently
+ * with any other call on it; a failed build keeps the previous coefficients, a successful one drops the cubic integral
+ * table.  ndi_interp1d_build_info then reports NDI_BUILD_INFO_HERMITE + kind.  Build before replicating. */
+#define NDI_HERMITE_PCHIP 0
+#define NDI_HERMITE_AKIMA 1
+#define NDI_HERMITE_MAKIMA 2
+#define NDI_HERMITE_GIVEN 3
+#define NDI_BUILD_INFO_HERMITE 1000
+ndi_status ndi_interp1d_hermite_build(ndi_interp1d* h, int32_t kind, const void* dydx, uint32_t flags);
+
 /* ---- src/interp2d ------------------------------------------------------------------------ */
 /* Interp2DBuilder::build data upload (interp2d/mod.rs:468-518).  x: n, y: m, data: (n, m, w).
  * NDI_NOT_MONOTONIC reports the failing axis in the message ("x-axis" before "y-axis"). */

@@ -22,6 +22,8 @@ EXTRAP_NO, EXTRAP_YES, EXTRAP_PERIODIC = 0, 1, 2
 BIN_AUTO, BIN_OFF, BIN_ON, BIN_SWEEP = 0, 1, 2, 3
 BUILD_AUTO, BUILD_SEQUENTIAL, BUILD_ROWSPLIT, BUILD_PARTITION = 0, 1, 2, 3
 INTEGRAL_LINEAR, INTEGRAL_CUBIC = 0, 1
+HERMITE_PCHIP, HERMITE_AKIMA, HERMITE_MAKIMA, HERMITE_GIVEN = 0, 1, 2, 3
+BUILD_INFO_HERMITE = 1000
 ERR_WORD_NONE = 2 ** 64 - 1
 
 DTYPES = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.int32): I32,
@@ -66,6 +68,7 @@ SIGNATURES = {
     "ndi_interp1d_cubic_integral_dev": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp]),
     "ndi_interp1d_linear_integral": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _pi64, _pi32]),
     "ndi_interp1d_linear_integral_dev": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "ndi_interp1d_hermite_build": (_i32, [_vp, _i32, _vp, _u32]),
     "ndi_interp2d_create": (_i32, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _u32, C.POINTER(_vp)]),
     "ndi_interp2d_create_strided": (_i32, [_i32, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _u32,
                                            C.POINTER(_vp)]),

@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libndi_b200.so")
-SOURCES = ["ndi_api.cu", "ndi_eval.cu", "ndi_bin.cu", "ndi_sweep.cu", "ndi_grid.cu", "ndi_spline.cu", "ndi_rowsplit.cu", "ndi_partition.cu", "ndi_integral.cu"]
+SOURCES = ["ndi_api.cu", "ndi_eval.cu", "ndi_bin.cu", "ndi_sweep.cu", "ndi_grid.cu", "ndi_spline.cu", "ndi_rowsplit.cu", "ndi_partition.cu", "ndi_integral.cu", "ndi_hermite.cu"]
 HEADERS = ["ndi_device.cuh", "ndi_spline.cuh", "ndi_internal.h", os.path.join("..", "..", "include", "ndi_b200.h")]
 
 NVCC_FLAGS = [

@@ -1205,6 +1205,49 @@ ndi_status ndi_interp1d_spline_build(ndi_interp1d* h, int32_t bc_kind, const int
     });
 }
 
+ndi_status ndi_interp1d_hermite_build(ndi_interp1d* h, int32_t kind, const void* dydx, uint32_t flags) {
+    if (!h) return fail(NDI_INVALID_ARGUMENT, "null handle");
+    if (h->dtype != NDI_F32 && h->dtype != NDI_F64) return fail(NDI_UNSUPPORTED_DTYPE, "cubic interpolants need a float dtype");
+    if (kind < NDI_HERMITE_PCHIP || kind > NDI_HERMITE_GIVEN) return fail(NDI_INVALID_ARGUMENT, "bad Hermite kind %d", kind);
+    if ((kind == NDI_HERMITE_GIVEN) != (dydx != nullptr))
+        return fail(NDI_INVALID_ARGUMENT, kind == NDI_HERMITE_GIVEN ? "given slopes need dydx" : "dydx is only read for given slopes");
+    if (h->n < 2) return fail(NDI_INVALID_ARGUMENT, "The chosen Interpolation strategy needs at least 2 data points");
+    DeviceGuard g(h->device);
+    ndi_status st; Workspace* ws = workspace(h->device, &st); if (!ws) return st;
+    // Akima's maximum: two words of the per-thread build buffer
+    if ((st = grow(&ws->d_build, &ws->d_build_cap, 2 * sizeof(unsigned long long))) != NDI_OK) return st;
+    cudaStream_t bs = ws->s[0];
+    const size_t es = elem_size(h->dtype), coef_bytes = (size_t)(h->n - 1) * h->w * es;
+    // a / b (and host slopes) from the stream-ordered pool, as in ndi_interp1d_spline_build: the previous pair stays
+    // valid until this build has succeeded
+    void *a = nullptr, *b = nullptr, *slopes = nullptr;
+    const void* d = dydx;
+    auto body = [&]() -> ndi_status {
+        CK(cudaMallocAsync(&a, coef_bytes, bs));
+        CK(cudaMallocAsync(&b, coef_bytes, bs));
+        if (dydx && !(flags & NDI_DEVICE_POINTERS)) {
+            CK(cudaMallocAsync(&slopes, (size_t)h->n * h->w * es, bs));
+            CK(cudaMemcpyAsync(slopes, dydx, (size_t)h->n * h->w * es, cudaMemcpyHostToDevice, bs));
+            d = slopes;
+        }
+        return dispatch_float(h->dtype, [&](auto tag) -> ndi_status {
+            using T = decltype(tag);
+            CK(launch_hermite_build<T>(kind, (const T*)h->x, h->n, (const T*)h->data, h->w, (const T*)d,
+                                       (unsigned long long*)ws->d_build, (T*)a, (T*)b, bs));
+            CK(cudaStreamSynchronize(bs));
+            return NDI_OK;
+        });
+    };
+    st = body();
+    if (slopes) cudaFreeAsync(slopes, bs);
+    if (st != NDI_OK) { cudaFreeAsync(a, bs); cudaFreeAsync(b, bs); cudaStreamSynchronize(bs); cudaGetLastError(); return st; }
+    if (h->owns_coeffs) { cudaFreeAsync(h->a, bs); cudaFreeAsync(h->b, bs); }
+    h->a = a; h->b = b; h->owns_coeffs = true;
+    drop_cubic_integral(h);
+    h->built_levels = NDI_BUILD_INFO_HERMITE + kind;
+    return NDI_OK;
+}
+
 ndi_status ndi_interp1d_set_build_mode(ndi_interp1d* h, int32_t mode, int32_t levels) {
     if (!h || mode < NDI_BUILD_AUTO || mode > NDI_BUILD_PARTITION || levels < 0) return fail(NDI_INVALID_ARGUMENT, "bad build mode");
     h->build_mode = mode; h->build_levels = levels;

@@ -85,6 +85,11 @@ size_t integral_build_scratch(int64_t n, int64_t w);
 template <class T>
 cudaError_t launch_integral_build(const T* x, int64_t n, const T* data, const T* a, const T* b, int64_t w, T* cum,
                                   double* scratch, cudaStream_t st);
+// knot slopes and cubic coefficients of a shape-preserving cubic (K10, ndi_hermite.cu); kind: NDI_HERMITE_*,
+// dydx: device slopes (n, w) for NDI_HERMITE_GIVEN, else nullptr; mx: two zeroable device words (Akima's maximum)
+template <class T>
+cudaError_t launch_hermite_build(int kind, const T* x, int64_t n, const T* data, int64_t w, const T* dydx,
+                                 unsigned long long* mx, T* a, T* b, cudaStream_t st);
 template <class T>
 cudaError_t launch_interp2d_bilinear(const T* gx, int64_t n, SearchCfg scx, const T* gy, int64_t m, SearchCfg scy,
                                      const T* data, int64_t w, const T* qx, const T* qy, int64_t nq, int extrapolate,

@@ -18,7 +18,8 @@ from .errors import BuilderError, InterpolateError, Panic, rust_debug
 from .vector_extensions import Monotonic, get_lower_index, monotonic_prop
 
 __all__ = ["Interp1D", "Interp1DBuilder", "Interp1DStrategy", "Interp1DStrategyBuilder", "Linear", "CubicSpline",
-           "CubicSplineStrategy", "BoundaryCondition", "RowBoundary", "SingleBoundary"]
+           "CubicSplineStrategy", "BoundaryCondition", "RowBoundary", "SingleBoundary", "Pchip", "Akima", "CubicHermite",
+           "HermiteStrategy"]
 
 
 # ---- plugin boundary ---------------------------------------------------------------------------------
@@ -322,6 +323,94 @@ class CubicSplineStrategy(Interp1DStrategy):
         CubicSpline.integrate(a, b, extrapolate), with interp_batch_into's handling of each bound (include/ndi_b200.h:
         ndi_interp1d_cubic_integral)"""
         _integral_batch(interpolator, L.INTEGRAL_CUBIC, self._mode, lo_flat, hi_flat, out_rows)
+
+
+# ---- shape-preserving cubics: NOT in the reference ---------------------------------------------------------------
+class _HermiteBuilder(Interp1DStrategyBuilder):
+    """common part of Pchip, Akima and CubicHermite: a C1 piecewise cubic from knot slopes computed on the device
+    (include/ndi_b200.h: ndi_interp1d_hermite_build), evaluated exactly like a CubicSpline"""
+    MINIMUM_DATA_LENGHT = 2
+
+    def __init__(self):
+        self._extrapolate = False
+
+    @classmethod
+    def new(cls):
+        return cls()
+
+    def extrapolate(self, extrapolate):
+        """does the strategy extrapolate (the edge intervals' polynomials)? Default is `false`"""
+        self._extrapolate = bool(extrapolate)
+        return self
+
+    def _kind(self):
+        raise NotImplementedError
+
+    def build(self, x, data):
+        if not np.issubdtype(data.dtype, np.floating):
+            raise TypeError(f"{type(self).__name__} needs a float element type")
+        return HermiteStrategy(self._kind(), None, L.EXTRAP_YES if self._extrapolate else L.EXTRAP_NO)
+
+
+class Pchip(_HermiteBuilder):
+    """NOT in the reference: the monotonicity-preserving cubic of scipy's PchipInterpolator"""
+
+    def _kind(self):
+        return L.HERMITE_PCHIP
+
+
+class Akima(_HermiteBuilder):
+    """NOT in the reference: scipy's Akima1DInterpolator, method "akima" (default) or "makima" """
+
+    def __init__(self):
+        super().__init__()
+        self._method = "akima"
+
+    def method(self, method):
+        if method not in ("akima", "makima"):
+            raise ValueError(f'Akima method must be "akima" or "makima", got {method!r}')
+        self._method = method
+        return self
+
+    def _kind(self):
+        return L.HERMITE_AKIMA if self._method == "akima" else L.HERMITE_MAKIMA
+
+
+class CubicHermite(_HermiteBuilder):
+    """NOT in the reference: scipy's CubicHermiteSpline(x, y, dydx) -- the slopes at the knots are given, shaped like
+    the data"""
+
+    def __init__(self, dydx):
+        super().__init__()
+        self._dydx = np.asarray(dydx)
+
+    @classmethod
+    def new(cls, dydx):
+        return cls(dydx)
+
+    def _kind(self):
+        return L.HERMITE_GIVEN
+
+    def build(self, x, data):
+        if self._dydx.shape != data.shape:
+            raise BuilderError.ShapeError(
+                f"dydx has wrong shape. Expected: {list(data.shape)}, got: {list(self._dydx.shape)}")
+        strat = super().build(x, data)
+        strat._dydx = np.ascontiguousarray(self._dydx, dtype=data.dtype)
+        return strat
+
+
+class HermiteStrategy(CubicSplineStrategy):
+    """the strategy Pchip, Akima and CubicHermite build: a CubicSplineStrategy whose coefficients come from knot slopes
+    instead of the spline's solve; every evaluation (values, derivatives, integrals, replication) is the spline's"""
+
+    def __init__(self, kind, dydx, mode):
+        super().__init__(None, None, mode)
+        self._kind, self._dydx = kind, dydx
+
+    def _bind(self, interpolator):
+        # the slopes stay with the strategy: like a CubicSplineStrategy it may be bound to several interpolators
+        L.check(L.load().ndi_interp1d_hermite_build(interpolator._handle(), self._kind, L.ptr(self._dydx), 0))
 
 
 def _ndarray_debug(a):

@@ -2,7 +2,7 @@
 //! No Triton, no multi-backend dispatch, no CPU fallback: without nvcc the build fails.
 use std::{env, path::PathBuf, process::Command};
 
-const SOURCES: [&str; 9] = ["ndi_api.cu", "ndi_eval.cu", "ndi_bin.cu", "ndi_sweep.cu", "ndi_grid.cu", "ndi_spline.cu", "ndi_rowsplit.cu", "ndi_partition.cu", "ndi_integral.cu"];
+const SOURCES: [&str; 10] = ["ndi_api.cu", "ndi_eval.cu", "ndi_bin.cu", "ndi_sweep.cu", "ndi_grid.cu", "ndi_spline.cu", "ndi_rowsplit.cu", "ndi_partition.cu", "ndi_integral.cu", "ndi_hermite.cu"];
 
 fn main() {
     let out = PathBuf::from(env::var("OUT_DIR").unwrap());

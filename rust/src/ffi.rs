@@ -13,6 +13,11 @@ pub const NDI_NO_INTEGRAL: ndi_status = 9;
 pub const NDI_INTEGRAL_LINEAR: i32 = 0;
 pub const NDI_INTEGRAL_CUBIC: i32 = 1;
 
+pub const NDI_HERMITE_PCHIP: i32 = 0;
+pub const NDI_HERMITE_AKIMA: i32 = 1;
+pub const NDI_HERMITE_MAKIMA: i32 = 2;
+pub const NDI_HERMITE_GIVEN: i32 = 3;
+
 pub const NDI_F32: i32 = 0;
 pub const NDI_F64: i32 = 1;
 pub const NDI_I32: i32 = 2;
@@ -53,6 +58,8 @@ extern "C" {
     pub fn ndi_interp1d_integral_build(h: *mut ndi_interp1d, kind: i32) -> ndi_status;
     pub fn ndi_interp1d_cubic_integral(h: *const ndi_interp1d, lo: *const c_void, hi: *const c_void, nq: i64, extrap_mode: i32, out: *mut c_void, first_bad: *mut i64, bad_bound: *mut i32) -> ndi_status;
     pub fn ndi_interp1d_linear_integral(h: *const ndi_interp1d, lo: *const c_void, hi: *const c_void, nq: i64, extrapolate: i32, out: *mut c_void, first_bad: *mut i64, bad_bound: *mut i32) -> ndi_status;
+    /// shape-preserving cubics (not in the reference): PCHIP, Akima, makima or given slopes (`dydx`, host memory)
+    pub fn ndi_interp1d_hermite_build(h: *mut ndi_interp1d, kind: i32, dydx: *const c_void, flags: u32) -> ndi_status;
 
     pub fn ndi_interp1d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp1d) -> ndi_status;
     pub fn ndi_interp2d_create_strided(dtype: i32, x: *const c_void, n: i64, x_stride: i64, y: *const c_void, m: i64, y_stride: i64, data: *const c_void, ndim: i32, shape: *const i64, strides: *const i64, flags: u32, out: *mut *mut ndi_interp2d) -> ndi_status;

@@ -16,6 +16,7 @@ use crate::{
 };
 
 pub mod cubic_spline;
+pub mod hermite;
 mod linear;
 pub use linear::Linear;
 
